@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ensemble member-timesteps/sec of the SIPNET integration loop on 1..8 B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU)
 
 Workload (BASELINE.json configs[3], "C4", the north-star target; weak scaling): ONE synthetic site, 10 years of
@@ -73,7 +73,15 @@ def parse_args():
     ap.add_argument("--workload", default="c4", choices=["c4", "c3"],
                     help="c4 = the bench workload; c3 = BASELINE.json configs[2] as one extra line (10k sites x 100 members)")
     ap.add_argument("--sites", type=int, default=0, help="c3: sites per GPU (default 10000 / n_gpus)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="c4 workload of --impl ours only: rank 0 writes what the last timed pass returned as "
+                         "DIR/<name>.npy (float64, under 64 MB in all), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c4"):
+        ap.error("--dump-outputs applies to the c4 workload of --impl ours only")
+    return args
 
 
 # ---------------------------------------------------------------------------- clocks
@@ -399,6 +407,8 @@ def section_c4(args, D: Dist, lib, site, fp64_peak_tflops):
     launches = ens.launch_count() - launches0
     ms_per_step = D.max(total_ms / args.steps)
     levels = ens.team_last_levels()
+    if args.dump_outputs and D.rank == 0:
+        dump_outputs(args.dump_outputs, ens, M, T)
 
     # phases of one pass (an extra, untimed pass with a stopwatch around each phase)
     kern, summ = [], []
@@ -459,20 +469,56 @@ def section_c4(args, D: Dist, lib, site, fp64_peak_tflops):
                 e2e_ms=e2e_ms, h2d=par_bytes, d2h=out_bytes, levels=levels, replayed=replayed, spot=spot)
 
 
+def kept_columns(ens, M: int, T: int):
+    """Zero-copy torch view [2][T][M] of the per-member NEE and GPP columns the summaries are taken over."""
+    import torch
+    from sipnet_b200 import _abi as A
+    from sipnet_b200.distributed import DeviceArray
+    ld = (M + 15) // 16 * 16
+    return DeviceArray(ens.device_ptr(A.GATHER_FULL), (2, T, M), (T * ld, ld, 1)).tensor(torch.cuda.current_device())
+
+
+DUMP_MEMBERS = 64       # per-member columns are 16 B per member-step (15 GB at the default size): the dump keeps a sample
+DUMP_BYTES = 60 << 20   # data of all --dump-outputs files; with the .npy headers the dump stays under 64 MB
+
+
+def dump_members(M: int) -> np.ndarray:
+    """The fixed, seeded sample of a rank's members whose NEE / GPP columns --dump-outputs keeps."""
+    return np.sort(np.random.default_rng(20261020).choice(M, size=min(M, DUMP_MEMBERS), replace=False))
+
+
+def dump_steps(T: int, values_per_step: int) -> np.ndarray:
+    """The steps --dump-outputs keeps: all T of them, or as many evenly spaced ones (first and last included) as fit
+    DUMP_BYTES when the run is too long for all."""
+    n = min(T, DUMP_BYTES // (8 * values_per_step))
+    return np.linspace(0, T - 1, n).round().astype(np.int64)
+
+
+def dump_outputs(path: str, ens, M: int, T: int) -> None:
+    """--dump-outputs: the team summaries of the last pass as its caller receives them, and the NEE / GPP columns of
+    dump_members(M), at the steps dump_steps() keeps."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"mean": ens.mean(), "variance": ens.variance(), "quantiles": ens.quantiles()}
+    pick = dump_members(M)
+    steps = dump_steps(T, sum(a.size for a in arrays.values()) // T + 2 * pick.size)
+    arrays = {name: a[..., steps] for name, a in arrays.items()}
+    arrays["member_nee_gpp"] = kept_columns(ens, M, T)[:, :, pick.tolist()][:, steps.tolist()].cpu().numpy()
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_BYTES
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def oracle_spot_check(site, params, ens):
     """A seeded sample of the bench ensemble's members against the oracle (CPU restatement, pinned to the reference),
     bit for bit: the kept summary columns of the big run, and all 32 columns through a small full-output handle."""
     from oracle.pyoracle import Oracle
     from sipnet_b200 import _abi as A, api, synth
     import torch
-    from sipnet_b200.distributed import DeviceArray
     rng = np.random.default_rng(20261017)
     pick = sorted(int(x) for x in rng.choice(params.shape[1], size=3, replace=False))
     T = site.nsteps
     M = params.shape[1]
-    ld = (M + 15) // 16 * 16
-    cols = DeviceArray(ens.device_ptr(A.GATHER_FULL), (2, T, M), (T * ld, ld, 1)).tensor(torch.cuda.current_device())
-    kept = cols[:, :, pick].cpu().numpy()                      # [2][T][3]: NEE, GPP of the picked members
+    kept = kept_columns(ens, M, T)[:, :, pick].cpu().numpy()  # [2][T][3]: NEE, GPP of the picked members
     orc = Oracle()
     with api.Ensemble([site], np.ascontiguousarray(params[:, pick]), None, dict(synth.SYNTH_FLAGS), outputs=A.OUT_FULL,
                       math=A.MATH_FAST, device=torch.cuda.current_device()) as small:

@@ -61,6 +61,75 @@ def test_our_arm_line():
     assert line["c2"]["d2h_probe"]["gb_s_all_ranks"] >= line["c2"]["e2e"]["d2h_gb_s_all_ranks"] > 0   # the ceiling beside it
 
 
+@pytest.mark.gpu
+def test_dumped_outputs_repeat_run_to_run_and_are_the_pass_results(tmp_path):
+    """--dump-outputs writes what the last timed pass returned; the same arguments give the same inputs, so two runs
+    write the same arrays.  They are the C4 pass's results: the members' NEE / GPP columns of a fresh run, bit for
+    bit and equal to the oracle, and the ensemble summaries of those columns."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from oracle.pyoracle import Oracle
+    from sipnet_b200 import _abi as A, api, synth
+    M = 2048
+    names = ("mean", "variance", "quantiles", "member_nee_gpp")
+    dumps = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        r, line = run_bench("--steps", "2", "--warmup", "1", "--members", str(M), "--years", "1", "--no-cpu-baseline",
+                            "--no-extras", "--dump-outputs", str(d))
+        assert r.returncode == 0 and line is not None, r.stderr[-2000:]
+        assert sorted(p.name for p in d.iterdir()) == sorted(n + ".npy" for n in names)
+        dumps.append({n: np.load(d / (n + ".npy")) for n in names})
+    T = line["config"]["model_steps"]
+    a, b = dumps
+    assert a["mean"].shape == a["variance"].shape == (1, 2, T) and a["quantiles"].shape == (1, 2, 3, T)
+    assert a["member_nee_gpp"].shape == (2, T, 64)
+    for n in names:
+        assert a[n].dtype == np.float64 and np.isfinite(a[n]).all(), n
+        assert np.array_equal(a[n], b[n]), n
+
+    site = synth.synth_site(0, 1, "half-daily")
+    params = synth.synth_params(M, stream=100)
+    with api.Ensemble([site], params, None, dict(synth.SYNTH_FLAGS), math=A.MATH_FAST, summary_cols=[A.O["nee"], A.O["gpp"]],
+                      outputs=A.OUT_MOMENTS | A.OUT_QUANTILES, quantiles=bench.QUANTILES) as ens:
+        ens.run()
+        ens.sync()
+        x = bench.kept_columns(ens, M, T).cpu().numpy()         # [2][T][M]: NEE, GPP of every member
+    pick = bench.dump_members(M)
+    assert np.array_equal(a["member_nee_gpp"], x[:, :, pick])
+    scale = np.abs(x).max()
+    np.testing.assert_allclose(a["mean"][0], x.mean(axis=2), rtol=1e-12, atol=1e-12 * scale)
+    np.testing.assert_allclose(a["variance"][0], x.var(axis=2), rtol=1e-9, atol=1e-9 * scale ** 2)
+    np.testing.assert_allclose(a["quantiles"][0], np.quantile(x, bench.QUANTILES, axis=2).transpose(1, 0, 2), rtol=4e-16,
+                               atol=1e-300)
+    orc = Oracle()
+    for j in (0, pick.size - 1):
+        rc, done, o_out, _, _ = orc.run(synth.SYNTH_FLAGS, params[:, pick[j]], site, want_debug=False)
+        assert rc == 0 and done == T
+        assert np.array_equal(a["member_nee_gpp"][:, :, j], o_out[:, [A.O["nee"], A.O["gpp"]]].T)
+
+
+def test_dump_stays_under_64_mb_for_long_runs():
+    """Past DUMP_BYTES the dump keeps evenly spaced steps, the first and the last included."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    assert np.array_equal(bench.dump_steps(7306, 10 + 2 * 64), np.arange(7306))
+    for T in (58440, 365 * 2 * 1000, 10 ** 7):
+        per_step = 10 + 2 * bench.dump_members(131072).size
+        s = bench.dump_steps(T, per_step)
+        assert s[0] == 0 and s[-1] == T - 1 and (np.diff(s) > 0).all()
+        assert 8 * per_step * s.size <= bench.DUMP_BYTES < 64_000_000 - 4096
+
+
+@pytest.mark.parametrize("args", [("--steps", "0"), ("--impl", "reference", "--dump-outputs", "d"),
+                                  ("--workload", "c3", "--dump-outputs", "d")])
+def test_bad_arguments_are_refused(args):
+    r, line = run_bench(*args)
+    assert r.returncode == 2 and line is None and "bench.py: error:" in r.stderr
+
+
 def test_both_arms_share_one_config_object():
     """`config` must be the same dict in both arms (the driver compares them)."""
     import argparse
