@@ -250,7 +250,7 @@ typedef struct sipnet_gpu_config {
   int32_t n_summary_cols;
   const int32_t *summary_cols; /* enum sipnet_gpu_out_col values */
   int32_t n_quantiles;
-  const double *quantiles;     /* probabilities in [0,1] */
+  const double *quantiles;     /* probabilities in [0,1], any order, repeats allowed; results in this order */
   double nee_sigma;            /* log-likelihood observation sigma (> 0) */
 
   int32_t max_event_records;   /* per member, for SIPNET_GPU_OUT_EVENTS */
@@ -433,7 +433,8 @@ int sipnet_gpu_measure_fp64_peak(int device, double *tflops);
  * mean / population variance over the finite entries and the requested quantiles (numpy "linear" rule).
  * Used for exact cross-GPU quantiles: after an all-to-all time-transpose each rank holds complete
  * ensembles for its share of the steps and summarises them locally.  d_mean/d_var are [nrows],
- * d_quant is [nq][nrows] (any of them may be NULL); `probs` is a host array; `stream` a cudaStream_t or NULL.
+ * d_quant is [nq][nrows] (any of them may be NULL); `probs` is a host array of probabilities in [0,1], in any order
+ * (row q of d_quant belongs to probs[q]); `stream` a cudaStream_t or NULL.
  * On a non-NULL stream the call only enqueues work (results are ordered on that stream); on the NULL stream it
  * returns when the results are complete.
  */
@@ -482,6 +483,13 @@ int sipnet_gpu_comm_member_counts(const sipnet_gpu_comm *c, int64_t *counts /* [
  *     whole sites per device when there are at least as many sites as devices, otherwise an even contiguous share
  *     of every site's members per device.  ndevices <= 0: all visible devices; devices == NULL: 0..ndevices-1.
  *     cfg->device and cfg->stream are ignored (a caller stream cannot span devices: rejected if set).
+ *     A device that would get no member (fewer members than devices in a site or in a device's site range) is left
+ *     out: the team is then smaller than the list.
+ *     A list that names ONE device several times (e.g. {0, 0, 0}) forms a loopback team: as many ranks as entries,
+ *     all on that device, partitioned as above; the team's collectives are device-to-device copies and a histogram
+ *     add instead of NCCL (NCCL does not put two ranks of a communicator on one GPU), and NCCL is not loaded.  It
+ *     exists to test the cross-rank select on one GPU; it is no faster than one rank.  A list that repeats a device
+ *     and also names others is rejected.
  *     gather() delivers exactly what one GPU would: per-member data in the configuration's member order, summaries
  *     per site (through the team select when a site is split).  This is what `sipnet_gpu --site-list` uses. */
 typedef struct sipnet_gpu_multi sipnet_gpu_multi;

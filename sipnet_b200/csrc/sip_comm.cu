@@ -18,6 +18,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <numeric>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -109,6 +110,7 @@ struct Local {
 
 struct sipnet_gpu_comm {
   int nranks = 1;
+  bool loopback = false;                 // every rank on one device: the collectives are device copies, not NCCL
   std::vector<Local> local;              // the ranks this process drives (1 with one process per GPU)
   std::vector<int64_t> memberCounts;     // [nranks]
   float lastExchangeMs = 0.f, lastSummaryMs = 0.f;
@@ -150,8 +152,28 @@ struct Group {
   }
 };
 
+// the local streams, all finished (the loopback collectives copy between the ranks' buffers on one device)
+int sync_all(sipnet_gpu_comm *c) {
+  for (Local &l : c->local) {
+    CUDA_OK(cudaSetDevice(l.h->device));
+    CUDA_OK(cudaStreamSynchronize(l.h->stream));
+  }
+  return 0;
+}
+
 int all_gather_bytes(sipnet_gpu_comm *c, size_t bytesPerRank, void *(*buf)(Local &)) {
   if (c->nranks == 1) return 0;
+  if (c->loopback) {
+    if (int rc = sync_all(c)) return rc;
+    for (Local &to : c->local)
+      for (Local &from : c->local)
+        if (&to != &from) {
+          const size_t off = (size_t)from.rank * bytesPerRank;
+          CUDA_OK(cudaMemcpyAsync(static_cast<char *>(buf(to)) + off, static_cast<char *>(buf(from)) + off, bytesPerRank,
+                                  cudaMemcpyDeviceToDevice, to.h->stream));
+        }
+    return sync_all(c);
+  }
   const Group g(c);
   if (int rc = g.begin()) return rc;
   for (Local &l : c->local) {
@@ -164,6 +186,15 @@ int all_gather_bytes(sipnet_gpu_comm *c, size_t bytesPerRank, void *(*buf)(Local
 
 int all_reduce_hist(sipnet_gpu_comm *c, size_t words) {
   if (c->nranks == 1) return 0;
+  if (c->loopback) {  // sum into rank 0's buffer, then copy the sum back to every other rank
+    if (int rc = sync_all(c)) return rc;
+    Local &l0 = c->local[0];
+    CUDA_OK(cudaSetDevice(l0.h->device));
+    for (size_t i = 1; i < c->local.size(); ++i) CUDA_OK(gs::launch_add_u32(l0.hist, c->local[i].hist, words, l0.h->stream));
+    for (size_t i = 1; i < c->local.size(); ++i)
+      CUDA_OK(cudaMemcpyAsync(c->local[i].hist, l0.hist, words * sizeof(uint32_t), cudaMemcpyDeviceToDevice, l0.h->stream));
+    return sync_all(c);
+  }
   const Group g(c);
   if (int rc = g.begin()) return rc;
   for (Local &l : c->local) {
@@ -243,6 +274,10 @@ int team_summaries(sipnet_gpu_comm *c) {
     a.nqTotal = nqTotal;
   }
   c->lastLevels = 0;
+  // the select takes the probabilities ascending (sip_gsum.cu resolve_level); results go to the caller's order
+  std::vector<int> order((size_t)nqTotal);
+  std::iota(order.begin(), order.end(), 0);
+  std::stable_sort(order.begin(), order.end(), [h0](int i, int j) { return h0->quantiles[(size_t)i] < h0->quantiles[(size_t)j]; });
   // quantiles in groups of kGsMaxQ; the moments ride with the first group
   for (int q0 = 0; q0 < std::max(nqTotal, 1); q0 += gs::kGsMaxQ) {
     const int nq = std::min(gs::kGsMaxQ, nqTotal - q0);
@@ -250,8 +285,10 @@ int team_summaries(sipnet_gpu_comm *c) {
       Local &l = c->local[i];
       gs::GsArgs &a = args[i];
       a.nq = std::max(nq, 0);
-      a.q0 = q0;
-      for (int k = 0; k < a.nq; ++k) a.probs[k] = l.h->quantiles[(size_t)(q0 + k)];
+      for (int k = 0; k < a.nq; ++k) {
+        a.qOut[k] = order[(size_t)(q0 + k)];
+        a.probs[k] = l.h->quantiles[(size_t)a.qOut[k]];
+      }
       a.wantMoments = (l.h->mean != nullptr && q0 == 0) ? 1 : 0;
       CUDA_OK(cudaSetDevice(l.h->device));
       cudaError_t e = gs::launch_pass0(a, l.h->stream);
@@ -325,10 +362,10 @@ extern "C" int sipnet_gpu_comm_unique_id(void *id) {
 }
 
 static int finish_comm(sipnet_gpu_comm *c) {
-  // member counts of all ranks (for the log-likelihood gather's layout)
+  // member counts of all ranks (for the log-likelihood gather's layout); no exchange when this process drives them all
   c->memberCounts.assign((size_t)c->nranks, 0);
-  if (c->nranks == 1) {
-    c->memberCounts[0] = c->local[0].h->nmembers;
+  if ((int)c->local.size() == c->nranks) {
+    for (const Local &l : c->local) c->memberCounts[(size_t)l.rank] = l.h->nmembers;
     return 0;
   }
   std::vector<int64_t *> dev(c->local.size(), nullptr);
@@ -519,6 +556,17 @@ extern "C" int sipnet_gpu_multi_init(const sipnet_gpu_config *cfg, int32_t ndevi
   } else {
     for (int i = 0; i < ndevices; ++i) devs.push_back(devices ? devices[i] : i);
   }
+  // one device named several times: a loopback team, every rank on that device (a test seam for the team select)
+  bool loopback = false;
+  {
+    std::vector<int> u(devs);
+    std::sort(u.begin(), u.end());
+    if (std::unique(u.begin(), u.end()) != u.end()) {
+      if (u.front() != u.back())
+        return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "a device list names distinct devices once each, or one device repeatedly");
+      loopback = true;
+    }
+  }
   for (int d : devs)
     if (d < 0 || d >= visible) return fail(SIPNET_GPU_ERR_NO_DEVICE, "device %d not present", d);
   if (cfg->nsites <= 0 || !cfg->sites || cfg->nmembers <= 0 || !cfg->params)
@@ -526,7 +574,7 @@ extern "C" int sipnet_gpu_multi_init(const sipnet_gpu_config *cfg, int32_t ndevi
   if (cfg->stream) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "a caller stream cannot be shared by several devices");
   // never more devices than members
   while ((int64_t)devs.size() > cfg->nmembers) devs.pop_back();
-  const int D = (int)devs.size();
+  int D = (int)devs.size();
 
   sipnet_gpu_multi *m = new sipnet_gpu_multi();
   m->nmembers = cfg->nmembers;
@@ -535,7 +583,6 @@ extern "C" int sipnet_gpu_multi_init(const sipnet_gpu_config *cfg, int32_t ndevi
   m->nquant = cfg->n_quantiles;
   m->outputs = cfg->outputs;
   m->split = cfg->nsites < D;
-  m->parts.resize((size_t)D);
   std::vector<int32_t> memberSite((size_t)cfg->nmembers, 0);
   if (cfg->member_site)
     for (int64_t i = 0; i < cfg->nmembers; ++i) memberSite[(size_t)i] = cfg->member_site[i];
@@ -561,24 +608,17 @@ extern "C" int sipnet_gpu_multi_init(const sipnet_gpu_config *cfg, int32_t ndevi
     ringSlots = (int32_t)std::min<double>(kRingMax, std::max(2.0, bound));
   }
 
+  // the partition over D devices; a device that would get no member is left out, so the team may be smaller than D
+  std::vector<std::vector<int64_t>> picks;  // per kept device: its global member indices, ascending
+  std::vector<int> keptDevs;
   for (int d = 0; d < D; ++d) {
-    sipnet_gpu_multi::Part &p = m->parts[(size_t)d];
-    sipnet_gpu_config sub = *cfg;
-    sub.device = devs[(size_t)d];
-    sub.ring_slots = ringSlots;
-    std::vector<int32_t> subSite;
-    std::vector<double> subParams;
-    std::vector<int64_t> pick;  // global member indices of this device, ascending
+    sipnet_gpu_multi::Part p;
+    std::vector<int64_t> pick;
     if (!m->split) {
       p.site0 = (cfg->nsites * d) / D;
       p.site1 = (cfg->nsites * (d + 1)) / D;
       for (int64_t i = 0; i < cfg->nmembers; ++i)
         if (memberSite[(size_t)i] >= p.site0 && memberSite[(size_t)i] < p.site1) pick.push_back(i);
-      p.member0 = pick.empty() ? 0 : pick.front();
-      p.member1 = pick.empty() ? 0 : pick.back() + 1;
-      sub.nsites = p.site1 - p.site0;
-      sub.sites = cfg->sites + p.site0;
-      for (int64_t i : pick) subSite.push_back(memberSite[(size_t)i] - (int32_t)p.site0);
     } else {
       p.site0 = 0;
       p.site1 = cfg->nsites;
@@ -588,17 +628,38 @@ extern "C" int sipnet_gpu_multi_init(const sipnet_gpu_config *cfg, int32_t ndevi
         p.siteGlobal0.push_back(siteM0[(size_t)s] + lo);
         p.siteLocal0.push_back(local);
         p.siteCount.push_back(hi - lo);
-        for (int64_t i = lo; i < hi; ++i) {
-          pick.push_back(siteM0[(size_t)s] + i);
-          subSite.push_back((int32_t)s);
-        }
+        for (int64_t i = lo; i < hi; ++i) pick.push_back(siteM0[(size_t)s] + i);
         local += hi - lo;
       }
     }
-    if (pick.empty()) {
-      sipnet_gpu_multi_destroy(m);
-      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "device %d would get no members", d);
+    if (pick.empty()) continue;
+    p.member0 = pick.front();
+    p.member1 = pick.back() + 1;
+    m->parts.push_back(p);
+    picks.push_back(std::move(pick));
+    keptDevs.push_back(devs[(size_t)d]);
+  }
+  devs = keptDevs;
+  D = (int)devs.size();
+  // whole sites: the site ranges of the devices left out hold no member; the kept devices take them over (each one
+  // up to the next kept device's first site), so the summaries still cover every site in order
+  if (!m->split)
+    for (int d = 0; d < D; ++d) {
+      m->parts[(size_t)d].site0 = d == 0 ? 0 : m->parts[(size_t)d - 1].site1;
+      m->parts[(size_t)d].site1 = d + 1 < D ? m->parts[(size_t)d + 1].site0 : cfg->nsites;
     }
+
+  for (int d = 0; d < D; ++d) {
+    const sipnet_gpu_multi::Part &p = m->parts[(size_t)d];
+    const std::vector<int64_t> &pick = picks[(size_t)d];
+    sipnet_gpu_config sub = *cfg;
+    sub.device = devs[(size_t)d];
+    sub.ring_slots = ringSlots;
+    std::vector<int32_t> subSite;
+    std::vector<double> subParams;
+    sub.nsites = p.site1 - p.site0;
+    sub.sites = cfg->sites + p.site0;
+    for (int64_t i : pick) subSite.push_back(memberSite[(size_t)i] - (int32_t)p.site0);
     const int64_t nm = (int64_t)pick.size();
     subParams.resize((size_t)SIPNET_GPU_NPARAMS * (size_t)nm);
     for (int k = 0; k < SIPNET_GPU_NPARAMS; ++k)
@@ -627,7 +688,8 @@ extern "C" int sipnet_gpu_multi_init(const sipnet_gpu_config *cfg, int32_t ndevi
     c->local[(size_t)d].rank = d;
   }
   m->comm = c;
-  if (D > 1) {
+  c->loopback = loopback && D > 1;
+  if (D > 1 && !c->loopback) {
     const NcclApi *api = nccl_api();
     if (!api) {
       sipnet_gpu_multi_destroy(m);

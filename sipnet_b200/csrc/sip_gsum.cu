@@ -6,6 +6,7 @@
 // The reference has no ensemble code (SURVEY 8c): definitions as in sip_reduce.cu; tests compare with numpy.
 #include "sip_gsum.cuh"
 
+#include <algorithm>
 #include <type_traits>
 
 namespace sip {
@@ -232,12 +233,12 @@ __device__ void resolve_level(const GsArgs &a, GsRow &S, const unsigned int *his
         continue;
       }
       done = false;
-      // statistics ascend, so equal prefixes are adjacent
-      if (r > 0 && rbits[r - 1] == 0 && S.prefix[r] == S.prefix[r - 1]) {
-        S.slotOf[r] = S.slotOf[r - 1];
-      } else {
-        S.slotOf[r] = (uint8_t)ns++;
-      }
+      // Precondition: the probabilities ascend, so a statistic's rank only steps back to a rank listed before it
+      // (hi_i = lo_i + 1 > lo_{i+1} = lo_i).  An open statistic shares the slot of an earlier open one with the
+      // same prefix, adjacent or not: two slots with one prefix would leave the first one's histogram empty.
+      int e = 0;
+      while (e < r && (rbits[e] != 0 || S.prefix[e] != S.prefix[r])) ++e;
+      S.slotOf[r] = e < r ? S.slotOf[e] : (uint8_t)ns++;
     }
     S.nslots = (uint8_t)ns;
     S.done = done ? 1 : 0;
@@ -585,7 +586,7 @@ __global__ void gs_finish_kernel(const GsArgs a, const int64_t rows) {
       // numpy's _lerp: a + (b - a) t, evaluated from the b side when t >= 0.5
       v = (fr >= 0.5) ? xhi - (xhi - xlo) * (1.0 - fr) : xlo + (xhi - xlo) * fr;
     }
-    a.quant[(sc * a.nqTotal + (a.q0 + i)) * a.nsteps + t] = v;
+    a.quant[(sc * a.nqTotal + a.qOut[i]) * a.nsteps + t] = v;
   }
   if (a.wantMoments && lane == 0) {
     const double n = gx->n;
@@ -614,6 +615,15 @@ cudaError_t launch_emit(const GsArgs &a, cudaStream_t stream) {
 cudaError_t launch_finish(const GsArgs &a, cudaStream_t stream) {
   const int64_t rows = gs_rows(a);
   gs_finish_kernel<<<(unsigned)((rows + 3) / 4), 128, 0, stream>>>(a, rows);
+  return cudaGetLastError();
+}
+
+__global__ void add_u32_kernel(uint32_t *dst, const uint32_t *src, size_t n) {
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) dst[i] += src[i];
+}
+cudaError_t launch_add_u32(uint32_t *dst, const uint32_t *src, size_t n, cudaStream_t stream) {
+  const size_t blocks = std::min<size_t>((n + 255) / 256, 4096);
+  add_u32_kernel<<<(unsigned)std::max<size_t>(blocks, 1), 256, 0, stream>>>(dst, src, n);
   return cudaGetLastError();
 }
 

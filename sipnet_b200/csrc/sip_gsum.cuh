@@ -63,7 +63,8 @@ struct GsArgs {
   int32_t nsites, ncols;
   int32_t colSlot[kGsMaxCols];  // slot of summary column i in `out`
   int32_t nq;
-  double probs[kGsMaxQ];
+  double probs[kGsMaxQ];  // ascending (the caller sorts them; the slot assignment of resolve_level relies on it)
+  int32_t qOut[kGsMaxQ];  // index of each probability's result among the column's nqTotal quantiles
   int32_t nranks, rank;
   int32_t wantMoments;
   // scratch (device).  *Local = this rank's contribution, *All = [nranks][...] after the gather (the same
@@ -78,7 +79,7 @@ struct GsArgs {
   int32_t *flags;      // [0] = some row needs the next level
   // results, in the handle's layout: mean/var [site][col][n], quant [site][col][q][n]
   double *mean, *var, *quant;
-  int32_t q0, nqTotal;  // quantile group offset and total count (quant rows are [nqTotal] per column)
+  int32_t nqTotal;  // quantiles per column (quant rows are [nqTotal] per column)
 };
 
 inline int64_t gs_rows(const GsArgs &a) { return (int64_t)a.nsites * a.ncols * a.nsteps; }
@@ -87,6 +88,8 @@ cudaError_t launch_pass0(const GsArgs &a, cudaStream_t stream);
 cudaError_t launch_level(const GsArgs &a, int level, cudaStream_t stream);
 cudaError_t launch_emit(const GsArgs &a, cudaStream_t stream);
 cudaError_t launch_finish(const GsArgs &a, cudaStream_t stream);
+// dst[i] += src[i] for i < n (the histogram sum of a team whose ranks share one device)
+cudaError_t launch_add_u32(uint32_t *dst, const uint32_t *src, size_t n, cudaStream_t stream);
 
 }  // namespace gs
 }  // namespace sip

@@ -13,7 +13,10 @@
 // bit-reproducible run to run.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cstdint>
+#include <numeric>
+#include <vector>
 
 #include "sip_libm.cuh"
 #include "sip_num.cuh"
@@ -93,7 +96,8 @@ struct RowSpan {
   int member0, memberCount;
 };
 struct QuantileProbs {
-  double p[kSelMaxQ];
+  double p[kSelMaxQ];    // ascending (the launcher sorts the caller's probabilities)
+  int out[kSelMaxQ];     // where each one's result goes: its index in the caller's list
 };
 
 struct SelState {
@@ -139,12 +143,18 @@ __device__ __forceinline__ void resolve_level(SelState &S, const unsigned int *h
     }
   }
   __syncthreads();
-  if (threadIdx.x == 0) {  // ranks ascend, so equal prefixes are adjacent
+  if (threadIdx.x == 0) {
+    // Precondition: the probabilities ascend.  The ranks lo_0, hi_0, lo_1, hi_1, ... then only step back to a rank
+    // already listed (hi_i = lo_i + 1 > lo_{i+1} = lo_i), so every new prefix is larger than the ones before it and
+    // the slots hold ascending key ranges.  A rank that steps back shares the slot of its earlier equal prefix.
     int ns = 0;
     unsigned int base = 0;
     for (int r = 0; r < nr; ++r) {
-      if (r > 0 && S.prefix[r] == S.prefix[r - 1]) {
-        S.slotOf[r] = ns - 1;
+      const uint64_t top = S.prefix[r] >> level_shift(level);
+      int s = 0;
+      while (s < ns && S.slotTop[s] != top) ++s;
+      if (s < ns) {
+        S.slotOf[r] = s;
         continue;
       }
       S.slotOf[r] = ns;
@@ -261,7 +271,7 @@ __device__ __forceinline__ void compact_pass(const double *row, int count, SelSt
 // ---- per-row summary: moments and exact quantiles in (typically) three reads of the row ----------
 // grid = (nsteps, nsites); block = kSelThreads; dynamic shared = kSelDynBytes.
 //   mean/var[site * momStride + t]              (either both or neither)
-//   quant[site * qStride + q * nsteps + t]      (nq <= kSelMaxQ)
+//   quant[site * qStride + probs.out[q] * nsteps + t]   (nq <= kSelMaxQ)
 // Pass 1: finite count + sum (+ level-0 histogram when the row is longer than kCandCap).
 // Pass 2: sum of squared deviations (+ level-1 histogram).  Further histogram passes only while the
 // wanted prefixes still hold more than kCandCap keys (heavily duplicated data).  Last pass: the few keys
@@ -327,7 +337,7 @@ __global__ void __launch_bounds__(kSelThreads, 2)
   }
 
   if (constantRow) {
-    if (tid < nq) quant[(int64_t)site * qStride + (int64_t)tid * nsteps + t] = vmin;
+    if (tid < nq) quant[(int64_t)site * qStride + (int64_t)probs.out[tid] * nsteps + t] = vmin;
   } else if (nq > 0 && n > 0) {
     if (tid < nq) {
       const double pos = probs.p[tid] * (n - 1.0);
@@ -381,7 +391,8 @@ __global__ void __launch_bounds__(kSelThreads, 2)
       __syncthreads();
       for (unsigned int i = ctot + tid; i < n2; i += kSelThreads) cand[i] = ~0ull;
       __syncthreads();
-      // slots hold ascending key ranges in ascending order, so one sort of the whole buffer sorts each slot in place
+      // slots hold ascending key ranges in ascending order (the probabilities ascend: see resolve_level), so one
+      // sort of the whole buffer sorts each slot in place
       for (unsigned int kk = 2; kk <= n2; kk <<= 1) {
         for (unsigned int j = kk >> 1; j > 0; j >>= 1) {
           for (unsigned int i = tid; i < n2; i += kSelThreads) {
@@ -405,11 +416,11 @@ __global__ void __launch_bounds__(kSelThreads, 2)
       const double xlo = val_of(S.prefix[2 * tid]), xhi = val_of(S.prefix[2 * tid + 1]);
       const double fr = S.frac[tid];
       // numpy's _lerp: a + (b - a) t, evaluated from the b side when t >= 0.5
-      quant[(int64_t)site * qStride + (int64_t)tid * nsteps + t] =
+      quant[(int64_t)site * qStride + (int64_t)probs.out[tid] * nsteps + t] =
           (fr >= 0.5) ? xhi - (xhi - xlo) * (1.0 - fr) : xlo + (xhi - xlo) * fr;
     }
   } else if (nq > 0 && tid < nq) {
-    quant[(int64_t)site * qStride + (int64_t)tid * nsteps + t] = nan("");
+    quant[(int64_t)site * qStride + (int64_t)probs.out[tid] * nsteps + t] = nan("");
   }
 
   if (mean != nullptr) {
@@ -478,7 +489,7 @@ __global__ void __launch_bounds__(kWarpRowsPerBlock * 32)
 
 // One column's summaries for every (site, step) row.  mean/var may be null (quantiles only), nq may be 0.
 // `sites` = the handle's device site table, or null: then every row is columns [0, maxMembers) (nsites must be 1).
-// `probs` is a HOST array.
+// `probs` is a HOST array, in any order: the kernels take them ascending, each with the index its result goes to.
 cudaError_t launch_row_summary(const double *cols, int64_t ld, int64_t nsteps, const SiteDev *sites, int64_t nsites,
                                int64_t maxMembers, const double *probs, int nq, double *mean, double *var,
                                int64_t momStride, double *quant, int64_t qStride, cudaStream_t stream) {
@@ -499,18 +510,24 @@ cudaError_t launch_row_summary(const double *cols, int64_t ld, int64_t nsteps, c
     }
     return cudaSuccess;
   }
+  std::vector<int> order((size_t)(nq > 0 ? nq : 0));
+  std::iota(order.begin(), order.end(), 0);
+  std::stable_sort(order.begin(), order.end(), [probs](int i, int j) { return probs[i] < probs[j]; });
   for (int q0 = 0; q0 < (nq > 0 ? nq : 1); q0 += kSelMaxQ) {
     const int nqq = nq - q0 < kSelMaxQ ? nq - q0 : kSelMaxQ;
     const bool first = q0 == 0;
     QuantileProbs qp{};
-    for (int i = 0; i < nqq && nq > 0; ++i) qp.p[i] = probs[q0 + i];
+    for (int i = 0; i < nqq && nq > 0; ++i) {
+      qp.p[i] = probs[order[(size_t)(q0 + i)]];
+      qp.out[i] = order[(size_t)(q0 + i)];
+    }
     for (int64_t s0 = 0; s0 < nsites; s0 += 65535) {  // gridDim.y <= 65535: tile sites
       const int ns = (int)((nsites - s0) < 65535 ? (nsites - s0) : 65535);
       dim3 grid((unsigned)nsteps, (unsigned)ns);
       row_summary_kernel<<<grid, kSelThreads, kSelDynBytes, stream>>>(
           cols, ld, nsteps, sites != nullptr ? sites + s0 : nullptr, one, qp, nq > 0 ? nqq : 0,
           first && mean ? mean + s0 * momStride : nullptr, first && var ? var + s0 * momStride : nullptr, momStride,
-          quant ? quant + s0 * qStride + (int64_t)q0 * nsteps : nullptr, qStride);
+          quant ? quant + s0 * qStride : nullptr, qStride);
       cudaError_t e = cudaGetLastError();
       if (e != cudaSuccess) return e;
     }

@@ -1066,6 +1066,8 @@ extern "C" int sipnet_gpu_rows_summary(int device, const double *d_rows, int64_t
   if (!d_rows || nrows <= 0 || ncols <= 0 || ld < ncols || nq < 0 || (nq > 0 && (!probs || !d_quant)))
     return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "bad rows_summary arguments");
   if ((d_mean == nullptr) != (d_var == nullptr)) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "mean and var go together");
+  for (int i = 0; i < nq; ++i)
+    if (!(probs[i] >= 0.0 && probs[i] <= 1.0)) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "quantile probability out of [0,1]");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev)
     return fail(SIPNET_GPU_ERR_NO_DEVICE, "device %d not present", device);

@@ -3,8 +3,8 @@
 * a team of ONE rank runs the cross-rank summary kernels (sip_gsum.cu) without any exchange: its results must equal
   the single-GPU row summaries (sip_reduce.cu) -- quantiles bit for bit (both pick exact order statistics and use the
   same lerp), moments to rounding;
-* with two or more GPUs on the box: sipnet_gpu_multi_* (one process, all GPUs) must deliver exactly what one GPU
-  delivers -- per-member output bit for bit in both partitions (whole sites per device / one site's members split),
+* sipnet_gpu_multi_* (one process, all GPUs of a box with two or more; or a loopback team of several ranks on
+  GPU 0) must deliver exactly what one GPU delivers -- per-member output bit for bit in both partitions (whole sites per device / one site's members split),
   split-site summaries through the NCCL team select, log-likelihoods, event records.
 """
 import numpy as np
@@ -69,10 +69,13 @@ def test_team_select_handles_ties_and_tiny_rows():
 
 
 needs2 = pytest.mark.skipif("ngpus() < 2", reason="needs two GPUs on the box")
+# every GPU of the box, or a loopback team of 2 / 3 ranks on GPU 0 (the same collectives done by device copies)
+DEVICES = [pytest.param(None, marks=needs2, id="all-gpus"), pytest.param([0, 0], id="loopback2"),
+           pytest.param([0, 0, 0], id="loopback3")]
 
 
-@needs2
-def test_multi_split_site_equals_one_gpu():
+@pytest.mark.parametrize("devices", DEVICES)
+def test_multi_split_site_equals_one_gpu(devices):
     sites, P, ms = _ensemble(5000)
     site = sites[0]
     rng = np.random.default_rng(5)
@@ -83,8 +86,8 @@ def test_multi_split_site_equals_one_gpu():
         ens.run()
         ref = dict(out=ens.output(), mean=ens.mean(), var=ens.variance(), q=ens.quantiles(), ll=ens.loglik(),
                    state=ens.state(), status=ens.status(), counts=ens.event_counts(), recs=ens.event_records())
-    with api.MultiEnsemble(sites, P, ms, synth.SYNTH_FLAGS, **kw) as me:
-        assert me.ndevices == min(ngpus(), 8) and me.ndevices >= 2
+    with api.MultiEnsemble(sites, P, ms, synth.SYNTH_FLAGS, devices=devices, **kw) as me:
+        assert me.ndevices == (min(ngpus(), 8) if devices is None else len(devices)) and me.ndevices >= 2
         me.run()
         assert np.array_equal(me.output(), ref["out"], equal_nan=True)
         assert np.array_equal(me.state(), ref["state"], equal_nan=True)
@@ -100,8 +103,8 @@ def test_multi_split_site_equals_one_gpu():
         np.testing.assert_allclose(me.variance(), ref["var"], rtol=1e-11, atol=1e-24)
 
 
-@needs2
-def test_multi_whole_sites_equal_one_gpu():
+@pytest.mark.parametrize("devices", DEVICES)
+def test_multi_whole_sites_equal_one_gpu(devices):
     # more sites than GPUs on any box: whole sites per device (fewer sites than devices would split them instead)
     sites, P, ms, flags = synth.config_c3(nsites=11, members_per_site=40, nyears=2)
     kw = dict(outputs=A.OUT_FULL | A.OUT_MOMENTS | A.OUT_EVENTS, summary_cols=[A.O["nee"]], math=A.MATH_FAST,
@@ -109,8 +112,8 @@ def test_multi_whole_sites_equal_one_gpu():
     with api.Ensemble(sites, P, ms, flags, **kw) as ens:
         ens.run()
         ref = dict(out=ens.output(), mean=ens.mean(), var=ens.variance(), status=ens.status(), counts=ens.event_counts())
-    with api.MultiEnsemble(sites, P, ms, flags, **kw) as me:
-        assert me.ndevices <= 11
+    with api.MultiEnsemble(sites, P, ms, flags, devices=devices, **kw) as me:
+        assert me.ndevices <= 11 and (devices is None or me.ndevices == len(devices))
         me.run()
         assert np.array_equal(me.output(), ref["out"], equal_nan=True)
         assert np.array_equal(me.mean(), ref["mean"], equal_nan=True)        # whole sites: the same local kernels
