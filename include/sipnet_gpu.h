@@ -311,6 +311,7 @@ enum sipnet_gpu_counter {
 #define SIPNET_GPU_ST_MINN_LIMITED 0x400u   /* leaching + volatilisation capped by the mineral N pool (:119-130) */
 #define SIPNET_GPU_ST_REPLAY 0x40u        /* the optimistic kernel met an input outside its guards and the member
                                              was re-run by the general kernel (informational; results are exact) */
+#define SIPNET_GPU_ST_ANALYSIS_FLOORED 0x800u /* an assimilation left a pool below 0 and set it to +0.0 */
 
 /* carried state rows for SIPNET_GPU_GATHER_STATE (restart.c:148-308 field list) */
 enum sipnet_gpu_state_row {
@@ -390,6 +391,45 @@ int sipnet_gpu_reset(sipnet_gpu_handle *h);
  */
 int sipnet_gpu_set_state(sipnet_gpu_handle *h, const double *state, int64_t state_ld, const double *ring_values,
                          const double *ring_weights, int64_t ring_ld, int64_t next_step);
+
+/*
+ * Sequential data assimilation: the serial ensemble adjustment Kalman filter (EAKF; Anderson 2001, 2003) on the
+ * carried pools, per site, between two run() segments.
+ *
+ * rows[n_rows] are distinct pool rows SIPNET_S_plantWoodC .. SIPNET_S_plantStorageN (0..11); op[n_obs][n_rows] is the
+ * linear observation operator: observation k of member i is y_i = sum_j op[k][j] * x_ji.  value / variance are
+ * [nsites][n_obs]; a NaN value means the site has no observation k.
+ *
+ * A member takes part at its site iff its status has neither SIPNET_GPU_ST_BAD_ALLOCATION nor
+ * SIPNET_GPU_ST_NONFINITE and all of its rows are finite; other members are neither read nor written.  For each
+ * observation k in order and each site with a finite value y_obs (variance r), over the N members that take part:
+ *   ybar, xbar_j = means;  S_yy = sum (y_i - ybar)^2;  S_jy = sum (x_ji - xbar_j)(y_i - ybar)   (two passes)
+ *   skipped if N < 2 or S_yy == 0 or S_yy is not finite; otherwise
+ *   s2 = S_yy / (N - 1);  ybar_a = ybar + s2 / (s2 + r) * (y_obs - ybar);  alpha = sqrt(r / (s2 + r))
+ *   dy_i = (ybar_a - ybar) + (alpha - 1)(y_i - ybar);  x_ji += (S_jy / S_yy) * dy_i
+ * Observation k + 1 sees the state observation k left.  After the last one, every value of a member that some
+ * observation of the call updated and that is below 0 becomes +0.0, and the member gets
+ * SIPNET_GPU_ST_ANALYSIS_FLOORED (sticky; reset() clears it).  Nothing else changes: other state rows, the ring,
+ * parameters, log-likelihoods, event records, the last run range's outputs and summaries, the next step.  isAlive is
+ * derived from the pools when the next run() starts, so an analysis can revive or end a plant there, exactly as
+ * set_state() can.
+ *
+ * diag (may be NULL) receives double [nsites][n_obs][4] = {N, ybar, s2, ybar_a} per site and observation, taken before
+ * that observation's update; N is always filled, the other three are NaN where the pair was skipped or unobserved.
+ *
+ * Rejected with SIPNET_GPU_ERR_BAD_ARGUMENT, state untouched: NULL pointers; n_rows or n_obs < 1; repeated or other
+ * rows; a non-finite op entry or an all-zero op row; an infinite value; a missing, non-finite or non-positive variance
+ * where the value is finite.  Every call returns when the update is complete.
+ */
+typedef struct sipnet_gpu_obs_spec {
+  int32_t n_rows;
+  const int32_t *rows;     /* pool rows the analysis adjusts */
+  int32_t n_obs;
+  const double *op;        /* [n_obs][n_rows] */
+  const double *value;     /* [nsites][n_obs], NaN = not observed */
+  const double *variance;  /* [nsites][n_obs], finite and > 0 where value is finite */
+} sipnet_gpu_obs_spec;
+int sipnet_gpu_assimilate(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs, double *diag);
 
 /* Slots of the mean-NPP ring this handle uses (config ring_slots, or the automatic choice). */
 int32_t sipnet_gpu_ring_slots(const sipnet_gpu_handle *h);
@@ -478,6 +518,11 @@ int32_t sipnet_gpu_comm_last_levels(const sipnet_gpu_comm *c);
 /* Collective.  Log-likelihoods of the members of all ranks, rank-major: double [sum of member counts]. */
 int sipnet_gpu_comm_gather_loglik(sipnet_gpu_comm *c, double *dst, size_t bytes);
 int sipnet_gpu_comm_member_counts(const sipnet_gpu_comm *c, int64_t *counts /* [nranks] */);
+/* Collective.  sipnet_gpu_assimilate() over the members of ALL ranks: every rank passes the same spec (a mismatch,
+ * found through an all-gathered hash, fails on every rank) and gets the same diag.  Per observation the ranks
+ * all-gather per-site partial sums (2 x 128 B per site) and sum them in rank order, so every rank applies identical
+ * coefficients; no member value leaves its GPU. */
+int sipnet_gpu_comm_assimilate(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, double *diag);
 
 /* (b) one process, one host thread, several GPUs: the single-GPU configuration, partitioned by the library --
  *     whole sites per device when there are at least as many sites as devices, otherwise an even contiguous share
@@ -501,6 +546,9 @@ int sipnet_gpu_multi_reset(sipnet_gpu_multi *m);
 int sipnet_gpu_multi_sync(sipnet_gpu_multi *m);
 int32_t sipnet_gpu_multi_ndevices(const sipnet_gpu_multi *m);
 sipnet_gpu_handle *sipnet_gpu_multi_handle(sipnet_gpu_multi *m, int32_t i); /* device i's handle (owned by m) */
+/* sipnet_gpu_assimilate() on the whole configuration (value / variance / diag in global site order): split sites go
+ * through the team exchange, whole sites are updated by each device alone. */
+int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, double *diag);
 void sipnet_gpu_multi_destroy(sipnet_gpu_multi *m);
 
 #ifdef __cplusplus

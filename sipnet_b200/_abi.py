@@ -138,6 +138,7 @@ ST_BAD_ALLOCATION, ST_RING_OVERFLOW, ST_CLAMPED, ST_DIED, ST_EVREC_OVERFLOW, \
     ST_NONFINITE, ST_REPLAY = 0x1, 0x2, 0x4, 0x8, 0x10, 0x20, 0x40
 ST_BALANCE = 0x80
 ST_LEAFON_LIMITED, ST_N_LIMITED, ST_MINN_LIMITED = 0x100, 0x200, 0x400
+ST_ANALYSIS_FLOORED = 0x800
 NBALANCE = 2
 (CNT_LEAFON_LIMITED, CNT_N_LIMITED, CNT_MINN_LIMITED, CNT_CLAMPED, NCOUNTERS) = range(5)   # sipnet_gpu_counter
 
@@ -186,4 +187,13 @@ class Config(C.Structure):
         ("max_event_records", C.c_int32), ("block_threads", C.c_int32),
         ("stream", C.c_void_p),
         ("ring_slots", C.c_int32),
+    ]
+
+
+class ObsSpec(C.Structure):
+    """sipnet_gpu_obs_spec: what sipnet_gpu_assimilate() fits the pools to."""
+    _fields_ = [
+        ("n_rows", C.c_int32), ("rows", C.POINTER(C.c_int32)),
+        ("n_obs", C.c_int32), ("op", C.POINTER(C.c_double)),
+        ("value", C.POINTER(C.c_double)), ("variance", C.POINTER(C.c_double)),
     ]

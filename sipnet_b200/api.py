@@ -124,6 +124,12 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.sipnet_gpu_multi_handle.argtypes = [C.c_void_p, C.c_int32]
     lib.sipnet_gpu_multi_destroy.restype = None
     lib.sipnet_gpu_multi_destroy.argtypes = [C.c_void_p]
+    lib.sipnet_gpu_assimilate.restype = C.c_int
+    lib.sipnet_gpu_assimilate.argtypes = [C.c_void_p, C.POINTER(A.ObsSpec), C.c_void_p]
+    lib.sipnet_gpu_comm_assimilate.restype = C.c_int
+    lib.sipnet_gpu_comm_assimilate.argtypes = [C.c_void_p, C.POINTER(A.ObsSpec), C.c_void_p]
+    lib.sipnet_gpu_multi_assimilate.restype = C.c_int
+    lib.sipnet_gpu_multi_assimilate.argtypes = [C.c_void_p, C.POINTER(A.ObsSpec), C.c_void_p]
     lib.sipnet_gpu_eval_libm.restype = C.c_int
     lib.sipnet_gpu_eval_libm.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
     if path is None:
@@ -393,6 +399,36 @@ class Ensemble:
         if rc != 0:
             raise SipnetGpuError(rc, (self.lib.sipnet_gpu_last_error() or b"").decode())
 
+    def obs_spec(self, rows, op, value, variance):
+        """(A.ObsSpec, the arrays it points into, n_obs) for sipnet_gpu_*_assimilate.  rows: pool rows (A.S indices
+        0..11); op: [n_obs][n_rows]; value, variance: [nsites][n_obs] (NaN value = not observed)."""
+        rows = np.ascontiguousarray(rows, dtype=np.int32).reshape(-1)
+        op = np.ascontiguousarray(op, dtype=np.float64)
+        value = np.ascontiguousarray(value, dtype=np.float64)
+        variance = np.ascontiguousarray(variance, dtype=np.float64)
+        if op.ndim != 2 or op.shape[1] != rows.size:
+            raise ValueError(f"op must be [n_obs][{rows.size}]")
+        nobs = op.shape[0]
+        if value.shape != (self.nsites, nobs) or variance.shape != value.shape:
+            raise ValueError(f"value and variance must be [{self.nsites}][{nobs}]")
+        spec = A.ObsSpec(rows.size, _ip(rows), nobs, _dp(op), _dp(value), _dp(variance))
+        return spec, (rows, op, value, variance), nobs
+
+    def _assimilate(self, fn, target, rows, op, value, variance) -> np.ndarray:
+        spec, _keep, nobs = self.obs_spec(rows, op, value, variance)
+        diag = np.empty((self.nsites, nobs, 4), np.float64)
+        self._check(fn(target, C.byref(spec), diag.ctypes.data))
+        return diag
+
+    def assimilate(self, rows, op, value, variance) -> np.ndarray:
+        """Ensemble adjustment Kalman filter on the carried pools (sipnet_gpu_assimilate; see include/sipnet_gpu.h).
+        Returns diag [nsites][n_obs][4] = (N, prior mean of y, its sample variance, analysis mean)."""
+        return self._assimilate(self.lib.sipnet_gpu_assimilate, self.handle, rows, op, value, variance)
+
+    def team_assimilate(self, rows, op, value, variance) -> np.ndarray:
+        """Collective.  assimilate() over the members of every rank of the team (same arguments on every rank)."""
+        return self._assimilate(self.lib.sipnet_gpu_comm_assimilate, self.comm, rows, op, value, variance)
+
     def mean(self) -> np.ndarray:
         return self._gather(A.GATHER_MEAN, np.float64, (self.nsites, self.n_summary_cols, self.nrun))
 
@@ -568,6 +604,9 @@ class MultiEnsemble(Ensemble):
         counts = self.event_counts()
         return [[buf[m * self.max_event_records + i] for i in range(min(int(counts[m]), self.max_event_records))]
                 for m in range(self.nmembers)]
+
+    def assimilate(self, rows, op, value, variance) -> np.ndarray:
+        return self._assimilate(self.lib.sipnet_gpu_multi_assimilate, self.multi, rows, op, value, variance)
 
     def sync(self) -> None:
         self.lib.sipnet_gpu_multi_sync(self.multi)

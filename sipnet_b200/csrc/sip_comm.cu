@@ -10,6 +10,8 @@
 //   * one process per GPU (torchrun, MPI, ...): sipnet_gpu_comm_init_rank() with an id made by rank 0 and
 //     broadcast by the caller's launcher;
 //   * one process, one host thread, all GPUs: sipnet_gpu_multi_* (ncclCommInitAll, grouped calls).
+// The host side of the ensemble adjustment Kalman filter lives here too (kernels: sip_assim.cu): a single handle runs
+// it as a team of one, which needs no exchange.
 // NCCL is bound at run time (dlopen of libnccl.so.2): single-GPU use never loads it, and a process that already
 // carries an NCCL (e.g. PyTorch's) shares that copy.
 #include <cuda_runtime.h>
@@ -25,6 +27,7 @@
 #include <string>
 #include <vector>
 
+#include "sip_assim.cuh"
 #include "sip_gsum.cuh"
 #include "sip_handle.h"
 
@@ -104,6 +107,8 @@ struct Local {
   int32_t *flags = nullptr;
   double *llAll = nullptr;  // [nranks][maxMembers] log-likelihood gather
   int64_t llCap = 0;
+  double *asAll = nullptr;  // [nranks][nsites][as::kRec] assimilation partials (rank slot 0 of each also the spec hash)
+  int64_t asCap = 0;        // sites
 };
 
 }  // namespace
@@ -441,6 +446,7 @@ extern "C" void sipnet_gpu_comm_destroy(sipnet_gpu_comm *c) {
       cudaStreamSynchronize(l.h->stream);
     }
     free_local(l);
+    if (l.asAll) cudaFree(l.asAll);
     if (l.comm) nccl_api()->CommDestroy(l.comm);
   }
   if (c->ev0) cudaEventDestroy(c->ev0);
@@ -859,5 +865,233 @@ extern "C" int sipnet_gpu_multi_gather(sipnet_gpu_multi *m, int what, void *dst,
         scatter((size_t)p.siteLocal0[s], (size_t)p.siteGlobal0[s], (size_t)p.siteCount[s]);
     }
   }
+  return 0;
+}
+
+// ---- sequential data assimilation: the ensemble adjustment Kalman filter (sip_assim.cuh) --------------------------
+namespace {
+
+// the spec against `nsites` sites: 0, or SIPNET_GPU_ERR_BAD_ARGUMENT with the reason
+int check_obs(const sipnet_gpu_obs_spec *o, int64_t nsites) {
+  if (!o || !o->rows || !o->op || !o->value || !o->variance)
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL observation spec or array");
+  if (o->n_rows < 1 || o->n_obs < 1) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "n_rows and n_obs must be at least 1");
+  if (o->n_rows > as::kMaxRows) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "at most %d rows", as::kMaxRows);
+  bool seen[as::kMaxRows] = {};
+  for (int j = 0; j < o->n_rows; ++j) {
+    const int32_t r = o->rows[j];
+    if (r < SIPNET_S_plantWoodC || r > SIPNET_S_plantStorageN)
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "state row %d is not a pool the analysis adjusts (0..11)", r);
+    if (seen[r]) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "state row %d listed twice", r);
+    seen[r] = true;
+  }
+  for (int k = 0; k < o->n_obs; ++k) {
+    bool nonzero = false;
+    for (int j = 0; j < o->n_rows; ++j) {
+      const double v = o->op[(size_t)k * o->n_rows + j];
+      if (!std::isfinite(v)) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "op[%d][%d] is not finite", k, j);
+      nonzero = nonzero || v != 0.0;
+    }
+    if (!nonzero) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "op row %d is all zero", k);
+  }
+  for (size_t i = 0; i < (size_t)nsites * (size_t)o->n_obs; ++i) {
+    const double v = o->value[i], r = o->variance[i];
+    if (std::isinf(v)) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "observation value %zu is infinite", i);
+    if (std::isfinite(v) && !(std::isfinite(r) && r > 0.0))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "observation %zu needs a finite variance > 0", i);
+  }
+  return 0;
+}
+
+uint64_t fnv1a(uint64_t h, const void *p, size_t n) {
+  const unsigned char *b = static_cast<const unsigned char *>(p);
+  for (size_t i = 0; i < n; ++i) h = (h ^ b[i]) * 0x100000001b3ull;
+  return h;
+}
+
+uint64_t spec_hash(const sipnet_gpu_obs_spec *o, int64_t nsites) {
+  uint64_t h = 0xcbf29ce484222325ull;
+  const size_t nv = (size_t)nsites * (size_t)o->n_obs;
+  h = fnv1a(h, &o->n_rows, sizeof o->n_rows);
+  h = fnv1a(h, o->rows, (size_t)o->n_rows * sizeof(int32_t));
+  h = fnv1a(h, &o->n_obs, sizeof o->n_obs);
+  h = fnv1a(h, o->op, (size_t)o->n_obs * o->n_rows * sizeof(double));
+  h = fnv1a(h, o->value, nv * sizeof(double));
+  h = fnv1a(h, o->variance, nv * sizeof(double));
+  return h == 0 ? 1 : h;  // 0 stands for an invalid spec
+}
+
+int ensure_as_scratch(sipnet_gpu_comm *c, Local &l) {
+  const int64_t S = l.h->nsites;
+  if (l.asCap >= S) return 0;
+  CUDA_OK(cudaSetDevice(l.h->device));
+  CUDA_OK(cudaStreamSynchronize(l.h->stream));
+  if (l.asAll) cudaFree(l.asAll);
+  l.asAll = nullptr;
+  l.asCap = 0;
+  CUDA_OK(cudaMalloc((void **)&l.asAll, (size_t)c->nranks * S * as::kRec * sizeof(double)));
+  l.asCap = S;
+  return 0;
+}
+
+// Queue the analysis on every local rank of `c`: value / variance hold the handles' sites (all ranks hold the same
+// sites).  A team of one needs no exchange and no host round trip; a larger team all-gathers each pass's per-site
+// partial sums and sums them in rank order on every rank.
+int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const double *value, const double *variance) {
+  const int R = c->nranks, nobs = o->n_obs, nr = o->n_rows;
+  std::vector<as::Args> args(c->local.size());
+  for (size_t i = 0; i < c->local.size(); ++i) {
+    Local &l = c->local[i];
+    sipnet_gpu_handle *h = l.h;
+    if (h->nsites != c->local[0].h->nsites)
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites");
+    CUDA_OK(cudaSetDevice(h->device));
+    if (int rc = as::ensure_scratch(h, nobs)) return rc;
+    if (R > 1)
+      if (int rc = ensure_as_scratch(c, l)) return rc;
+    const size_t nv = (size_t)h->nsites * nobs;
+    CUDA_OK(cudaMemcpyAsync(h->asObs, value, nv * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(cudaMemcpyAsync(h->asObs + nv, variance, nv * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(cudaMemsetAsync(h->asCoef, 0, (size_t)h->nsites * as::kRec * sizeof(double), h->stream));
+    as::Args &a = args[i];
+    memset(&a, 0, sizeof a);
+    a.state = h->state;
+    a.status = h->status;
+    a.ld = h->ld;
+    a.sites = h->sites;
+    a.nsites = (int32_t)h->nsites;
+    a.nchunks = (int32_t)h->asChunks;
+    a.chunk = h->asChunk;
+    a.siteChunks = h->asSiteChunks;
+    a.nrows = nr;
+    a.nobs = nobs;
+    a.nranks = R;
+    a.rank = l.rank;
+    for (int j = 0; j < nr; ++j) a.rows[j] = o->rows[j];
+    a.part = h->asPart;
+    a.mom = h->asMom;
+    a.coef = h->asCoef;
+    a.value = h->asObs;
+    a.variance = h->asObs + nv;
+    a.diag = h->asDiag;
+    a.rankRec = l.asAll;
+  }
+  auto launched = [](sipnet_gpu_handle *h, cudaError_t e) {
+    h->launches++;
+    return e == cudaSuccess ? 0 : fail(SIPNET_GPU_ERR_NO_DEVICE, "assimilation launch failed: %s", cudaGetErrorString(e));
+  };
+  for (int k = 0; k < nobs; ++k) {
+    for (int pass = 1; pass <= 2; ++pass) {
+      for (size_t i = 0; i < c->local.size(); ++i) {
+        as::Args &a = args[i];
+        sipnet_gpu_handle *h = c->local[i].h;
+        a.k = k;
+        for (int j = 0; j < nr; ++j) {
+          a.opCur[j] = o->op[(size_t)k * nr + j];
+          a.opPrev[j] = k > 0 ? o->op[(size_t)(k - 1) * nr + j] : 0.0;
+        }
+        CUDA_OK(cudaSetDevice(h->device));
+        // pass 1 of observation k first applies observation k - 1
+        if (int rc = launched(h, as::launch_members(a, pass, pass == 1 && k > 0, false, h->stream))) return rc;
+        if (int rc = launched(h, as::launch_site_reduce(a, pass, h->stream))) return rc;
+      }
+      if (R > 1) {
+        const size_t bytes = (size_t)args[0].nsites * as::kRec * sizeof(double);
+        if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.asAll; })) return rc;
+        for (size_t i = 0; i < c->local.size(); ++i) {
+          sipnet_gpu_handle *h = c->local[i].h;
+          CUDA_OK(cudaSetDevice(h->device));
+          if (int rc = launched(h, as::launch_site_combine(args[i], pass, h->stream))) return rc;
+        }
+      }
+    }
+  }
+  for (size_t i = 0; i < c->local.size(); ++i) {  // the last observation's update and the floor
+    as::Args &a = args[i];
+    sipnet_gpu_handle *h = c->local[i].h;
+    for (int j = 0; j < nr; ++j) a.opPrev[j] = o->op[(size_t)(nobs - 1) * nr + j];
+    CUDA_OK(cudaSetDevice(h->device));
+    if (int rc = launched(h, as::launch_members(a, 0, true, true, h->stream))) return rc;
+  }
+  return 0;
+}
+
+// wait for the analysis of `h`; diag (may be NULL) gets its [nsites][nobs][4] diagnostics
+int finish_assimilation(sipnet_gpu_handle *h, double *diag, int nobs) {
+  CUDA_OK(cudaSetDevice(h->device));
+  if (diag)
+    CUDA_OK(cudaMemcpyAsync(diag, h->asDiag, (size_t)h->nsites * nobs * 4 * sizeof(double), cudaMemcpyDeviceToHost,
+                            h->stream));
+  CUDA_OK(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
+// one handle alone: a team of one rank (no exchange)
+int assimilate_alone(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *o, const double *value, const double *variance) {
+  sipnet_gpu_comm one;
+  one.local.resize(1);
+  one.local[0].h = h;
+  return run_assimilation(&one, o, value, variance);
+}
+
+}  // namespace
+
+extern "C" int sipnet_gpu_assimilate(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs, double *diag) {
+  if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  if (int rc = check_obs(obs, h->nsites)) return rc;
+  if (int rc = assimilate_alone(h, obs, obs->value, obs->variance)) return rc;
+  return finish_assimilation(h, diag, obs->n_obs);
+}
+
+extern "C" int sipnet_gpu_comm_assimilate(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, double *diag) {
+  if (!c) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL comm");
+  const int64_t S = c->local[0].h->nsites;
+  const int bad = check_obs(obs, S);
+  if (c->nranks > 1) {
+    // every rank sees every rank's spec hash before any rank returns: a bad or differing spec fails on all of them
+    const std::string why = bad ? sipnet_gpu_last_error() : "";
+    const uint64_t mine = bad ? 0 : spec_hash(obs, S);
+    for (Local &l : c->local) {
+      if (int rc = ensure_as_scratch(c, l)) return rc;
+      CUDA_OK(cudaMemcpyAsync(l.asAll + l.rank, &mine, sizeof mine, cudaMemcpyHostToDevice, l.h->stream));
+      CUDA_OK(cudaStreamSynchronize(l.h->stream));
+    }
+    if (int rc = all_gather_bytes(c, sizeof(uint64_t), [](Local &l) -> void * { return l.asAll; })) return rc;
+    std::vector<uint64_t> all((size_t)c->nranks);
+    Local &l0 = c->local[0];
+    CUDA_OK(cudaSetDevice(l0.h->device));
+    CUDA_OK(cudaMemcpyAsync(all.data(), l0.asAll, all.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, l0.h->stream));
+    CUDA_OK(cudaStreamSynchronize(l0.h->stream));
+    for (uint64_t v : all)
+      if (v == 0 || v != all[0]) {
+        if (bad) return fail(bad, "%s", why.c_str());
+        return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of the team passed different or invalid observation specs");
+      }
+  }
+  if (bad) return bad;
+  if (int rc = run_assimilation(c, obs, obs->value, obs->variance)) return rc;
+  for (Local &l : c->local)
+    if (int rc = finish_assimilation(l.h, diag, obs->n_obs)) return rc;
+  return 0;
+}
+
+extern "C" int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, double *diag) {
+  if (!m) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  if (int rc = check_obs(obs, m->nsites)) return rc;
+  const int nobs = obs->n_obs;
+  if (m->split) {  // every device ends with the same diagnostics: take device 0's
+    if (int rc = run_assimilation(m->comm, obs, obs->value, obs->variance)) return rc;
+    for (size_t d = 0; d < m->handles.size(); ++d)
+      if (int rc = finish_assimilation(m->handles[d], d == 0 ? diag : nullptr, nobs)) return rc;
+    return 0;
+  }
+  // whole sites: each device alone on its site range, all devices side by side
+  for (size_t d = 0; d < m->handles.size(); ++d) {
+    const size_t off = (size_t)m->parts[d].site0 * nobs;
+    if (int rc = assimilate_alone(m->handles[d], obs, obs->value + off, obs->variance + off)) return rc;
+  }
+  for (size_t d = 0; d < m->handles.size(); ++d)
+    if (int rc = finish_assimilation(m->handles[d], diag ? diag + (size_t)m->parts[d].site0 * nobs * 4 : nullptr, nobs))
+      return rc;
   return 0;
 }

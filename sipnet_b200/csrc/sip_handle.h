@@ -56,6 +56,11 @@ struct sipnet_gpu_handle {
   std::vector<sip::SiteDev> hostSites;
   bool mixedBlocks = false;          // some block holds members of two sites
   sip::StepConsts kc = {};           // launch-lifetime constants of the step (device-evaluated at init)
+  // ensemble adjustment Kalman filter scratch (sip_assim.cu), made by the first assimilation
+  int64_t asChunks = 0;
+  int asObsCap = 0;
+  int2 *asChunk = nullptr, *asSiteChunks = nullptr;
+  double *asPart = nullptr, *asMom = nullptr, *asCoef = nullptr, *asObs = nullptr, *asDiag = nullptr;
 };
 
 namespace sip {

@@ -343,7 +343,8 @@ static void free_handle(sipnet_gpu_handle *h) {
   void *ptrs[] = {h->params, h->state, h->ringV, h->ringW, h->status, h->memberSite, h->blocks, h->sites, h->out,
                   h->dbg,    h->counters, h->loglik, h->loglikN, h->recs, h->recCount, h->mean, h->var, h->quant,
                   h->stateBk, h->ringVBk, h->ringWBk, h->loglikBk, h->loglikNBk, h->statusBk,
-                  h->recCountBk, h->sched};
+                  h->recCountBk, h->sched, h->asChunk, h->asSiteChunks, h->asPart, h->asMom, h->asCoef,
+                  h->asObs, h->asDiag};
   for (void *p : ptrs)
     if (p) cudaFree(p);
   for (void *p : h->siteAllocs)
