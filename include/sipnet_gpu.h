@@ -431,6 +431,42 @@ typedef struct sipnet_gpu_obs_spec {
 } sipnet_gpu_obs_spec;
 int sipnet_gpu_assimilate(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs, double *diag);
 
+/*
+ * Sequential Monte Carlo: the bootstrap particle filter (Gordon, Salmond & Smith 1993), per site, between two run()
+ * segments.  Members of a site are weighted by a log-weight and replaced by copies of well-weighted members, chosen by
+ * systematic resampling.  A copy carries its parameters with its pools, so forecast -> resample cycles also filter the
+ * parameters.
+ *
+ * Log-weights: l_i = log_weights[i] (host, [nmembers]) when given, else the handle's log-likelihood (needs
+ * SIPNET_GPU_OUT_LOGLIK).  Member i takes part iff its status has neither SIPNET_GPU_ST_BAD_ALLOCATION nor
+ * SIPNET_GPU_ST_NONFINITE and l_i is finite (NaN and -inf: not taking part).  For a site of n members, N >= 1 of them
+ * taking part, lmax = the largest l_i of the participants:
+ *   w_i = exp(l_i - lmax) (glibc-exact exp);  ESS = (sum w)^2 / sum w^2, where both sums are sums of
+ *   floor(x * 2^100) in integers, each converted to double (round to nearest) and scaled by 2^-100;
+ *   the site is resampled iff u[s] is not NaN and ESS < ess_fraction * n (ess_fraction = INFINITY: always).
+ * Ancestors, in integers: W_i = (uint64)(w_i * 2^40) (0 for non-participants); C_i = the exclusive prefix of W in
+ * site-local member order; T = sum W; U = floor(u[s] * 2^32); slot k in [0, n) takes
+ *   t_k = floor(((k * 2^32 + U) * T) / (n * 2^32))
+ * and its ancestor is the i with C_i <= t_k < C_i + W_i.  Ancestors do not decrease with k.  Nothing depends on the
+ * order of a sum, so a site gives the same bits in any partition.
+ *
+ * Every member (slot) of a resampled site, non-participants included, becomes a copy of its ancestor: every device
+ * parameter row (nothing is re-derived), the carried state, both mean-NPP ring rows, the status (without internal
+ * bits), the event count and records (SIPNET_GPU_OUT_EVENTS) and the message counters (SIPNET_GPU_OUT_DEBUG).  Its
+ * log-likelihood and observation count become 0.  Members of other sites, the last run range's outputs and summaries,
+ * and the next step do not change.
+ *
+ * ancestors (may be NULL) receives int64 [nmembers]: the ancestor's member index, -1 where the site was not resampled.
+ * diag (may be NULL) receives double [nsites][4] = {N, ESS, lmax + log(sum w / N) (the incremental log-evidence
+ * estimate), distinct ancestors (0 where not resampled)}; ESS and the log-evidence are NaN where N = 0.
+ *
+ * Rejected with SIPNET_GPU_ERR_BAD_ARGUMENT, nothing changed: NULL handle or u; u[s] neither NaN nor in [0, 1);
+ * ess_fraction NaN or negative; a +inf log-weight; no log_weights on a handle without a log-likelihood; a site of more
+ * than 2^23 members.  Every call returns when the copies are complete.
+ */
+int sipnet_gpu_resample(sipnet_gpu_handle *h, const double *u, double ess_fraction, const double *log_weights,
+                        int64_t *ancestors, double *diag);
+
 /* Slots of the mean-NPP ring this handle uses (config ring_slots, or the automatic choice). */
 int32_t sipnet_gpu_ring_slots(const sipnet_gpu_handle *h);
 
@@ -523,6 +559,13 @@ int sipnet_gpu_comm_member_counts(const sipnet_gpu_comm *c, int64_t *counts /* [
  * all-gather per-site partial sums (2 x 128 B per site) and sum them in rank order, so every rank applies identical
  * coefficients; no member value leaves its GPU. */
 int sipnet_gpu_comm_assimilate(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, double *diag);
+/* Collective.  sipnet_gpu_resample() over the members of ALL ranks, in site-local order rank by rank: u and
+ * ess_fraction are the same on every rank (a mismatch, found through an all-gathered hash, fails on every rank),
+ * log_weights holds the rank's own members.  ancestors receives the team's int64 [sum of member counts], rank-major
+ * (as sipnet_gpu_comm_gather_loglik); every rank gets the same diag.  The ranks exchange two per-site records, then
+ * each source rank sends every destination rank the records of the slots it supplies (NCCL send / receive). */
+int sipnet_gpu_comm_resample(sipnet_gpu_comm *c, const double *u, double ess_fraction, const double *log_weights,
+                             int64_t *ancestors, double *diag);
 
 /* (b) one process, one host thread, several GPUs: the single-GPU configuration, partitioned by the library --
  *     whole sites per device when there are at least as many sites as devices, otherwise an even contiguous share
@@ -549,6 +592,10 @@ sipnet_gpu_handle *sipnet_gpu_multi_handle(sipnet_gpu_multi *m, int32_t i); /* d
 /* sipnet_gpu_assimilate() on the whole configuration (value / variance / diag in global site order): split sites go
  * through the team exchange, whole sites are updated by each device alone. */
 int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, double *diag);
+/* sipnet_gpu_resample() on the whole configuration (u, log_weights, ancestors, diag in configuration order): split
+ * sites go through the team exchange, whole sites are resampled by each device alone. */
+int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, double ess_fraction, const double *log_weights,
+                              int64_t *ancestors, double *diag);
 void sipnet_gpu_multi_destroy(sipnet_gpu_multi *m);
 
 #ifdef __cplusplus

@@ -11,6 +11,7 @@ The names mirror the reference interface this path replaces
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
 import time
 from dataclasses import dataclass, field
@@ -130,6 +131,9 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.sipnet_gpu_comm_assimilate.argtypes = [C.c_void_p, C.POINTER(A.ObsSpec), C.c_void_p]
     lib.sipnet_gpu_multi_assimilate.restype = C.c_int
     lib.sipnet_gpu_multi_assimilate.argtypes = [C.c_void_p, C.POINTER(A.ObsSpec), C.c_void_p]
+    for name in ("sipnet_gpu_resample", "sipnet_gpu_comm_resample", "sipnet_gpu_multi_resample"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.sipnet_gpu_eval_libm.restype = C.c_int
     lib.sipnet_gpu_eval_libm.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
     if path is None:
@@ -429,6 +433,34 @@ class Ensemble:
         """Collective.  assimilate() over the members of every rank of the team (same arguments on every rank)."""
         return self._assimilate(self.lib.sipnet_gpu_comm_assimilate, self.comm, rows, op, value, variance)
 
+    def _resample(self, fn, target, nmembers, u, ess_fraction, log_weights):
+        u = np.ascontiguousarray(u, dtype=np.float64).reshape(-1)
+        if u.size != self.nsites:
+            raise ValueError(f"u must hold one value per site ({self.nsites})")
+        lw = None
+        if log_weights is not None:
+            lw = np.ascontiguousarray(log_weights, dtype=np.float64).reshape(-1)
+            if lw.size != self.nmembers:
+                raise ValueError(f"log_weights must hold one value per member ({self.nmembers})")
+        ancestors = np.empty(nmembers, np.int64)
+        diag = np.empty((self.nsites, 4), np.float64)
+        self._check(fn(target, u.ctypes.data, float(ess_fraction), None if lw is None else lw.ctypes.data,
+                       ancestors.ctypes.data, diag.ctypes.data))
+        return ancestors, diag
+
+    def resample(self, u, ess_fraction: float = math.inf, log_weights=None):
+        """Per-site systematic resampling of the members (sipnet_gpu_resample; see include/sipnet_gpu.h).  u: one
+        value in [0, 1) per site (NaN: leave the site alone); log_weights: [nmembers], or None for the handle's
+        log-likelihood.  Returns (ancestors [nmembers], -1 where a site was not resampled; diag [nsites][4] =
+        (N, ESS, incremental log-evidence, distinct ancestors))."""
+        return self._resample(self.lib.sipnet_gpu_resample, self.handle, self.nmembers, u, ess_fraction, log_weights)
+
+    def team_resample(self, u, ess_fraction: float = math.inf, log_weights=None):
+        """Collective.  resample() over the members of every rank (same u and ess_fraction on every rank;
+        log_weights: this rank's members).  ancestors cover the whole team, rank-major."""
+        n = int(self.team_member_counts().sum())
+        return self._resample(self.lib.sipnet_gpu_comm_resample, self.comm, n, u, ess_fraction, log_weights)
+
     def mean(self) -> np.ndarray:
         return self._gather(A.GATHER_MEAN, np.float64, (self.nsites, self.n_summary_cols, self.nrun))
 
@@ -607,6 +639,9 @@ class MultiEnsemble(Ensemble):
 
     def assimilate(self, rows, op, value, variance) -> np.ndarray:
         return self._assimilate(self.lib.sipnet_gpu_multi_assimilate, self.multi, rows, op, value, variance)
+
+    def resample(self, u, ess_fraction: float = math.inf, log_weights=None):
+        return self._resample(self.lib.sipnet_gpu_multi_resample, self.multi, self.nmembers, u, ess_fraction, log_weights)
 
     def sync(self) -> None:
         self.lib.sipnet_gpu_multi_sync(self.multi)

@@ -10,8 +10,8 @@
 //   * one process per GPU (torchrun, MPI, ...): sipnet_gpu_comm_init_rank() with an id made by rank 0 and
 //     broadcast by the caller's launcher;
 //   * one process, one host thread, all GPUs: sipnet_gpu_multi_* (ncclCommInitAll, grouped calls).
-// The host side of the ensemble adjustment Kalman filter lives here too (kernels: sip_assim.cu): a single handle runs
-// it as a team of one, which needs no exchange.
+// The host sides of the ensemble adjustment Kalman filter (kernels: sip_assim.cu) and of the particle filter
+// (sip_resample.cu) live here too: a single handle runs them as a team of one, which needs no exchange.
 // NCCL is bound at run time (dlopen of libnccl.so.2): single-GPU use never loads it, and a process that already
 // carries an NCCL (e.g. PyTorch's) shares that copy.
 #include <cuda_runtime.h>
@@ -30,6 +30,7 @@
 #include "sip_assim.cuh"
 #include "sip_gsum.cuh"
 #include "sip_handle.h"
+#include "sip_resample.cuh"
 
 using namespace sip;
 
@@ -43,6 +44,8 @@ struct NcclApi {
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
   ncclResult_t (*AllReduce)(const void *, void *, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*AllGather)(const void *, void *, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*Send)(const void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*Recv)(void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*GroupStart)() = nullptr;
   ncclResult_t (*GroupEnd)() = nullptr;
   const char *(*GetErrorString)(ncclResult_t) = nullptr;
@@ -70,6 +73,8 @@ const NcclApi *nccl_api() {
   SIP_BIND(CommDestroy, "ncclCommDestroy")
   SIP_BIND(AllReduce, "ncclAllReduce")
   SIP_BIND(AllGather, "ncclAllGather")
+  SIP_BIND(Send, "ncclSend")
+  SIP_BIND(Recv, "ncclRecv")
   SIP_BIND(GroupStart, "ncclGroupStart")
   SIP_BIND(GroupEnd, "ncclGroupEnd")
   SIP_BIND(GetErrorString, "ncclGetErrorString")
@@ -463,21 +468,22 @@ extern "C" int sipnet_gpu_comm_summaries(sipnet_gpu_comm *c) {
 
 extern "C" int32_t sipnet_gpu_comm_last_levels(const sipnet_gpu_comm *c) { return c ? c->lastLevels : 0; }
 
-// log-likelihoods of every member of the team, rank-major, into each local rank's gather buffer; returns the
-// device pointer of local rank `i`'s copy through `dev` (or copies to `dst` on the host when given)
-static int team_loglik(sipnet_gpu_comm *c, double *dst, size_t bytes, int what) {
+// one 8-byte word per member of the team (`src` of every handle: log-likelihoods, ancestors), rank-major, into each
+// local rank's gather buffer, and to `dst` on the host when given
+static int team_member_words(sipnet_gpu_comm *c, void *dst, size_t bytes, const void *(*src)(const sipnet_gpu_handle *),
+                             const char *what) {
   int64_t total = 0, width = 0;
   for (int64_t m : c->memberCounts) {
     total += m;
     width = std::max(width, m);
   }
   if (dst && bytes != (size_t)total * sizeof(double))
-    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "log-likelihood gather: buffer is %zu bytes, expected %zu", bytes,
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "%s gather: buffer is %zu bytes, expected %zu", what, bytes,
                 (size_t)total * sizeof(double));
   for (Local &l : c->local) {
     sipnet_gpu_handle *h = l.h;
-    const double *src = what == SIPNET_GPU_GATHER_LOGLIK ? h->loglik : h->loglikN;
-    if (!src) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "log-likelihood output was not requested at init");
+    const void *from = src(h);
+    if (!from) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "%s output was not requested at init", what);
     CUDA_OK(cudaSetDevice(h->device));
     if (l.llCap < width) {
       if (l.llAll) cudaFree(l.llAll);
@@ -485,7 +491,7 @@ static int team_loglik(sipnet_gpu_comm *c, double *dst, size_t bytes, int what) 
       CUDA_OK(cudaMalloc((void **)&l.llAll, (size_t)c->nranks * width * sizeof(double)));
       l.llCap = width;
     }
-    CUDA_OK(cudaMemcpyAsync(l.llAll + (size_t)l.rank * width, src, (size_t)h->nmembers * sizeof(double),
+    CUDA_OK(cudaMemcpyAsync(l.llAll + (size_t)l.rank * width, from, (size_t)h->nmembers * sizeof(double),
                             cudaMemcpyDeviceToDevice, h->stream));
   }
   if (int rc = all_gather_bytes(c, (size_t)width * sizeof(double), [](Local &l) -> void * { return l.llAll; })) return rc;
@@ -494,7 +500,7 @@ static int team_loglik(sipnet_gpu_comm *c, double *dst, size_t bytes, int what) 
     CUDA_OK(cudaSetDevice(l.h->device));
     int64_t off = 0;
     for (int q = 0; q < c->nranks; ++q) {
-      CUDA_OK(cudaMemcpyAsync(dst + off, l.llAll + (size_t)q * width, (size_t)c->memberCounts[(size_t)q] * sizeof(double),
+      CUDA_OK(cudaMemcpyAsync(static_cast<double *>(dst) + off, l.llAll + (size_t)q * width, (size_t)c->memberCounts[(size_t)q] * sizeof(double),
                               cudaMemcpyDeviceToHost, l.h->stream));
       off += c->memberCounts[(size_t)q];
     }
@@ -510,7 +516,8 @@ static int team_loglik(sipnet_gpu_comm *c, double *dst, size_t bytes, int what) 
 
 extern "C" int sipnet_gpu_comm_gather_loglik(sipnet_gpu_comm *c, double *dst, size_t bytes) {
   if (!c || !dst) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL comm or destination");
-  return team_loglik(c, dst, bytes, SIPNET_GPU_GATHER_LOGLIK);
+  return team_member_words(c, dst, bytes, [](const sipnet_gpu_handle *h) -> const void * { return h->loglik; },
+                           "log-likelihood");
 }
 
 extern "C" int sipnet_gpu_comm_member_counts(const sipnet_gpu_comm *c, int64_t *counts) {
@@ -1043,32 +1050,35 @@ extern "C" int sipnet_gpu_assimilate(sipnet_gpu_handle *h, const sipnet_gpu_obs_
   return finish_assimilation(h, diag, obs->n_obs);
 }
 
+// Collective: every rank sees every rank's argument hash (`mine`; 0 = this rank's arguments are invalid, with the
+// reason in the last error) before any rank returns, so a bad or differing argument fails on all of them.
+static int team_agree(sipnet_gpu_comm *c, int bad, uint64_t mine, const char *what) {
+  if (c->nranks == 1) return bad;
+  const std::string why = bad ? sipnet_gpu_last_error() : "";
+  for (Local &l : c->local) {
+    if (int rc = ensure_as_scratch(c, l)) return rc;
+    CUDA_OK(cudaMemcpyAsync(l.asAll + l.rank, &mine, sizeof mine, cudaMemcpyHostToDevice, l.h->stream));
+    CUDA_OK(cudaStreamSynchronize(l.h->stream));
+  }
+  if (int rc = all_gather_bytes(c, sizeof(uint64_t), [](Local &l) -> void * { return l.asAll; })) return rc;
+  std::vector<uint64_t> all((size_t)c->nranks);
+  Local &l0 = c->local[0];
+  CUDA_OK(cudaSetDevice(l0.h->device));
+  CUDA_OK(cudaMemcpyAsync(all.data(), l0.asAll, all.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, l0.h->stream));
+  CUDA_OK(cudaStreamSynchronize(l0.h->stream));
+  for (uint64_t v : all)
+    if (v == 0 || v != all[0]) {
+      if (bad) return fail(bad, "%s", why.c_str());
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of the team passed different or invalid %s", what);
+    }
+  return bad;
+}
+
 extern "C" int sipnet_gpu_comm_assimilate(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, double *diag) {
   if (!c) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL comm");
   const int64_t S = c->local[0].h->nsites;
   const int bad = check_obs(obs, S);
-  if (c->nranks > 1) {
-    // every rank sees every rank's spec hash before any rank returns: a bad or differing spec fails on all of them
-    const std::string why = bad ? sipnet_gpu_last_error() : "";
-    const uint64_t mine = bad ? 0 : spec_hash(obs, S);
-    for (Local &l : c->local) {
-      if (int rc = ensure_as_scratch(c, l)) return rc;
-      CUDA_OK(cudaMemcpyAsync(l.asAll + l.rank, &mine, sizeof mine, cudaMemcpyHostToDevice, l.h->stream));
-      CUDA_OK(cudaStreamSynchronize(l.h->stream));
-    }
-    if (int rc = all_gather_bytes(c, sizeof(uint64_t), [](Local &l) -> void * { return l.asAll; })) return rc;
-    std::vector<uint64_t> all((size_t)c->nranks);
-    Local &l0 = c->local[0];
-    CUDA_OK(cudaSetDevice(l0.h->device));
-    CUDA_OK(cudaMemcpyAsync(all.data(), l0.asAll, all.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, l0.h->stream));
-    CUDA_OK(cudaStreamSynchronize(l0.h->stream));
-    for (uint64_t v : all)
-      if (v == 0 || v != all[0]) {
-        if (bad) return fail(bad, "%s", why.c_str());
-        return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of the team passed different or invalid observation specs");
-      }
-  }
-  if (bad) return bad;
+  if (int rc = team_agree(c, bad, bad ? 0 : spec_hash(obs, S), "observation specs")) return rc;
   if (int rc = run_assimilation(c, obs, obs->value, obs->variance)) return rc;
   for (Local &l : c->local)
     if (int rc = finish_assimilation(l.h, diag, obs->n_obs)) return rc;
@@ -1093,5 +1103,421 @@ extern "C" int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu
   for (size_t d = 0; d < m->handles.size(); ++d)
     if (int rc = finish_assimilation(m->handles[d], diag ? diag + (size_t)m->parts[d].site0 * nobs * 4 : nullptr, nobs))
       return rc;
+  return 0;
+}
+
+// ---- the particle filter: per-site systematic resampling (sip_resample.cuh) ---------------------------------------
+namespace {
+
+typedef unsigned __int128 u128;
+
+int check_resample(const sipnet_gpu_handle *h, const double *u, int64_t nsites, double essFraction, const double *logw) {
+  if (!u) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL u");
+  if (std::isnan(essFraction) || essFraction < 0.0)
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "ess_fraction must be >= 0 (INFINITY: always resample)");
+  for (int64_t s = 0; s < nsites; ++s)
+    if (!std::isnan(u[s]) && !(u[s] >= 0.0 && u[s] < 1.0))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "u[%lld] = %g is neither NaN nor in [0, 1)", (long long)s, u[s]);
+  if (!logw && !h->loglik)
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "no log_weights, and the handle keeps no log-likelihood (SIPNET_GPU_OUT_LOGLIK)");
+  return 0;
+}
+
+// K(C): the first slot k with t_k >= C, i.e. clamp(ceil((ceil(C n 2^32 / T) - U) / 2^32), 0, n)
+int64_t first_slot(uint64_t C, uint64_t T, uint64_t U, int64_t n) {
+  const u128 a = ((((u128)C * (uint64_t)n) << 32) + T - 1) / T;
+  if (a <= U) return 0;
+  const u128 k = (a - U + 0xffffffffu) >> 32;
+  return k < (u128)n ? (int64_t)k : n;
+}
+
+// every rank's per-site record of the last site pass, rank-major, on the host
+int site_records(sipnet_gpu_comm *c, std::vector<uint64_t> &out) {
+  const size_t S = (size_t)c->local[0].h->nsites;
+  if (int rc = all_gather_bytes(c, S * rs::kRec * sizeof(uint64_t), [](Local &l) -> void * { return l.h->rsSite; }))
+    return rc;
+  Local &l0 = c->local[0];
+  out.resize((size_t)c->nranks * S * rs::kRec);
+  CUDA_OK(cudaSetDevice(l0.h->device));
+  CUDA_OK(cudaMemcpyAsync(out.data(), l0.h->rsSite, out.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, l0.h->stream));
+  CUDA_OK(cudaStreamSynchronize(l0.h->stream));
+  return 0;
+}
+
+template <class T>
+int grow(T *&p, size_t &cap, size_t need, cudaStream_t stream) {
+  if (need <= cap && p) return 0;
+  CUDA_OK(cudaStreamSynchronize(stream));
+  if (p) cudaFree(p);
+  p = nullptr;
+  cap = 0;
+  CUDA_OK(cudaMalloc((void **)&p, std::max<size_t>(need, 1) * sizeof(T)));
+  cap = std::max<size_t>(need, 1);
+  return 0;
+}
+
+// this rank's part of the copy: segment sizes (records) and where they sit (doubles)
+struct CopyPlan {
+  std::vector<int64_t> tab;
+  std::vector<int64_t> sendCnt, sendBase, recvCnt, recvBase;
+};
+
+// Resample every local rank of `c` (all ranks hold the same sites): logw[i] is local rank i's host log-weights or
+// NULL (its log-likelihood).  diag (may be NULL) gets [nsites][4]; ancAll the team's ancestors, rank-major.
+int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const std::vector<const double *> &logw,
+                 double *diag, std::vector<int64_t> &ancAll) {
+  const int R = c->nranks;
+  const int64_t S = c->local[0].h->nsites;
+  const int words = rs::record_words(c->local[0].h);
+  const size_t L = c->local.size();
+  std::vector<rs::Args> args(L);
+  auto launched = [](sipnet_gpu_handle *h, cudaError_t e) {
+    h->launches++;
+    return e == cudaSuccess ? 0 : fail(SIPNET_GPU_ERR_NO_DEVICE, "resampling launch failed: %s", cudaGetErrorString(e));
+  };
+  std::vector<int64_t> rankBase((size_t)R + 1, 0);
+  for (int q = 0; q < R; ++q) rankBase[(size_t)q + 1] = rankBase[(size_t)q] + c->memberCounts[(size_t)q];
+  for (size_t i = 0; i < L; ++i) {
+    Local &l = c->local[i];
+    sipnet_gpu_handle *h = l.h;
+    if (h->nsites != S || rs::record_words(h) != words)
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites and outputs");
+    CUDA_OK(cudaSetDevice(h->device));
+    if (int rc = rs::ensure_scratch(h)) return rc;
+    if (int rc = grow(h->rsSite, h->rsSiteCap, (size_t)R * S * rs::kRec, h->stream)) return rc;
+    if (logw[i])
+      CUDA_OK(cudaMemcpyAsync(h->rsLogw, logw[i], (size_t)h->nmembers * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    rs::Args &a = args[i];
+    memset(&a, 0, sizeof a);
+    a.logw = logw[i] ? h->rsLogw : h->loglik;
+    a.status = h->status;
+    a.sites = h->sites;
+    a.memberSite = h->memberSite;
+    a.nmembers = h->nmembers;
+    a.ld = h->ld;
+    a.nsites = (int32_t)S;
+    a.nchunks = (int32_t)h->asChunks;
+    a.chunk = h->asChunk;
+    a.siteChunks = h->asSiteChunks;
+    a.params = h->params;
+    a.state = h->state;
+    a.ringV = h->ringV;
+    a.ringW = h->ringW;
+    a.loglik = h->loglik;
+    a.loglikN = h->loglikN;
+    a.counters = h->counters;
+    a.recs = h->recs;
+    a.recCount = h->recCount;
+    a.ringCap = h->ringCap;
+    a.maxRecs = h->maxRecs;
+    a.words = words;
+    a.nranks = R;
+    a.rank = l.rank;
+    a.idBase = rankBase[(size_t)l.rank];
+    a.part = reinterpret_cast<uint64_t *>(h->asPart);
+    a.w = h->rsW;
+    a.c = h->rsC;
+    a.siteRec = h->rsSite;
+    a.lmax = h->rsLmax;
+    a.anc = h->rsAnc;
+    if (int rc = launched(h, rs::launch_weights(a, 0, h->stream))) return rc;
+    if (int rc = launched(h, rs::launch_site(a, 0, h->stream))) return rc;
+  }
+  // pass a over the ranks: participants, members and the largest log-weight of every site
+  std::vector<uint64_t> recA, recB;
+  if (int rc = site_records(c, recA)) return rc;
+  std::vector<double> lmax((size_t)S, -INFINITY);
+  std::vector<int64_t> N((size_t)S, 0), n((size_t)S, 0);
+  for (int r = 0; r < R; ++r)
+    for (int64_t s = 0; s < S; ++s) {
+      const uint64_t *p = &recA[((size_t)r * S + s) * rs::kRec];
+      if (p[3]) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "a log-weight of site %lld is +inf", (long long)s);
+      N[(size_t)s] += (int64_t)p[0];
+      n[(size_t)s] += (int64_t)p[2];
+      double v;
+      memcpy(&v, &p[1], sizeof v);
+      if (p[0]) lmax[(size_t)s] = std::max(lmax[(size_t)s], v);
+    }
+  for (int64_t s = 0; s < S; ++s)
+    if (n[(size_t)s] > rs::kMaxSiteMembers)
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "site %lld has %lld members; resampling takes at most 2^23 per site",
+                  (long long)s, (long long)n[(size_t)s]);
+  for (size_t i = 0; i < L; ++i) {
+    sipnet_gpu_handle *h = c->local[i].h;
+    CUDA_OK(cudaSetDevice(h->device));
+    CUDA_OK(cudaMemcpyAsync(h->rsLmax, lmax.data(), (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    if (int rc = launched(h, rs::launch_weights(args[i], 1, h->stream))) return rc;
+    if (int rc = launched(h, rs::launch_site(args[i], 1, h->stream))) return rc;
+  }
+  // pass b over the ranks: ESS, the decision and the slot ranges of every site (integer sums: any order, same bits)
+  if (int rc = site_records(c, recB)) return rc;
+  const size_t R1 = (size_t)R + 1;
+  std::vector<int64_t> flag((size_t)S, 0), U((size_t)S, 0), T((size_t)S, 0), slot0((size_t)S * R1, 0), mem0((size_t)S * R1, 0);
+  std::vector<uint64_t> toff((size_t)S * R1, 0);
+  std::vector<double> dg((size_t)S * 4, 0.0);
+  for (int64_t s = 0; s < S; ++s) {
+    u128 f1 = 0, f2 = 0;
+    for (int r = 0; r < R; ++r) {
+      const uint64_t *p = &recB[((size_t)r * S + s) * rs::kRec];
+      f1 += (u128)p[1] << 64 | p[0];
+      f2 += (u128)p[3] << 64 | p[2];
+      toff[(size_t)s * R1 + r + 1] = toff[(size_t)s * R1 + r] + p[4];
+      mem0[(size_t)s * R1 + r + 1] = mem0[(size_t)s * R1 + r] + (int64_t)recA[((size_t)r * S + s) * rs::kRec + 2];
+    }
+    double *d = &dg[(size_t)s * 4];
+    d[0] = (double)N[(size_t)s];
+    d[1] = d[2] = __builtin_nan("");
+    if (N[(size_t)s] == 0) continue;
+    const double s1 = std::ldexp((double)f1, -rs::kFixBits), s2 = std::ldexp((double)f2, -rs::kFixBits);
+    d[1] = s1 * s1 / s2;
+    d[2] = lmax[(size_t)s] + std::log(s1 / (double)N[(size_t)s]);
+    if (std::isnan(u[s]) || !(d[1] < essFraction * (double)n[(size_t)s])) continue;
+    flag[(size_t)s] = 1;
+    U[(size_t)s] = (int64_t)(uint64_t)std::ldexp(u[s], 32);
+    T[(size_t)s] = (int64_t)toff[(size_t)s * R1 + R];
+    for (size_t p = 0; p <= (size_t)R; ++p)
+      slot0[(size_t)s * R1 + p] = first_slot(toff[(size_t)s * R1 + p], (uint64_t)T[(size_t)s], (uint64_t)U[(size_t)s], n[(size_t)s]);
+  }
+  // records travelling from rank p to rank q for site s
+  auto count = [&](int p, int q, int64_t s) {
+    const int64_t *a = &slot0[(size_t)s * R1], *b = &mem0[(size_t)s * R1];
+    return std::max<int64_t>(0, std::min(a[p + 1], b[q + 1]) - std::max(a[p], b[q]));
+  };
+  std::vector<CopyPlan> plan(L);
+  for (size_t i = 0; i < L; ++i) {
+    Local &l = c->local[i];
+    sipnet_gpu_handle *h = l.h;
+    const int r = l.rank;
+    CopyPlan &P = plan[i];
+    P.sendCnt.assign((size_t)R, 0);
+    P.recvCnt.assign((size_t)R, 0);
+    P.sendBase.assign((size_t)R, 0);
+    P.recvBase.assign((size_t)R, 0);
+    std::vector<int64_t> sendPos((size_t)S * R), recvPos((size_t)S * R), outPre((size_t)S + 1, 0), rtoff((size_t)S);
+    for (int64_t s = 0; s < S; ++s) {
+      for (int q = 0; q < R; ++q) {
+        sendPos[(size_t)s * R + q] = P.sendCnt[(size_t)q];
+        P.sendCnt[(size_t)q] += count(r, q, s);
+        recvPos[(size_t)s * R + q] = P.recvCnt[(size_t)q];
+        P.recvCnt[(size_t)q] += count(q, r, s);
+      }
+      outPre[(size_t)s + 1] = outPre[(size_t)s] + slot0[(size_t)s * R1 + r + 1] - slot0[(size_t)s * R1 + r];
+      rtoff[(size_t)s] = (int64_t)toff[(size_t)s * R1 + r];
+    }
+    size_t sendWords = 0, recvWords = 0;
+    for (int q = 0; q < R; ++q) {
+      P.sendBase[(size_t)q] = (int64_t)sendWords;
+      sendWords += (size_t)P.sendCnt[(size_t)q] * words;
+      if (q == r) continue;
+      P.recvBase[(size_t)q] = (int64_t)recvWords;
+      recvWords += (size_t)P.recvCnt[(size_t)q] * words;
+    }
+    CUDA_OK(cudaSetDevice(h->device));
+    if (int rc = grow(h->rsSend, h->rsSendCap, sendWords, h->stream)) return rc;
+    if (int rc = grow(h->rsRecv, h->rsRecvCap, recvWords, h->stream)) return rc;
+    std::vector<int64_t> src((size_t)R);
+    for (int p = 0; p < R; ++p)
+      src[(size_t)p] = reinterpret_cast<int64_t>(p == r ? h->rsSend + P.sendBase[(size_t)r] : h->rsRecv + P.recvBase[(size_t)p]);
+    std::vector<int64_t> &tab = P.tab;
+    std::vector<size_t> at;
+    for (const std::vector<int64_t> *v : {&flag, &U, &T, &n, &rtoff, &slot0, &mem0, &sendPos, &recvPos, &outPre, &P.sendBase,
+                                          &P.sendCnt, &P.recvCnt, &src}) {
+      at.push_back(tab.size());
+      tab.insert(tab.end(), v->begin(), v->end());
+    }
+    if (int rc = grow(h->rsTab, h->rsTabCap, tab.size(), h->stream)) return rc;
+    CUDA_OK(cudaMemcpyAsync(h->rsTab, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
+    rs::Args &a = args[i];
+    const int64_t *t = h->rsTab;
+    a.flag = t + at[0];
+    a.U = t + at[1];
+    a.T = t + at[2];
+    a.n = t + at[3];
+    a.toff = t + at[4];
+    a.slot0 = t + at[5];
+    a.mem0 = t + at[6];
+    a.sendPos = t + at[7];
+    a.recvPos = t + at[8];
+    a.outPre = t + at[9];
+    a.sendBase = t + at[10];
+    a.sendCnt = t + at[11];
+    a.recvCnt = t + at[12];
+    a.src = reinterpret_cast<double *const *>(t + at[13]);
+    a.sendBuf = h->rsSend;
+    a.nOut = outPre[(size_t)S];
+    if (int rc = launched(h, rs::launch_prefix(a, h->stream))) return rc;
+    if (int rc = launched(h, rs::launch_pack(a, h->stream))) return rc;
+  }
+  // the segments between ranks
+  if (R > 1 && c->loopback) {
+    if (int rc = sync_all(c)) return rc;
+    for (size_t i = 0; i < L; ++i)
+      for (size_t j = 0; j < L; ++j) {
+        const int p = c->local[j].rank, q = c->local[i].rank;
+        const int64_t cnt = plan[i].recvCnt[(size_t)p];
+        if (p == q || cnt == 0) continue;
+        CUDA_OK(cudaMemcpyAsync(c->local[i].h->rsRecv + plan[i].recvBase[(size_t)p],
+                                c->local[j].h->rsSend + plan[j].sendBase[(size_t)q], (size_t)cnt * words * sizeof(double),
+                                cudaMemcpyDeviceToDevice, c->local[i].h->stream));
+      }
+    if (int rc = sync_all(c)) return rc;
+  } else if (R > 1) {  // send and receive of one pair must sit in one group
+    NCCL_OK(nccl_api()->GroupStart());
+    for (size_t i = 0; i < L; ++i) {
+      Local &l = c->local[i];
+      CUDA_OK(cudaSetDevice(l.h->device));
+      for (int q = 0; q < R; ++q) {
+        if (q == l.rank) continue;
+        if (const int64_t cnt = plan[i].sendCnt[(size_t)q])
+          NCCL_OK(nccl_api()->Send(l.h->rsSend + plan[i].sendBase[(size_t)q], (size_t)cnt * words * sizeof(double), ncclUint8,
+                                   q, l.comm, l.h->stream));
+        if (const int64_t cnt = plan[i].recvCnt[(size_t)q])
+          NCCL_OK(nccl_api()->Recv(l.h->rsRecv + plan[i].recvBase[(size_t)q], (size_t)cnt * words * sizeof(double), ncclUint8,
+                                   q, l.comm, l.h->stream));
+      }
+    }
+    NCCL_OK(nccl_api()->GroupEnd());
+  }
+  for (size_t i = 0; i < L; ++i) {
+    sipnet_gpu_handle *h = c->local[i].h;
+    CUDA_OK(cudaSetDevice(h->device));
+    if (int rc = launched(h, rs::launch_unpack(args[i], h->stream))) return rc;
+  }
+  // the ancestors of the whole team, and the distinct ancestors of every resampled site
+  ancAll.assign((size_t)rankBase[(size_t)R], -1);
+  if (R == 1) {
+    sipnet_gpu_handle *h = c->local[0].h;
+    CUDA_OK(cudaMemcpyAsync(ancAll.data(), h->rsAnc, ancAll.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_OK(cudaStreamSynchronize(h->stream));
+  } else if (int rc = team_member_words(c, ancAll.data(), ancAll.size() * sizeof(int64_t),
+                                        [](const sipnet_gpu_handle *h) -> const void * { return h->rsAnc; }, "ancestor")) {
+    return rc;
+  }
+  std::vector<int64_t> last((size_t)S, -1);
+  for (int r = 0; r < R; ++r) {
+    const int64_t *a = ancAll.data() + rankBase[(size_t)r];
+    for (int64_t s = 0; s < S; ++s) {  // a rank's members are in site order
+      const int64_t cnt = (int64_t)recA[((size_t)r * S + s) * rs::kRec + 2];
+      for (int64_t k = 0; k < cnt; ++k, ++a)
+        if (*a >= 0 && *a != last[(size_t)s]) {
+          dg[(size_t)s * 4 + 3] += 1.0;
+          last[(size_t)s] = *a;
+        }
+    }
+  }
+  if (diag) memcpy(diag, dg.data(), dg.size() * sizeof(double));
+  return 0;
+}
+
+}  // namespace
+
+extern "C" int sipnet_gpu_resample(sipnet_gpu_handle *h, const double *u, double ess_fraction, const double *log_weights,
+                                   int64_t *ancestors, double *diag) {
+  if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  if (int rc = check_resample(h, u, h->nsites, ess_fraction, log_weights)) return rc;
+  sipnet_gpu_comm one;
+  one.local.resize(1);
+  one.local[0].h = h;
+  one.memberCounts.assign(1, h->nmembers);
+  std::vector<int64_t> anc;
+  if (int rc = run_resample(&one, u, ess_fraction, {log_weights}, diag, anc)) return rc;
+  if (ancestors) memcpy(ancestors, anc.data(), anc.size() * sizeof(int64_t));
+  return 0;
+}
+
+extern "C" int sipnet_gpu_comm_resample(sipnet_gpu_comm *c, const double *u, double ess_fraction, const double *log_weights,
+                                        int64_t *ancestors, double *diag) {
+  if (!c) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL comm");
+  sipnet_gpu_handle *h = c->local[0].h;
+  const int64_t S = h->nsites;
+  const int bad = check_resample(h, u, S, ess_fraction, log_weights);
+  uint64_t hash = 0;
+  if (!bad) {
+    const int64_t words = rs::record_words(h);
+    hash = fnv1a(0xcbf29ce484222325ull, &S, sizeof S);
+    hash = fnv1a(hash, &words, sizeof words);
+    hash = fnv1a(hash, &ess_fraction, sizeof ess_fraction);
+    hash = fnv1a(hash, u, (size_t)S * sizeof(double));
+    hash = hash == 0 ? 1 : hash;
+  }
+  if (int rc = team_agree(c, bad, hash, "resampling arguments")) return rc;
+  std::vector<int64_t> anc;
+  if (int rc = run_resample(c, u, ess_fraction, std::vector<const double *>(c->local.size(), log_weights), diag, anc))
+    return rc;
+  if (ancestors) memcpy(ancestors, anc.data(), anc.size() * sizeof(int64_t));
+  return 0;
+}
+
+extern "C" int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, double ess_fraction, const double *log_weights,
+                                         int64_t *ancestors, double *diag) {
+  if (!m) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  if (int rc = check_resample(m->handles[0], u, m->nsites, ess_fraction, log_weights)) return rc;
+  const size_t D = m->handles.size();
+  // configuration index of every device's members
+  std::vector<std::vector<int64_t>> glob(D);
+  for (size_t d = 0; d < D; ++d) {
+    const sipnet_gpu_multi::Part &p = m->parts[d];
+    glob[d].resize((size_t)m->handles[d]->nmembers);
+    if (!m->split) {
+      std::iota(glob[d].begin(), glob[d].end(), p.member0);
+    } else {
+      for (size_t s = 0; s < p.siteCount.size(); ++s)
+        for (int64_t i = 0; i < p.siteCount[s]; ++i) glob[d][(size_t)(p.siteLocal0[s] + i)] = p.siteGlobal0[s] + i;
+    }
+  }
+  // the log-weights per device, checked here: a device must not resample before another one rejects the call
+  std::vector<double> all;
+  if (!log_weights) {
+    all.resize((size_t)m->nmembers);
+    if (int rc = sipnet_gpu_multi_gather(m, SIPNET_GPU_GATHER_LOGLIK, all.data(), all.size() * sizeof(double))) return rc;
+    log_weights = all.data();
+  }
+  for (int64_t i = 0; i < m->nmembers; ++i)
+    if (log_weights[i] == INFINITY) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "log_weights[%lld] is +inf", (long long)i);
+  std::vector<int64_t> siteN((size_t)m->nsites, 0);
+  for (size_t d = 0; d < D; ++d)
+    for (size_t s = 0; s < m->handles[d]->hostSites.size(); ++s)
+      siteN[(size_t)m->parts[d].site0 + s] += m->handles[d]->hostSites[s].memberCount;
+  for (int64_t s = 0; s < m->nsites; ++s)
+    if (siteN[(size_t)s] > rs::kMaxSiteMembers)
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "site %lld has %lld members; resampling takes at most 2^23 per site",
+                  (long long)s, (long long)siteN[(size_t)s]);
+  std::vector<std::vector<double>> lw(D);
+  for (size_t d = 0; d < D; ++d) {
+    lw[d].resize(glob[d].size());
+    for (size_t j = 0; j < glob[d].size(); ++j) lw[d][j] = log_weights[glob[d][j]];
+  }
+  std::vector<int64_t> anc;
+  if (m->split) {
+    std::vector<const double *> ptrs;
+    for (size_t d = 0; d < D; ++d) ptrs.push_back(lw[d].data());
+    if (int rc = run_resample(m->comm, u, ess_fraction, ptrs, diag, anc)) return rc;
+    if (ancestors) {  // rank-major -> configuration order
+      std::vector<int64_t> base(D + 1, 0);
+      for (size_t d = 0; d < D; ++d) base[d + 1] = base[d] + m->handles[d]->nmembers;
+      for (size_t d = 0; d < D; ++d)
+        for (size_t j = 0; j < glob[d].size(); ++j) {
+          const int64_t v = anc[(size_t)base[d] + j];
+          int64_t g = -1;
+          if (v >= 0) {
+            const size_t q = (size_t)(std::upper_bound(base.begin(), base.end(), v) - base.begin()) - 1;
+            g = glob[q][(size_t)(v - base[q])];
+          }
+          ancestors[glob[d][j]] = g;
+        }
+    }
+    return 0;
+  }
+  // whole sites: each device alone on its site range
+  for (size_t d = 0; d < D; ++d) {
+    sipnet_gpu_comm one;
+    one.local.resize(1);
+    one.local[0].h = m->handles[d];
+    one.memberCounts.assign(1, m->handles[d]->nmembers);
+    const size_t s0 = (size_t)m->parts[d].site0;
+    if (int rc = run_resample(&one, u + s0, ess_fraction, {lw[d].data()}, diag ? diag + s0 * 4 : nullptr, anc)) return rc;
+    if (ancestors)
+      for (size_t j = 0; j < glob[d].size(); ++j) ancestors[glob[d][j]] = anc[j] < 0 ? -1 : glob[d][(size_t)anc[j]];
+  }
   return 0;
 }

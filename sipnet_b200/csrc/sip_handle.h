@@ -61,6 +61,11 @@ struct sipnet_gpu_handle {
   int asObsCap = 0;
   int2 *asChunk = nullptr, *asSiteChunks = nullptr;
   double *asPart = nullptr, *asMom = nullptr, *asCoef = nullptr, *asObs = nullptr, *asDiag = nullptr;
+  // particle filter scratch (sip_resample.cu), made by the first resampling; the tables and the record buffers grow
+  uint64_t *rsW = nullptr, *rsC = nullptr, *rsSite = nullptr;
+  double *rsLogw = nullptr, *rsLmax = nullptr, *rsSend = nullptr, *rsRecv = nullptr;
+  int64_t *rsAnc = nullptr, *rsTab = nullptr;
+  size_t rsSiteCap = 0, rsTabCap = 0, rsSendCap = 0, rsRecvCap = 0;  // elements
 };
 
 namespace sip {

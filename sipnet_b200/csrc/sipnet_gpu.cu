@@ -344,7 +344,8 @@ static void free_handle(sipnet_gpu_handle *h) {
                   h->dbg,    h->counters, h->loglik, h->loglikN, h->recs, h->recCount, h->mean, h->var, h->quant,
                   h->stateBk, h->ringVBk, h->ringWBk, h->loglikBk, h->loglikNBk, h->statusBk,
                   h->recCountBk, h->sched, h->asChunk, h->asSiteChunks, h->asPart, h->asMom, h->asCoef,
-                  h->asObs, h->asDiag};
+                  h->asObs, h->asDiag, h->rsW, h->rsC, h->rsSite, h->rsLogw, h->rsLmax, h->rsSend, h->rsRecv,
+                  h->rsAnc, h->rsTab};
   for (void *p : ptrs)
     if (p) cudaFree(p);
   for (void *p : h->siteAllocs)
