@@ -282,9 +282,14 @@ enum sipnet_gpu_gather_what {
   SIPNET_GPU_GATHER_RING_WEIGHTS = 13, /* double [ring_slots][M]: MeanTracker.weights */
   SIPNET_GPU_GATHER_BALANCE = 14,      /* double [SIPNET_GPU_NBALANCE][n][M]: deltaC, deltaN of the mass-balance check
                                           (needs SIPNET_GPU_OUT_DEBUG) */
-  SIPNET_GPU_GATHER_COUNTERS = 15      /* uint32 [SIPNET_GPU_NCOUNTERS][M]: how often, since init / reset, the reference
+  SIPNET_GPU_GATHER_COUNTERS = 15,     /* uint32 [SIPNET_GPU_NCOUNTERS][M]: how often, since init / reset, the reference
                                           would have printed each of its informational messages for the member
                                           (SIPNET_GPU_CNT_* order; needs SIPNET_GPU_OUT_DEBUG) */
+  SIPNET_GPU_GATHER_PARAMS = 16        /* double [SIPNET_GPU_NPARAMS][M]: the device's parameter rows, in device units:
+                                          the values after setupModel() -- the nine rates it divides by 365 are per
+                                          day, psnTMax and coarseRootAllocation are derived, fAnoxia and
+                                          anaerobicDecompRate clamped.  They include resample() copies and
+                                          rejuvenate() moves */
 };
 
 /* rows of SIPNET_GPU_GATHER_COUNTERS: the status bits say WHETHER, these say HOW OFTEN (validation dump only) */
@@ -467,6 +472,60 @@ int sipnet_gpu_assimilate(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs, 
 int sipnet_gpu_resample(sipnet_gpu_handle *h, const double *u, double ess_fraction, const double *log_weights,
                         int64_t *ancestors, double *diag);
 
+/*
+ * Parameter rejuvenation after a resample: the kernel-shrinkage move of Liu & West (2001), per site, on listed
+ * parameter rows.  Resampling only copies parameter vectors, so after a few cycles a site holds a few distinct ones;
+ * this move spreads them again while keeping the site's ensemble mean and covariance (in the transformed space).
+ *
+ * Units: every value is in device units, i.e. after setupModel() (see SIPNET_GPU_GATHER_PARAMS).  A LOG or LOGIT move
+ * is invariant to the 1/365 rescaling up to rounding, and so is an IDENTITY move, because the move is affine.
+ *
+ * rows[n_rows] (1..16) are distinct SIPNET_P_* rows other than psnTMax and coarseRootAllocation (derived); row j is
+ * moved in phi = g_j(theta), transform[j] = SIPNET_GPU_TF_IDENTITY (phi = theta), SIPNET_GPU_TF_LOG (phi = log theta,
+ * domain theta > 0) or SIPNET_GPU_TF_LOGIT (phi = log((theta - lo) / (hi - theta)), domain lo < theta < hi with
+ * lo = lower[j], hi = upper[j]; lower / upper are read for LOGIT rows only and may be NULL without one).
+ * shrink[nsites] is a in (0, 1) per site, NaN = leave the site alone.  z[n_rows][nmembers] (host) are standard normals
+ * for the handle's members, supplied by the caller as resample() takes u.
+ *
+ * Member i takes part at its site iff its status has neither SIPNET_GPU_ST_BAD_ALLOCATION nor SIPNET_GPU_ST_NONFINITE
+ * and every listed row is finite and inside its transform's domain.  A site with shrink[s] not NaN and N >= 2
+ * participants is moved; with a = shrink[s], h = sqrt(1 - a^2), over the participants:
+ *   phi_ij = g_j(theta_ij);  mean_j = (1/N) sum_i phi_ij;
+ *   V_jl = (1/N) sum_i (phi_ij - mean_j)(phi_il - mean_l)   (population covariance, two passes)
+ *   L: semidefinite Cholesky factor of V in column order: for each j, d = V_jj - sum_{m<j} L_jm^2; if
+ *      d > 2^-40 V_jj then L_jj = sqrt(d) and L_ij = (V_ij - sum_{m<j} L_im L_jm) / L_jj (i > j), else column j is
+ *      zero; rank = the number of nonzero columns
+ *   phi'_ij = a phi_ij + (1 - a) mean_j + h sum_{m<=j} L_jm z_mi;  theta'_ij = g_j^-1(phi'_ij)
+ * The population covariance is what makes the mixture keep the ensemble's mean and covariance exactly.  A member's
+ * proposal is rejected -- the member stays bit-identical and counts as kept -- when some theta' is not finite or not
+ * inside its domain (the inverse can round onto a bound or underflow to 0), or when the proposed allocation fractions
+ * fail ensureAllocation (sipnet.c:1111-1123).  Otherwise the listed rows become theta' and every row setupModel()
+ * derives from other rows is derived again exactly as setupModel() does: coarseRootAllocation, psnTMax, the fAnoxia
+ * and anaerobicDecompRate clamps, and the library's internal per-member constants.
+ *
+ * Nothing else changes: status bits, carried state, rings, log-likelihoods, event records, the last run range's
+ * outputs and summaries, the next step.  Non-participants and sites left alone are untouched.  A later reset() starts
+ * from the moved parameters; set_params() replaces them.
+ *
+ * diag (may be NULL) receives double [nsites][4] = {N, rank (-1 where the site was left alone), moved, kept}.
+ *
+ * Rejected with SIPNET_GPU_ERR_BAD_ARGUMENT, nothing changed: NULL handle, spec or arrays; n_rows outside 1..16;
+ * a repeated, derived or out-of-range row; an unknown transform; LOGIT bounds that are not finite or with lo >= hi;
+ * a shrink neither NaN nor in (0, 1); a non-finite z.  Every call returns when the move is complete.
+ */
+#define SIPNET_GPU_TF_IDENTITY 0 /* phi = theta */
+#define SIPNET_GPU_TF_LOG 1      /* phi = log(theta), domain theta > 0 */
+#define SIPNET_GPU_TF_LOGIT 2    /* phi = log((theta - lo) / (hi - theta)), domain lo < theta < hi */
+typedef struct sipnet_gpu_jitter_spec {
+  int32_t n_rows;              /* 1 .. 16 */
+  const int32_t *rows;         /* distinct SIPNET_P_* rows; not psnTMax, not coarseRootAllocation (derived) */
+  const int32_t *transform;    /* [n_rows] SIPNET_GPU_TF_* */
+  const double *lower, *upper; /* [n_rows] bounds of LOGIT rows (read only for those; may be NULL without one) */
+  const double *shrink;        /* [nsites] a in (0, 1); NaN = leave the site alone */
+  const double *z;             /* [n_rows][nmembers] standard normals for this handle's members (host) */
+} sipnet_gpu_jitter_spec;
+int sipnet_gpu_rejuvenate(sipnet_gpu_handle *h, const sipnet_gpu_jitter_spec *spec, double *diag);
+
 /* Slots of the mean-NPP ring this handle uses (config ring_slots, or the automatic choice). */
 int32_t sipnet_gpu_ring_slots(const sipnet_gpu_handle *h);
 
@@ -566,6 +625,11 @@ int sipnet_gpu_comm_assimilate(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *ob
  * each source rank sends every destination rank the records of the slots it supplies (NCCL send / receive). */
 int sipnet_gpu_comm_resample(sipnet_gpu_comm *c, const double *u, double ess_fraction, const double *log_weights,
                              int64_t *ancestors, double *diag);
+/* Collective.  sipnet_gpu_rejuvenate() over the members of ALL ranks: every rank passes the same spec except z, which
+ * holds the rank's own members (a mismatch, found through an all-gathered hash of everything but z, fails on every
+ * rank); every rank gets the same diag.  The ranks all-gather two per-site partial sums (N and the sums of phi, then
+ * the centred cross sums) and add them in rank order, so every rank applies identical coefficients. */
+int sipnet_gpu_comm_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *spec, double *diag);
 
 /* (b) one process, one host thread, several GPUs: the single-GPU configuration, partitioned by the library --
  *     whole sites per device when there are at least as many sites as devices, otherwise an even contiguous share
@@ -596,6 +660,9 @@ int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *
  * sites go through the team exchange, whole sites are resampled by each device alone. */
 int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, double ess_fraction, const double *log_weights,
                               int64_t *ancestors, double *diag);
+/* sipnet_gpu_rejuvenate() on the whole configuration (shrink, z [n_rows][nmembers] and diag in configuration order):
+ * split sites go through the team exchange, whole sites are moved by each device alone. */
+int sipnet_gpu_multi_rejuvenate(sipnet_gpu_multi *m, const sipnet_gpu_jitter_spec *spec, double *diag);
 void sipnet_gpu_multi_destroy(sipnet_gpu_multi *m);
 
 #ifdef __cplusplus

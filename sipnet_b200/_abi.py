@@ -132,7 +132,9 @@ MATH_VALIDATION, MATH_FAST, MATH_THROUGHPUT = 0, 1, 2
 
 (GATHER_FULL, GATHER_DEBUG, GATHER_LOGLIK, GATHER_STATUS, GATHER_STATE,
  GATHER_MEAN, GATHER_VARIANCE, GATHER_QUANTILES, GATHER_EVENT_COUNTS,
- GATHER_EVENT_RECORDS, GATHER_LOGLIK_N, GATHER_RING_VALUES, GATHER_RING_WEIGHTS, GATHER_BALANCE, GATHER_COUNTERS) = range(1, 16)
+ GATHER_EVENT_RECORDS, GATHER_LOGLIK_N, GATHER_RING_VALUES, GATHER_RING_WEIGHTS, GATHER_BALANCE, GATHER_COUNTERS,
+ GATHER_PARAMS) = range(1, 17)
+TF_IDENTITY, TF_LOG, TF_LOGIT = 0, 1, 2      # sipnet_gpu_jitter_spec transforms
 
 ST_BAD_ALLOCATION, ST_RING_OVERFLOW, ST_CLAMPED, ST_DIED, ST_EVREC_OVERFLOW, \
     ST_NONFINITE, ST_REPLAY = 0x1, 0x2, 0x4, 0x8, 0x10, 0x20, 0x40
@@ -196,4 +198,13 @@ class ObsSpec(C.Structure):
         ("n_rows", C.c_int32), ("rows", C.POINTER(C.c_int32)),
         ("n_obs", C.c_int32), ("op", C.POINTER(C.c_double)),
         ("value", C.POINTER(C.c_double)), ("variance", C.POINTER(C.c_double)),
+    ]
+
+
+class JitterSpec(C.Structure):
+    """sipnet_gpu_jitter_spec: which parameter rows sipnet_gpu_rejuvenate() moves, how, and with which normals."""
+    _fields_ = [
+        ("n_rows", C.c_int32), ("rows", C.POINTER(C.c_int32)), ("transform", C.POINTER(C.c_int32)),
+        ("lower", C.POINTER(C.c_double)), ("upper", C.POINTER(C.c_double)),
+        ("shrink", C.POINTER(C.c_double)), ("z", C.POINTER(C.c_double)),
     ]

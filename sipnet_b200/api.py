@@ -134,6 +134,9 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     for name in ("sipnet_gpu_resample", "sipnet_gpu_comm_resample", "sipnet_gpu_multi_resample"):
         getattr(lib, name).restype = C.c_int
         getattr(lib, name).argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]
+    for name in ("sipnet_gpu_rejuvenate", "sipnet_gpu_comm_rejuvenate", "sipnet_gpu_multi_rejuvenate"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [C.c_void_p, C.POINTER(A.JitterSpec), C.c_void_p]
     lib.sipnet_gpu_eval_libm.restype = C.c_int
     lib.sipnet_gpu_eval_libm.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
     if path is None:
@@ -461,6 +464,42 @@ class Ensemble:
         n = int(self.team_member_counts().sum())
         return self._resample(self.lib.sipnet_gpu_comm_resample, self.comm, n, u, ess_fraction, log_weights)
 
+    def params(self) -> np.ndarray:
+        """[80][M]: the device's parameter rows, in device units (after setupModel(); see GATHER_PARAMS)."""
+        return self._gather(A.GATHER_PARAMS, np.float64, (A.NPARAMS, self.nmembers))
+
+    def jitter_spec(self, rows, transform, shrink, z, lower=None, upper=None):
+        """(A.JitterSpec, the arrays it points into) for sipnet_gpu_*_rejuvenate.  rows: A.P indices; transform:
+        A.TF_* per row; shrink: [nsites] (NaN = leave the site alone); z: [n_rows][nmembers]; lower / upper: the
+        bounds of LOGIT rows (other entries are not read)."""
+        rows = np.ascontiguousarray(rows, dtype=np.int32).reshape(-1)
+        tf = np.ascontiguousarray(np.broadcast_to(transform, rows.shape), dtype=np.int32)
+        shrink = np.ascontiguousarray(np.broadcast_to(shrink, (self.nsites,)), dtype=np.float64)
+        z = np.ascontiguousarray(z, dtype=np.float64)
+        if z.shape != (rows.size, self.nmembers):
+            raise ValueError(f"z must be [{rows.size}][{self.nmembers}]")
+        lo = None if lower is None else np.ascontiguousarray(np.broadcast_to(lower, rows.shape), dtype=np.float64)
+        hi = None if upper is None else np.ascontiguousarray(np.broadcast_to(upper, rows.shape), dtype=np.float64)
+        spec = A.JitterSpec(rows.size, _ip(rows), _ip(tf), None if lo is None else _dp(lo), None if hi is None else _dp(hi),
+                            _dp(shrink), _dp(z))
+        return spec, (rows, tf, lo, hi, shrink, z)
+
+    def _rejuvenate(self, fn, target, rows, transform, shrink, z, lower, upper) -> np.ndarray:
+        spec, _keep = self.jitter_spec(rows, transform, shrink, z, lower, upper)
+        diag = np.empty((self.nsites, 4), np.float64)
+        self._check(fn(target, C.byref(spec), diag.ctypes.data))
+        return diag
+
+    def rejuvenate(self, rows, transform, shrink, z, lower=None, upper=None) -> np.ndarray:
+        """Liu-West kernel-shrinkage move of the listed parameter rows, per site (sipnet_gpu_rejuvenate; see
+        include/sipnet_gpu.h).  Returns diag [nsites][4] = (N, rank (-1: site left alone), moved, kept)."""
+        return self._rejuvenate(self.lib.sipnet_gpu_rejuvenate, self.handle, rows, transform, shrink, z, lower, upper)
+
+    def team_rejuvenate(self, rows, transform, shrink, z, lower=None, upper=None) -> np.ndarray:
+        """Collective.  rejuvenate() over the members of every rank (same arguments on every rank except z, which
+        holds this rank's members)."""
+        return self._rejuvenate(self.lib.sipnet_gpu_comm_rejuvenate, self.comm, rows, transform, shrink, z, lower, upper)
+
     def mean(self) -> np.ndarray:
         return self._gather(A.GATHER_MEAN, np.float64, (self.nsites, self.n_summary_cols, self.nrun))
 
@@ -642,6 +681,9 @@ class MultiEnsemble(Ensemble):
 
     def resample(self, u, ess_fraction: float = math.inf, log_weights=None):
         return self._resample(self.lib.sipnet_gpu_multi_resample, self.multi, self.nmembers, u, ess_fraction, log_weights)
+
+    def rejuvenate(self, rows, transform, shrink, z, lower=None, upper=None) -> np.ndarray:
+        return self._rejuvenate(self.lib.sipnet_gpu_multi_rejuvenate, self.multi, rows, transform, shrink, z, lower, upper)
 
     def sync(self) -> None:
         self.lib.sipnet_gpu_multi_sync(self.multi)

@@ -10,8 +10,9 @@
 //   * one process per GPU (torchrun, MPI, ...): sipnet_gpu_comm_init_rank() with an id made by rank 0 and
 //     broadcast by the caller's launcher;
 //   * one process, one host thread, all GPUs: sipnet_gpu_multi_* (ncclCommInitAll, grouped calls).
-// The host sides of the ensemble adjustment Kalman filter (kernels: sip_assim.cu) and of the particle filter
-// (sip_resample.cu) live here too: a single handle runs them as a team of one, which needs no exchange.
+// The host sides of the ensemble adjustment Kalman filter (kernels: sip_assim.cu), of the particle filter
+// (sip_resample.cu) and of its parameter move (sip_jitter.cu) live here too: a single handle runs them as a team of
+// one, which needs no exchange.
 // NCCL is bound at run time (dlopen of libnccl.so.2): single-GPU use never loads it, and a process that already
 // carries an NCCL (e.g. PyTorch's) shares that copy.
 #include <cuda_runtime.h>
@@ -30,6 +31,7 @@
 #include "sip_assim.cuh"
 #include "sip_gsum.cuh"
 #include "sip_handle.h"
+#include "sip_jitter.cuh"
 #include "sip_resample.cuh"
 
 using namespace sip;
@@ -114,6 +116,7 @@ struct Local {
   int64_t llCap = 0;
   double *asAll = nullptr;  // [nranks][nsites][as::kRec] assimilation partials (rank slot 0 of each also the spec hash)
   int64_t asCap = 0;        // sites
+  double *jtAll = nullptr;  // [nranks][nsites][jt::kRec] parameter move partials
 };
 
 }  // namespace
@@ -452,6 +455,7 @@ extern "C" void sipnet_gpu_comm_destroy(sipnet_gpu_comm *c) {
     }
     free_local(l);
     if (l.asAll) cudaFree(l.asAll);
+    if (l.jtAll) cudaFree(l.jtAll);
     if (l.comm) nccl_api()->CommDestroy(l.comm);
   }
   if (c->ev0) cudaEventDestroy(c->ev0);
@@ -774,6 +778,7 @@ static bool member_output_shape(const sipnet_gpu_multi *m, int what, size_t *col
     case SIPNET_GPU_GATHER_LOGLIK_N: *cols = 1; return h0->loglik != nullptr;
     case SIPNET_GPU_GATHER_STATUS: *cols = 1; *elem = 4; return true;
     case SIPNET_GPU_GATHER_STATE: *cols = SIPNET_GPU_NSTATE; return true;
+    case SIPNET_GPU_GATHER_PARAMS: *cols = SIPNET_GPU_NPARAMS; return true;
     case SIPNET_GPU_GATHER_RING_VALUES:
     case SIPNET_GPU_GATHER_RING_WEIGHTS: *cols = (size_t)h0->ringCap; return true;
     case SIPNET_GPU_GATHER_EVENT_COUNTS: *cols = 1; *elem = 4; return h0->recCount != nullptr;
@@ -1518,6 +1523,189 @@ extern "C" int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, d
     if (int rc = run_resample(&one, u + s0, ess_fraction, {lw[d].data()}, diag ? diag + s0 * 4 : nullptr, anc)) return rc;
     if (ancestors)
       for (size_t j = 0; j < glob[d].size(); ++j) ancestors[glob[d][j]] = anc[j] < 0 ? -1 : glob[d][(size_t)anc[j]];
+  }
+  return 0;
+}
+
+// ---- parameter rejuvenation: the Liu-West move (sip_jitter.cuh) ---------------------------------------------------
+namespace {
+
+bool derived_row(int32_t r) { return r == SIPNET_P_psnTMax || r == SIPNET_P_coarseRootAllocation; }
+
+// the spec against `nsites` sites and `nmembers` members (z): 0, or SIPNET_GPU_ERR_BAD_ARGUMENT with the reason
+int check_jitter(const sipnet_gpu_jitter_spec *sp, int64_t nsites, int64_t nmembers) {
+  if (!sp || !sp->rows || !sp->transform || !sp->shrink || !sp->z)
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL jitter spec or array");
+  if (sp->n_rows < 1 || sp->n_rows > jt::kMaxRows)
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "n_rows must be 1..%d", jt::kMaxRows);
+  bool seen[SIPNET_GPU_NPARAMS] = {};
+  for (int j = 0; j < sp->n_rows; ++j) {
+    const int32_t r = sp->rows[j], tf = sp->transform[j];
+    if (r < 0 || r >= SIPNET_GPU_NPARAMS) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "parameter row %d out of range", r);
+    if (derived_row(r)) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "parameter row %d is derived by setupModel()", r);
+    if (seen[r]) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "parameter row %d listed twice", r);
+    seen[r] = true;
+    if (tf != SIPNET_GPU_TF_IDENTITY && tf != SIPNET_GPU_TF_LOG && tf != SIPNET_GPU_TF_LOGIT)
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "unknown transform %d of row %d", tf, r);
+    if (tf == SIPNET_GPU_TF_LOGIT) {
+      if (!sp->lower || !sp->upper) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "LOGIT row %d without lower / upper", r);
+      const double lo = sp->lower[j], hi = sp->upper[j];
+      if (!std::isfinite(lo) || !std::isfinite(hi) || !(lo < hi))
+        return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "LOGIT bounds of row %d must be finite with lower < upper", r);
+    }
+  }
+  for (int64_t s = 0; s < nsites; ++s) {
+    const double a = sp->shrink[s];
+    if (!std::isnan(a) && !(a > 0.0 && a < 1.0))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "shrink[%lld] = %g is neither NaN nor in (0, 1)", (long long)s, a);
+  }
+  for (size_t i = 0; i < (size_t)sp->n_rows * (size_t)nmembers; ++i)
+    if (!std::isfinite(sp->z[i])) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "z[%zu] is not finite", i);
+  return 0;
+}
+
+uint64_t jitter_hash(const sipnet_gpu_jitter_spec *sp, int64_t nsites) {
+  uint64_t h = 0xcbf29ce484222325ull;
+  h = fnv1a(h, &nsites, sizeof nsites);
+  h = fnv1a(h, &sp->n_rows, sizeof sp->n_rows);
+  h = fnv1a(h, sp->rows, (size_t)sp->n_rows * sizeof(int32_t));
+  h = fnv1a(h, sp->transform, (size_t)sp->n_rows * sizeof(int32_t));
+  for (int j = 0; j < sp->n_rows; ++j)
+    if (sp->transform[j] == SIPNET_GPU_TF_LOGIT) {
+      h = fnv1a(h, &sp->lower[j], sizeof(double));
+      h = fnv1a(h, &sp->upper[j], sizeof(double));
+    }
+  h = fnv1a(h, sp->shrink, (size_t)nsites * sizeof(double));
+  return h == 0 ? 1 : h;
+}
+
+// Move every local rank of `c` (all ranks hold the same sites): shrink holds the handles' sites, z[i] local rank i's
+// members.  A team of one needs no exchange and no host round trip; a larger team all-gathers the per-site partial
+// sums of the two moment passes and of the counts, and sums them in rank order on every rank.  diag (may be NULL)
+// gets local rank 0's [nsites][4].
+int run_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *sp, const double *shrink,
+                   const std::vector<const double *> &z, double *diag) {
+  const int R = c->nranks, n = sp->n_rows;
+  const int64_t S = c->local[0].h->nsites;
+  std::vector<jt::Args> args(c->local.size());
+  for (size_t i = 0; i < c->local.size(); ++i) {
+    Local &l = c->local[i];
+    sipnet_gpu_handle *h = l.h;
+    if (h->nsites != S) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites");
+    CUDA_OK(cudaSetDevice(h->device));
+    if (int rc = jt::ensure_scratch(h)) return rc;
+    if (R > 1 && !l.jtAll) CUDA_OK(cudaMalloc((void **)&l.jtAll, (size_t)R * S * jt::kRec * sizeof(double)));
+    CUDA_OK(cudaMemcpyAsync(h->jtShrink, shrink, (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(cudaMemcpyAsync(h->jtZ, z[i], (size_t)n * h->nmembers * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    jt::Args &a = args[i];
+    memset(&a, 0, sizeof a);
+    a.params = h->params;
+    a.status = h->status;
+    a.ld = h->ld;
+    a.nmembers = h->nmembers;
+    a.sites = h->sites;
+    a.nsites = (int32_t)S;
+    a.nchunks = (int32_t)h->asChunks;
+    a.chunk = h->asChunk;
+    a.siteChunks = h->asSiteChunks;
+    a.nrows = n;
+    a.nranks = R;
+    a.rank = l.rank;
+    for (int j = 0; j < n; ++j) {
+      a.rows[j] = sp->rows[j];
+      a.transform[j] = sp->transform[j];
+      a.lower[j] = sp->transform[j] == SIPNET_GPU_TF_LOGIT ? sp->lower[j] : 0.0;
+      a.upper[j] = sp->transform[j] == SIPNET_GPU_TF_LOGIT ? sp->upper[j] : 0.0;
+    }
+    a.shrink = h->jtShrink;
+    a.z = h->jtZ;
+    a.part = h->jtPart;
+    a.mom = h->jtMom;
+    a.coef = h->jtCoef;
+    a.diag = h->jtDiag;
+    a.rankRec = l.jtAll;
+  }
+  auto launched = [](sipnet_gpu_handle *h, cudaError_t e) {
+    h->launches++;
+    return e == cudaSuccess ? 0 : fail(SIPNET_GPU_ERR_NO_DEVICE, "rejuvenation launch failed: %s", cudaGetErrorString(e));
+  };
+  for (int pass = 1; pass <= 3; ++pass) {
+    for (size_t i = 0; i < c->local.size(); ++i) {
+      sipnet_gpu_handle *h = c->local[i].h;
+      CUDA_OK(cudaSetDevice(h->device));
+      if (int rc = launched(h, jt::launch_members(args[i], pass, h->stream))) return rc;
+      if (int rc = launched(h, jt::launch_site(args[i], pass, h->stream))) return rc;
+    }
+    if (R > 1) {
+      if (int rc = all_gather_bytes(c, (size_t)S * jt::kRec * sizeof(double), [](Local &l) -> void * { return l.jtAll; }))
+        return rc;
+      for (size_t i = 0; i < c->local.size(); ++i) {
+        sipnet_gpu_handle *h = c->local[i].h;
+        CUDA_OK(cudaSetDevice(h->device));
+        if (int rc = launched(h, jt::launch_combine(args[i], pass, h->stream))) return rc;
+      }
+    }
+  }
+  if (diag) {
+    sipnet_gpu_handle *h = c->local[0].h;
+    CUDA_OK(cudaSetDevice(h->device));
+    CUDA_OK(cudaMemcpyAsync(diag, h->jtDiag, (size_t)S * 4 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  }
+  return sync_all(c);
+}
+
+}  // namespace
+
+extern "C" int sipnet_gpu_rejuvenate(sipnet_gpu_handle *h, const sipnet_gpu_jitter_spec *spec, double *diag) {
+  if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  if (int rc = check_jitter(spec, h->nsites, h->nmembers)) return rc;
+  sipnet_gpu_comm one;
+  one.local.resize(1);
+  one.local[0].h = h;
+  return run_rejuvenate(&one, spec, spec->shrink, {spec->z}, diag);
+}
+
+extern "C" int sipnet_gpu_comm_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *spec, double *diag) {
+  if (!c) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL comm");
+  sipnet_gpu_handle *h = c->local[0].h;
+  const int64_t S = h->nsites;
+  const int bad = check_jitter(spec, S, h->nmembers);
+  if (int rc = team_agree(c, bad, bad ? 0 : jitter_hash(spec, S), "rejuvenation specs")) return rc;
+  return run_rejuvenate(c, spec, spec->shrink, std::vector<const double *>(c->local.size(), spec->z), diag);
+}
+
+extern "C" int sipnet_gpu_multi_rejuvenate(sipnet_gpu_multi *m, const sipnet_gpu_jitter_spec *spec, double *diag) {
+  if (!m) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  if (int rc = check_jitter(spec, m->nsites, m->nmembers)) return rc;
+  const size_t D = m->handles.size(), n = (size_t)spec->n_rows, M = (size_t)m->nmembers;
+  // every device's normals, [n_rows][its members], from the configuration-order z
+  std::vector<std::vector<double>> zd(D);
+  for (size_t d = 0; d < D; ++d) {
+    const sipnet_gpu_multi::Part &p = m->parts[d];
+    const size_t nm = (size_t)m->handles[d]->nmembers;
+    zd[d].resize(n * nm);
+    for (size_t j = 0; j < n; ++j) {
+      const double *zj = spec->z + j * M;
+      if (!m->split) {
+        memcpy(zd[d].data() + j * nm, zj + p.member0, nm * sizeof(double));
+      } else {
+        for (size_t s = 0; s < p.siteCount.size(); ++s)
+          memcpy(zd[d].data() + j * nm + p.siteLocal0[s], zj + p.siteGlobal0[s], (size_t)p.siteCount[s] * sizeof(double));
+      }
+    }
+  }
+  if (m->split) {  // every device ends with the same diagnostics: take device 0's
+    std::vector<const double *> ptrs;
+    for (size_t d = 0; d < D; ++d) ptrs.push_back(zd[d].data());
+    return run_rejuvenate(m->comm, spec, spec->shrink, ptrs, diag);
+  }
+  // whole sites: each device alone on its site range
+  for (size_t d = 0; d < D; ++d) {
+    sipnet_gpu_comm one;
+    one.local.resize(1);
+    one.local[0].h = m->handles[d];
+    const size_t s0 = (size_t)m->parts[d].site0;
+    if (int rc = run_rejuvenate(&one, spec, spec->shrink + s0, {zd[d].data()}, diag ? diag + s0 * 4 : nullptr)) return rc;
   }
   return 0;
 }

@@ -66,6 +66,8 @@ struct sipnet_gpu_handle {
   double *rsLogw = nullptr, *rsLmax = nullptr, *rsSend = nullptr, *rsRecv = nullptr;
   int64_t *rsAnc = nullptr, *rsTab = nullptr;
   size_t rsSiteCap = 0, rsTabCap = 0, rsSendCap = 0, rsRecvCap = 0;  // elements
+  // parameter move scratch (sip_jitter.cu), made by the first rejuvenation
+  double *jtPart = nullptr, *jtMom = nullptr, *jtCoef = nullptr, *jtDiag = nullptr, *jtShrink = nullptr, *jtZ = nullptr;
 };
 
 namespace sip {

@@ -6,77 +6,29 @@
 // kernel is bit-identical to the reference binary.
 #include <cuda_runtime.h>
 
+#include "sip_derive.cuh"
 #include "sip_step.cuh"
 
 namespace sip {
 namespace k1 {
 
 // ---- setup kernels: setupModel(), sipnet.c:1858-1951 ----------------------------------------
-// (1) parameter derivation, in place on the uploaded raw rows
+// (1) parameter derivation, in place on the uploaded raw rows: the unit changes, then the rows that depend on other
+// rows (sip_derive.cuh, shared with the parameter move of sip_jitter.cu)
 __global__ void derive_params_kernel(double *params, int64_t ld, int64_t nmembers, uint32_t *status) {
   const int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (m >= nmembers) return;
   auto P = [&](int k) -> double & { return params[(int64_t)k * ld + m]; };
-  uint32_t st = 0;
-  // ensureAllocation, sipnet.c:1111-1123
-  P(SIPNET_P_coarseRootAllocation) =
-      1 - P(SIPNET_P_leafAllocation) - P(SIPNET_P_woodAllocation) - P(SIPNET_P_fineRootAllocation);
-  if ((P(SIPNET_P_leafAllocation) >= 1.0) || (P(SIPNET_P_woodAllocation) >= 1.0) ||
-      (P(SIPNET_P_fineRootAllocation) >= 1.0) || (P(SIPNET_P_coarseRootAllocation) < 0)) {
-    st |= SIPNET_GPU_ST_BAD_ALLOCATION;
-  }
   P(SIPNET_P_baseVegResp) /= 365.0;  // :1873-1877
   P(SIPNET_P_litterBreakdownRate) /= 365.0;
   P(SIPNET_P_baseSoilResp) /= 365.0;
   P(SIPNET_P_woodTurnoverRate) /= 365.0;
   P(SIPNET_P_leafTurnoverRate) /= 365.0;
-  P(SIPNET_P_psnTMax) = P(SIPNET_P_psnTOpt) + (P(SIPNET_P_psnTOpt) - P(SIPNET_P_psnTMin));  // :1880-1881
   P(SIPNET_P_fineRootTurnoverRate) /= 365.0;  // :1898-1902
   P(SIPNET_P_coarseRootTurnoverRate) /= 365.0;
   P(SIPNET_P_baseCoarseRootResp) /= 365.0;
   P(SIPNET_P_baseFineRootResp) /= 365.0;
-  if (P(SIPNET_P_fAnoxia) <= 0.0) {  // :1905-1909
-    P(SIPNET_P_fAnoxia) = kTiny;
-  } else if (P(SIPNET_P_fAnoxia) >= 1.0) {
-    P(SIPNET_P_fAnoxia) = 1.0 - kTiny;
-  }
-  if (P(SIPNET_P_anaerobicDecompRate) <= 0.0) {  // :1912-1916
-    P(SIPNET_P_anaerobicDecompRate) = kTiny;
-  } else if (P(SIPNET_P_anaerobicDecompRate) > 1.0) {
-    P(SIPNET_P_anaerobicDecompRate) = 1.0;
-  }
-  // member constant of potPsn(): pow((psnTMax - psnTMin) / 2.0, 2), sipnet.c:622
-  P(kPsnTRangeSqSlot) = sip_pow((P(SIPNET_P_psnTMax) - P(SIPNET_P_psnTMin)) / 2.0, 2.0);
-  // division seeds of the member-constant divisors and member-constant sub-expressions (sip_num.cuh)
-  {
-    const FastNum fn;
-    P(kOneMinusFa) = 1 - P(SIPNET_P_fAnoxia);
-    P(kTwoWhc) = 2.0 * P(SIPNET_P_soilWHC);
-    P(kOneMinusFracLitResp) = 1.0 - P(SIPNET_P_fracLitterRespired);
-    P(kRespPerGram) = P(SIPNET_P_baseFolRespFrac) * P(SIPNET_P_aMax);
-    P(kGrossAMax) = P(SIPNET_P_aMax) * P(SIPNET_P_aMaxFrac) + P(kRespPerGram);
-    P(kConvBase) = 12.0 * (1.0 / 1000000000.0) * (P(SIPNET_P_leafCSpWt) / P(SIPNET_P_cFracLeaf));
-    P(kSeedLeafCSpWt) = fn.seed(P(SIPNET_P_leafCSpWt));
-    P(kSeedPsnTRangeSq) = fn.seed(P(kPsnTRangeSqSlot));
-    P(kSeedHalfSatPar) = fn.seed(P(SIPNET_P_halfSatPar));
-    P(kSeedWhc) = fn.seed(P(SIPNET_P_soilWHC));
-    P(kSeedTwoWhc) = fn.seed(P(kTwoWhc));
-    P(kSeedLeafCN) = fn.seed(P(SIPNET_P_leafCN));
-    P(kSeedWoodCN) = fn.seed(P(SIPNET_P_woodCN));
-    P(kSeedFineRootCN) = fn.seed(P(SIPNET_P_fineRootCN));
-    P(kSeedFAnoxia) = fn.seed(P(SIPNET_P_fAnoxia));
-    P(kSeedOneMinusFa) = fn.seed(P(kOneMinusFa));
-    P(kSeedCSat) = fn.seed(P(SIPNET_P_soilCSaturation));
-  }
-  // log_inline() of the member-constant pow() bases
-  const int bases[4] = {SIPNET_P_vegRespQ10, SIPNET_P_coarseRootQ10, SIPNET_P_fineRootQ10, SIPNET_P_soilRespQ10};
-  const int slots[4] = {kLogVegQ10, kLogCoarseQ10, kLogFineQ10, kLogSoilQ10};
-  for (int i = 0; i < 4; ++i) {
-    const libm::LogHL l = libm::pow_log(P(bases[i]));
-    P(slots[i]) = l.hi;
-    P(slots[i] + 1) = l.lo;
-  }
-  status[m] = st;
+  status[m] = derive_dependent(P) ? SIPNET_GPU_ST_BAD_ALLOCATION : 0u;
 }
 
 // (2) initial pools / trackers (also used by reset())

@@ -345,7 +345,7 @@ static void free_handle(sipnet_gpu_handle *h) {
                   h->stateBk, h->ringVBk, h->ringWBk, h->loglikBk, h->loglikNBk, h->statusBk,
                   h->recCountBk, h->sched, h->asChunk, h->asSiteChunks, h->asPart, h->asMom, h->asCoef,
                   h->asObs, h->asDiag, h->rsW, h->rsC, h->rsSite, h->rsLogw, h->rsLmax, h->rsSend, h->rsRecv,
-                  h->rsAnc, h->rsTab};
+                  h->rsAnc, h->rsTab, h->jtPart, h->jtMom, h->jtCoef, h->jtDiag, h->jtShrink, h->jtZ};
   for (void *p : ptrs)
     if (p) cudaFree(p);
   for (void *p : h->siteAllocs)
@@ -945,6 +945,7 @@ extern "C" size_t sipnet_gpu_gather_bytes(const sipnet_gpu_handle *h, int what) 
     case SIPNET_GPU_GATHER_QUANTILES: return h->quant ? (size_t)h->nsites * ns * h->quantiles.size() * n * 8 : 0;
     case SIPNET_GPU_GATHER_EVENT_COUNTS: return h->recCount ? M * 4 : 0;
     case SIPNET_GPU_GATHER_EVENT_RECORDS: return h->recs ? M * (size_t)h->maxRecs * sizeof(sipnet_gpu_event_record) : 0;
+    case SIPNET_GPU_GATHER_PARAMS: return (size_t)SIPNET_GPU_NPARAMS * M * 8;
     default: return 0;
   }
 }
@@ -975,6 +976,7 @@ extern "C" int sipnet_gpu_gather(sipnet_gpu_handle *h, int what, void *dst, size
     case SIPNET_GPU_GATHER_STATUS: return copy_rows(h, dst, h->status, 1, 4);
     case SIPNET_GPU_GATHER_COUNTERS: return copy_rows(h, dst, h->counters, SIPNET_GPU_NCOUNTERS, 4);
     case SIPNET_GPU_GATHER_STATE: return copy_rows(h, dst, h->state, SIPNET_GPU_NSTATE, 8);
+    case SIPNET_GPU_GATHER_PARAMS: return copy_rows(h, dst, h->params, SIPNET_GPU_NPARAMS, 8);
     case SIPNET_GPU_GATHER_RING_VALUES: return copy_rows(h, dst, h->ringV, (size_t)h->ringCap, 8);
     case SIPNET_GPU_GATHER_RING_WEIGHTS: return copy_rows(h, dst, h->ringW, (size_t)h->ringCap, 8);
     case SIPNET_GPU_GATHER_EVENT_COUNTS: return copy_rows(h, dst, h->recCount, 1, 4);
