@@ -5,7 +5,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <vector>
 
 #include "sip_assim.cuh"
 
@@ -214,25 +213,13 @@ unsigned blocks_for(int64_t units, int per) { return (unsigned)std::max<int64_t>
 }  // namespace
 
 int ensure_scratch(sipnet_gpu_handle *h, int nobs) {
+  if (int rc = ensure_chunks(h)) return rc;
   const size_t S = (size_t)h->nsites;
-  if (!h->asChunk) {
-    std::vector<int2> chunk, siteChunks(S);
-    for (size_t s = 0; s < S; ++s) {
-      const int32_t cnt = h->hostSites[s].memberCount;
-      siteChunks[s] = make_int2((int)chunk.size(), (cnt + kChunk - 1) / kChunk);
-      for (int32_t i = 0; i < cnt; i += kChunk) chunk.push_back(make_int2((int)s, i));
-    }
-    const size_t nc = std::max<size_t>(chunk.size(), 1);
-    cudaError_t e = cudaMalloc((void **)&h->asChunk, nc * sizeof(int2));
-    if (e == cudaSuccess) e = cudaMalloc((void **)&h->asSiteChunks, S * sizeof(int2));
-    if (e == cudaSuccess) e = cudaMalloc((void **)&h->asPart, nc * kRec * sizeof(double));
+  if (!h->asPart) {
+    cudaError_t e = cudaMalloc((void **)&h->asPart, (size_t)std::max<int64_t>(h->nchunks, 1) * kRec * sizeof(double));
     if (e == cudaSuccess) e = cudaMalloc((void **)&h->asMom, S * kRec * sizeof(double));
     if (e == cudaSuccess) e = cudaMalloc((void **)&h->asCoef, S * kRec * sizeof(double));
-    if (e == cudaSuccess && !chunk.empty())
-      e = cudaMemcpy(h->asChunk, chunk.data(), chunk.size() * sizeof(int2), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(h->asSiteChunks, siteChunks.data(), S * sizeof(int2), cudaMemcpyHostToDevice);
     if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "assimilation scratch: %s", cudaGetErrorString(e));
-    h->asChunks = (int64_t)chunk.size();
   }
   if (nobs > h->asObsCap) {
     cudaFree(h->asObs);

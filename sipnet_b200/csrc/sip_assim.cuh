@@ -26,8 +26,6 @@ namespace as {
 
 constexpr int kMaxRows = 12;   // the pools SIPNET_S_plantWoodC .. SIPNET_S_plantStorageN
 constexpr int kRec = 16;       // doubles per chunk / site / rank record
-constexpr int kChunk = 128;    // site-local members per chunk
-constexpr uint32_t kExcluded = SIPNET_GPU_ST_BAD_ALLOCATION | SIPNET_GPU_ST_NONFINITE;
 
 // Record layouts (doubles):
 //   pass-1 partial  [0] N  [1] Σy  [2+j] Σx_j          means  [0] N  [1] ȳ  [2+j] x̄_j
@@ -57,7 +55,7 @@ struct Args {
   double *rankRec;          // [nranks][nsites][kRec] (teams only)
 };
 
-// chunk tables and per-call buffers of the handle (made once; the observation buffers grow with nobs)
+// the handle's chunk tables and per-call buffers (made once; the observation buffers grow with nobs)
 int ensure_scratch(sipnet_gpu_handle *h, int nobs);
 // pass 0 / 1 / 2; `apply`: first add the update of observation k - 1; `floor`: then the final floor
 cudaError_t launch_members(const Args &a, int pass, bool apply, bool floor, cudaStream_t stream);

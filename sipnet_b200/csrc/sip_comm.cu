@@ -98,6 +98,25 @@ const NcclApi *nccl_api() {
       return fail(SIPNET_GPU_ERR_NO_DEVICE, "%s failed: %s", #expr, nccl_api()->GetErrorString(r__)); \
   } while (0)
 
+// `p` holds at least `need` elements (at least one), reallocated after `stream` has finished with the old buffer
+template <class T>
+int grow(T *&p, size_t &cap, size_t need, cudaStream_t stream) {
+  if (need <= cap && p) return 0;
+  CUDA_OK(cudaStreamSynchronize(stream));
+  if (p) cudaFree(p);
+  p = nullptr;
+  cap = 0;
+  CUDA_OK(cudaMalloc((void **)&p, std::max<size_t>(need, 1) * sizeof(T)));
+  cap = std::max<size_t>(need, 1);
+  return 0;
+}
+
+// count a launch on `h` and map its error
+int launched(sipnet_gpu_handle *h, cudaError_t e, const char *what) {
+  h->launches++;
+  return e == cudaSuccess ? 0 : fail(SIPNET_GPU_ERR_NO_DEVICE, "%s launch failed: %s", what, cudaGetErrorString(e));
+}
+
 // one local rank of the team: a handle, its communicator and its scratch for the cross-rank summaries
 struct Local {
   sipnet_gpu_handle *h = nullptr;
@@ -112,11 +131,9 @@ struct Local {
   gs::GsTie *tieAll = nullptr;
   uint64_t *emitAll = nullptr;
   int32_t *flags = nullptr;
-  double *llAll = nullptr;  // [nranks][maxMembers] log-likelihood gather
-  int64_t llCap = 0;
-  double *asAll = nullptr;  // [nranks][nsites][as::kRec] assimilation partials (rank slot 0 of each also the spec hash)
-  int64_t asCap = 0;        // sites
-  double *jtAll = nullptr;  // [nranks][nsites][jt::kRec] parameter move partials
+  // [nranks][bytes per rank] of one all-gather at a time: argument hashes, the filters' per-site partials, member words
+  unsigned char *xchg = nullptr;
+  size_t xchgCap = 0;
 };
 
 }  // namespace
@@ -133,21 +150,22 @@ struct sipnet_gpu_comm {
 
 namespace {
 
+// all scratch of `l`: the rank keeps its handle, communicator and rank
 void free_local(Local &l) {
   if (l.h) cudaSetDevice(l.h->device);
-  void *ptrs[] = {l.statAll, l.q2All, l.hist, l.state, l.tieAll, l.emitAll, l.flags, l.llAll};
+  void *ptrs[] = {l.statAll, l.q2All, l.hist, l.state, l.tieAll, l.emitAll, l.flags, l.xchg};
   for (void *p : ptrs)
     if (p) cudaFree(p);
-  l.statAll = nullptr;
-  l.q2All = nullptr;
-  l.hist = nullptr;
-  l.state = nullptr;
-  l.tieAll = nullptr;
-  l.emitAll = nullptr;
-  l.flags = nullptr;
-  l.llAll = nullptr;
-  l.rowsCap = 0;
-  l.llCap = 0;
+  l = Local{l.h, l.comm, l.rank};
+}
+
+// one handle alone: a team of one rank, which needs no exchange
+sipnet_gpu_comm team_of_one(sipnet_gpu_handle *h) {
+  sipnet_gpu_comm one;
+  one.local.resize(1);
+  one.local[0].h = h;
+  one.memberCounts.assign(1, h->nmembers);
+  return one;
 }
 
 // collectives over the team; with one rank they are no-ops (local data already sits at index `rank` = 0)
@@ -223,12 +241,7 @@ int ensure_scratch(sipnet_gpu_comm *c, Local &l, int64_t rows) {
   sipnet_gpu_handle *h = l.h;
   CUDA_OK(cudaSetDevice(h->device));
   CUDA_OK(cudaStreamSynchronize(h->stream));
-  void *keepLl = l.llAll;
-  const int64_t keepCap = l.llCap;
-  l.llAll = nullptr;
   free_local(l);
-  l.llAll = static_cast<double *>(keepLl);
-  l.llCap = keepCap;
   CUDA_OK(cudaMalloc((void **)&l.statAll, (size_t)R * rows * sizeof(gs::GsStat)));
   CUDA_OK(cudaMalloc((void **)&l.q2All, (size_t)R * rows * sizeof(double)));
   CUDA_OK(cudaMalloc((void **)&l.hist, (size_t)rows * gs::kGsHistWords * sizeof(uint32_t)));
@@ -304,9 +317,7 @@ int team_summaries(sipnet_gpu_comm *c) {
       }
       a.wantMoments = (l.h->mean != nullptr && q0 == 0) ? 1 : 0;
       CUDA_OK(cudaSetDevice(l.h->device));
-      cudaError_t e = gs::launch_pass0(a, l.h->stream);
-      l.h->launches++;
-      if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "summary launch failed: %s", cudaGetErrorString(e));
+      if (int rc = launched(l.h, gs::launch_pass0(a, l.h->stream), "summary")) return rc;
     }
     if (int rc = all_gather_bytes(c, (size_t)rows * sizeof(gs::GsStat), [](Local &l) -> void * { return l.statAll; })) return rc;
     if (args[0].nq > 0)
@@ -316,9 +327,7 @@ int team_summaries(sipnet_gpu_comm *c) {
         Local &l = c->local[i];
         CUDA_OK(cudaSetDevice(l.h->device));
         CUDA_OK(cudaMemsetAsync(l.flags, 0, 16, l.h->stream));
-        cudaError_t e = gs::launch_level(args[i], level, l.h->stream);
-        l.h->launches++;
-        if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "summary launch failed: %s", cudaGetErrorString(e));
+        if (int rc = launched(l.h, gs::launch_level(args[i], level, l.h->stream), "summary")) return rc;
       }
       // the flag is a function of exchanged data only: every rank reads the same value
       int32_t flag = 0;
@@ -340,9 +349,7 @@ int team_summaries(sipnet_gpu_comm *c) {
       for (size_t i = 0; i < c->local.size(); ++i) {
         Local &l = c->local[i];
         CUDA_OK(cudaSetDevice(l.h->device));
-        cudaError_t e = gs::launch_emit(args[i], l.h->stream);
-        l.h->launches++;
-        if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "summary launch failed: %s", cudaGetErrorString(e));
+        if (int rc = launched(l.h, gs::launch_emit(args[i], l.h->stream), "summary")) return rc;
       }
       if (int rc = all_gather_bytes(c, (size_t)rows * gs::kGsMaxStat * gs::kGsEmit * sizeof(uint64_t),
                                     [](Local &l) -> void * { return l.emitAll; }))
@@ -351,9 +358,7 @@ int team_summaries(sipnet_gpu_comm *c) {
     for (size_t i = 0; i < c->local.size(); ++i) {
       Local &l = c->local[i];
       CUDA_OK(cudaSetDevice(l.h->device));
-      cudaError_t e = gs::launch_finish(args[i], l.h->stream);
-      l.h->launches++;
-      if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "summary launch failed: %s", cudaGetErrorString(e));
+      if (int rc = launched(l.h, gs::launch_finish(args[i], l.h->stream), "summary")) return rc;
     }
   }
   for (Local &l : c->local) l.h->summariesValid = true;
@@ -454,8 +459,6 @@ extern "C" void sipnet_gpu_comm_destroy(sipnet_gpu_comm *c) {
       cudaStreamSynchronize(l.h->stream);
     }
     free_local(l);
-    if (l.asAll) cudaFree(l.asAll);
-    if (l.jtAll) cudaFree(l.jtAll);
     if (l.comm) nccl_api()->CommDestroy(l.comm);
   }
   if (c->ev0) cudaEventDestroy(c->ev0);
@@ -489,23 +492,18 @@ static int team_member_words(sipnet_gpu_comm *c, void *dst, size_t bytes, const 
     const void *from = src(h);
     if (!from) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "%s output was not requested at init", what);
     CUDA_OK(cudaSetDevice(h->device));
-    if (l.llCap < width) {
-      if (l.llAll) cudaFree(l.llAll);
-      l.llAll = nullptr;
-      CUDA_OK(cudaMalloc((void **)&l.llAll, (size_t)c->nranks * width * sizeof(double)));
-      l.llCap = width;
-    }
-    CUDA_OK(cudaMemcpyAsync(l.llAll + (size_t)l.rank * width, from, (size_t)h->nmembers * sizeof(double),
+    if (int rc = grow(l.xchg, l.xchgCap, (size_t)c->nranks * width * sizeof(double), h->stream)) return rc;
+    CUDA_OK(cudaMemcpyAsync(l.xchg + (size_t)l.rank * width * sizeof(double), from, (size_t)h->nmembers * sizeof(double),
                             cudaMemcpyDeviceToDevice, h->stream));
   }
-  if (int rc = all_gather_bytes(c, (size_t)width * sizeof(double), [](Local &l) -> void * { return l.llAll; })) return rc;
+  if (int rc = all_gather_bytes(c, (size_t)width * sizeof(double), [](Local &l) -> void * { return l.xchg; })) return rc;
   if (dst) {
     Local &l = c->local[0];
     CUDA_OK(cudaSetDevice(l.h->device));
     int64_t off = 0;
     for (int q = 0; q < c->nranks; ++q) {
-      CUDA_OK(cudaMemcpyAsync(static_cast<double *>(dst) + off, l.llAll + (size_t)q * width, (size_t)c->memberCounts[(size_t)q] * sizeof(double),
-                              cudaMemcpyDeviceToHost, l.h->stream));
+      CUDA_OK(cudaMemcpyAsync(static_cast<double *>(dst) + off, l.xchg + (size_t)q * width * sizeof(double),
+                              (size_t)c->memberCounts[(size_t)q] * sizeof(double), cudaMemcpyDeviceToHost, l.h->stream));
       off += c->memberCounts[(size_t)q];
     }
     CUDA_OK(cudaStreamSynchronize(l.h->stream));
@@ -541,21 +539,21 @@ struct sipnet_gpu_multi {
   bool split = false;  // sites are split over devices (else whole sites per device)
   int64_t nmembers = 0, nsites = 0, nsummary = 0, nquant = 0;
   uint32_t outputs = 0;
-  // per device: for whole-site partitions the global member / site range; for split sites per site the global
-  // offset of the device's share
+  // per device: its site range, and its members as runs of consecutive members, `count` members from local index
+  // `local0` and configuration index `global0` on (whole sites: one run; split sites: one run per site)
+  struct Run {
+    int64_t local0, global0, count;
+  };
   struct Part {
-    int64_t site0 = 0, site1 = 0, member0 = 0, member1 = 0;
-    std::vector<int64_t> siteGlobal0, siteLocal0, siteCount;  // split: per site
+    int64_t site0 = 0, site1 = 0;
+    std::vector<Run> runs;
   };
   std::vector<Part> parts;
 };
 
 extern "C" void sipnet_gpu_multi_destroy(sipnet_gpu_multi *m) {
   if (!m) return;
-  if (m->comm) {
-    for (Local &l : m->comm->local) l.h = l.h;  // handles are destroyed below, after the communicators
-    sipnet_gpu_comm_destroy(m->comm);
-  }
+  sipnet_gpu_comm_destroy(m->comm);  // first: it synchronises the handles' streams
   for (sipnet_gpu_handle *h : m->handles) sipnet_gpu_destroy(h);
   delete m;
 }
@@ -636,22 +634,17 @@ extern "C" int sipnet_gpu_multi_init(const sipnet_gpu_config *cfg, int32_t ndevi
       p.site1 = (cfg->nsites * (d + 1)) / D;
       for (int64_t i = 0; i < cfg->nmembers; ++i)
         if (memberSite[(size_t)i] >= p.site0 && memberSite[(size_t)i] < p.site1) pick.push_back(i);
+      if (!pick.empty()) p.runs.push_back({0, pick.front(), (int64_t)pick.size()});  // member_site is non-decreasing
     } else {
       p.site0 = 0;
       p.site1 = cfg->nsites;
-      int64_t local = 0;
       for (int64_t s = 0; s < cfg->nsites; ++s) {
         const int64_t lo = (siteCnt[(size_t)s] * d) / D, hi = (siteCnt[(size_t)s] * (d + 1)) / D;
-        p.siteGlobal0.push_back(siteM0[(size_t)s] + lo);
-        p.siteLocal0.push_back(local);
-        p.siteCount.push_back(hi - lo);
+        p.runs.push_back({(int64_t)pick.size(), siteM0[(size_t)s] + lo, hi - lo});
         for (int64_t i = lo; i < hi; ++i) pick.push_back(siteM0[(size_t)s] + i);
-        local += hi - lo;
       }
     }
     if (pick.empty()) continue;
-    p.member0 = pick.front();
-    p.member1 = pick.back() + 1;
     m->parts.push_back(p);
     picks.push_back(std::move(pick));
     keptDevs.push_back(devs[(size_t)d]);
@@ -854,28 +847,20 @@ extern "C" int sipnet_gpu_multi_gather(sipnet_gpu_multi *m, int what, void *dst,
     sipnet_gpu_handle *h = m->handles[d];
     const size_t nm = (size_t)h->nmembers;
     const size_t nd = perStep ? (size_t)(h->lastEnd - h->lastBegin) : 1;
-    const sipnet_gpu_multi::Part &p = m->parts[d];
     if (nd > 0) {
       tmp.resize(cols * nd * nm * elem);
       if (int rc = sipnet_gpu_gather(h, what, tmp.data(), tmp.size())) return rc;
     }
-    auto scatter = [&](size_t local0, size_t global0, size_t count) {
+    for (const sipnet_gpu_multi::Run &r : m->parts[d].runs)
       for (size_t c = 0; c < cols; ++c)
         for (size_t t = 0; t < steps; ++t) {
-          char *to = static_cast<char *>(dst) + ((c * steps + t) * M + global0) * elem;
+          char *to = static_cast<char *>(dst) + ((c * steps + t) * M + (size_t)r.global0) * elem;
           if (t < nd) {
-            memcpy(to, tmp.data() + ((c * nd + t) * nm + local0) * elem, count * elem);
+            memcpy(to, tmp.data() + ((c * nd + t) * nm + (size_t)r.local0) * elem, (size_t)r.count * elem);
           } else {  // steps this device's (shorter) sites never ran: NaN, as on one GPU
-            memset(to, 0xFF, count * elem);
+            memset(to, 0xFF, (size_t)r.count * elem);
           }
         }
-    };
-    if (!m->split) {
-      scatter(0, (size_t)p.member0, nm);
-    } else {
-      for (size_t s = 0; s < p.siteCount.size(); ++s)
-        scatter((size_t)p.siteLocal0[s], (size_t)p.siteGlobal0[s], (size_t)p.siteCount[s]);
-    }
   }
   return 0;
 }
@@ -915,35 +900,27 @@ int check_obs(const sipnet_gpu_obs_spec *o, int64_t nsites) {
   return 0;
 }
 
-uint64_t fnv1a(uint64_t h, const void *p, size_t n) {
-  const unsigned char *b = static_cast<const unsigned char *>(p);
-  for (size_t i = 0; i < n; ++i) h = (h ^ b[i]) * 0x100000001b3ull;
-  return h;
-}
+// FNV-1a of a collective's arguments, for team_agree: never 0, which stands for invalid arguments
+struct ArgHash {
+  uint64_t h = 0xcbf29ce484222325ull;
+  ArgHash &add(const void *p, size_t n) {
+    const unsigned char *b = static_cast<const unsigned char *>(p);
+    for (size_t i = 0; i < n; ++i) h = (h ^ b[i]) * 0x100000001b3ull;
+    return *this;
+  }
+  uint64_t value() const { return h == 0 ? 1 : h; }
+};
 
 uint64_t spec_hash(const sipnet_gpu_obs_spec *o, int64_t nsites) {
-  uint64_t h = 0xcbf29ce484222325ull;
   const size_t nv = (size_t)nsites * (size_t)o->n_obs;
-  h = fnv1a(h, &o->n_rows, sizeof o->n_rows);
-  h = fnv1a(h, o->rows, (size_t)o->n_rows * sizeof(int32_t));
-  h = fnv1a(h, &o->n_obs, sizeof o->n_obs);
-  h = fnv1a(h, o->op, (size_t)o->n_obs * o->n_rows * sizeof(double));
-  h = fnv1a(h, o->value, nv * sizeof(double));
-  h = fnv1a(h, o->variance, nv * sizeof(double));
-  return h == 0 ? 1 : h;  // 0 stands for an invalid spec
-}
-
-int ensure_as_scratch(sipnet_gpu_comm *c, Local &l) {
-  const int64_t S = l.h->nsites;
-  if (l.asCap >= S) return 0;
-  CUDA_OK(cudaSetDevice(l.h->device));
-  CUDA_OK(cudaStreamSynchronize(l.h->stream));
-  if (l.asAll) cudaFree(l.asAll);
-  l.asAll = nullptr;
-  l.asCap = 0;
-  CUDA_OK(cudaMalloc((void **)&l.asAll, (size_t)c->nranks * S * as::kRec * sizeof(double)));
-  l.asCap = S;
-  return 0;
+  return ArgHash()
+      .add(&o->n_rows, sizeof o->n_rows)
+      .add(o->rows, (size_t)o->n_rows * sizeof(int32_t))
+      .add(&o->n_obs, sizeof o->n_obs)
+      .add(o->op, (size_t)o->n_obs * o->n_rows * sizeof(double))
+      .add(o->value, nv * sizeof(double))
+      .add(o->variance, nv * sizeof(double))
+      .value();
 }
 
 // Queue the analysis on every local rank of `c`: value / variance hold the handles' sites (all ranks hold the same
@@ -960,7 +937,7 @@ int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const dou
     CUDA_OK(cudaSetDevice(h->device));
     if (int rc = as::ensure_scratch(h, nobs)) return rc;
     if (R > 1)
-      if (int rc = ensure_as_scratch(c, l)) return rc;
+      if (int rc = grow(l.xchg, l.xchgCap, (size_t)R * h->nsites * as::kRec * sizeof(double), h->stream)) return rc;
     const size_t nv = (size_t)h->nsites * nobs;
     CUDA_OK(cudaMemcpyAsync(h->asObs, value, nv * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CUDA_OK(cudaMemcpyAsync(h->asObs + nv, variance, nv * sizeof(double), cudaMemcpyHostToDevice, h->stream));
@@ -972,9 +949,9 @@ int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const dou
     a.ld = h->ld;
     a.sites = h->sites;
     a.nsites = (int32_t)h->nsites;
-    a.nchunks = (int32_t)h->asChunks;
-    a.chunk = h->asChunk;
-    a.siteChunks = h->asSiteChunks;
+    a.nchunks = (int32_t)h->nchunks;
+    a.chunk = h->chunk;
+    a.siteChunks = h->siteChunks;
     a.nrows = nr;
     a.nobs = nobs;
     a.nranks = R;
@@ -986,12 +963,8 @@ int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const dou
     a.value = h->asObs;
     a.variance = h->asObs + nv;
     a.diag = h->asDiag;
-    a.rankRec = l.asAll;
+    a.rankRec = reinterpret_cast<double *>(l.xchg);
   }
-  auto launched = [](sipnet_gpu_handle *h, cudaError_t e) {
-    h->launches++;
-    return e == cudaSuccess ? 0 : fail(SIPNET_GPU_ERR_NO_DEVICE, "assimilation launch failed: %s", cudaGetErrorString(e));
-  };
   for (int k = 0; k < nobs; ++k) {
     for (int pass = 1; pass <= 2; ++pass) {
       for (size_t i = 0; i < c->local.size(); ++i) {
@@ -1004,16 +977,17 @@ int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const dou
         }
         CUDA_OK(cudaSetDevice(h->device));
         // pass 1 of observation k first applies observation k - 1
-        if (int rc = launched(h, as::launch_members(a, pass, pass == 1 && k > 0, false, h->stream))) return rc;
-        if (int rc = launched(h, as::launch_site_reduce(a, pass, h->stream))) return rc;
+        if (int rc = launched(h, as::launch_members(a, pass, pass == 1 && k > 0, false, h->stream), "assimilation"))
+          return rc;
+        if (int rc = launched(h, as::launch_site_reduce(a, pass, h->stream), "assimilation")) return rc;
       }
       if (R > 1) {
         const size_t bytes = (size_t)args[0].nsites * as::kRec * sizeof(double);
-        if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.asAll; })) return rc;
+        if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.xchg; })) return rc;
         for (size_t i = 0; i < c->local.size(); ++i) {
           sipnet_gpu_handle *h = c->local[i].h;
           CUDA_OK(cudaSetDevice(h->device));
-          if (int rc = launched(h, as::launch_site_combine(args[i], pass, h->stream))) return rc;
+          if (int rc = launched(h, as::launch_site_combine(args[i], pass, h->stream), "assimilation")) return rc;
         }
       }
     }
@@ -1023,7 +997,7 @@ int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const dou
     sipnet_gpu_handle *h = c->local[i].h;
     for (int j = 0; j < nr; ++j) a.opPrev[j] = o->op[(size_t)(nobs - 1) * nr + j];
     CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = launched(h, as::launch_members(a, 0, true, true, h->stream))) return rc;
+    if (int rc = launched(h, as::launch_members(a, 0, true, true, h->stream), "assimilation")) return rc;
   }
   return 0;
 }
@@ -1038,20 +1012,13 @@ int finish_assimilation(sipnet_gpu_handle *h, double *diag, int nobs) {
   return 0;
 }
 
-// one handle alone: a team of one rank (no exchange)
-int assimilate_alone(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *o, const double *value, const double *variance) {
-  sipnet_gpu_comm one;
-  one.local.resize(1);
-  one.local[0].h = h;
-  return run_assimilation(&one, o, value, variance);
-}
-
 }  // namespace
 
 extern "C" int sipnet_gpu_assimilate(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs, double *diag) {
   if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
   if (int rc = check_obs(obs, h->nsites)) return rc;
-  if (int rc = assimilate_alone(h, obs, obs->value, obs->variance)) return rc;
+  sipnet_gpu_comm one = team_of_one(h);
+  if (int rc = run_assimilation(&one, obs, obs->value, obs->variance)) return rc;
   return finish_assimilation(h, diag, obs->n_obs);
 }
 
@@ -1061,15 +1028,16 @@ static int team_agree(sipnet_gpu_comm *c, int bad, uint64_t mine, const char *wh
   if (c->nranks == 1) return bad;
   const std::string why = bad ? sipnet_gpu_last_error() : "";
   for (Local &l : c->local) {
-    if (int rc = ensure_as_scratch(c, l)) return rc;
-    CUDA_OK(cudaMemcpyAsync(l.asAll + l.rank, &mine, sizeof mine, cudaMemcpyHostToDevice, l.h->stream));
+    CUDA_OK(cudaSetDevice(l.h->device));
+    if (int rc = grow(l.xchg, l.xchgCap, (size_t)c->nranks * sizeof mine, l.h->stream)) return rc;
+    CUDA_OK(cudaMemcpyAsync(l.xchg + l.rank * sizeof mine, &mine, sizeof mine, cudaMemcpyHostToDevice, l.h->stream));
     CUDA_OK(cudaStreamSynchronize(l.h->stream));
   }
-  if (int rc = all_gather_bytes(c, sizeof(uint64_t), [](Local &l) -> void * { return l.asAll; })) return rc;
+  if (int rc = all_gather_bytes(c, sizeof mine, [](Local &l) -> void * { return l.xchg; })) return rc;
   std::vector<uint64_t> all((size_t)c->nranks);
   Local &l0 = c->local[0];
   CUDA_OK(cudaSetDevice(l0.h->device));
-  CUDA_OK(cudaMemcpyAsync(all.data(), l0.asAll, all.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, l0.h->stream));
+  CUDA_OK(cudaMemcpyAsync(all.data(), l0.xchg, all.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, l0.h->stream));
   CUDA_OK(cudaStreamSynchronize(l0.h->stream));
   for (uint64_t v : all)
     if (v == 0 || v != all[0]) {
@@ -1103,7 +1071,8 @@ extern "C" int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu
   // whole sites: each device alone on its site range, all devices side by side
   for (size_t d = 0; d < m->handles.size(); ++d) {
     const size_t off = (size_t)m->parts[d].site0 * nobs;
-    if (int rc = assimilate_alone(m->handles[d], obs, obs->value + off, obs->variance + off)) return rc;
+    sipnet_gpu_comm one = team_of_one(m->handles[d]);
+    if (int rc = run_assimilation(&one, obs, obs->value + off, obs->variance + off)) return rc;
   }
   for (size_t d = 0; d < m->handles.size(); ++d)
     if (int rc = finish_assimilation(m->handles[d], diag ? diag + (size_t)m->parts[d].site0 * nobs * 4 : nullptr, nobs))
@@ -1128,6 +1097,16 @@ int check_resample(const sipnet_gpu_handle *h, const double *u, int64_t nsites, 
   return 0;
 }
 
+uint64_t resample_hash(const sipnet_gpu_handle *h, const double *u, double essFraction) {
+  const int64_t S = h->nsites, words = rs::record_words(h);
+  return ArgHash()
+      .add(&S, sizeof S)
+      .add(&words, sizeof words)
+      .add(&essFraction, sizeof essFraction)
+      .add(u, (size_t)S * sizeof(double))
+      .value();
+}
+
 // K(C): the first slot k with t_k >= C, i.e. clamp(ceil((ceil(C n 2^32 / T) - U) / 2^32), 0, n)
 int64_t first_slot(uint64_t C, uint64_t T, uint64_t U, int64_t n) {
   const u128 a = ((((u128)C * (uint64_t)n) << 32) + T - 1) / T;
@@ -1149,18 +1128,6 @@ int site_records(sipnet_gpu_comm *c, std::vector<uint64_t> &out) {
   return 0;
 }
 
-template <class T>
-int grow(T *&p, size_t &cap, size_t need, cudaStream_t stream) {
-  if (need <= cap && p) return 0;
-  CUDA_OK(cudaStreamSynchronize(stream));
-  if (p) cudaFree(p);
-  p = nullptr;
-  cap = 0;
-  CUDA_OK(cudaMalloc((void **)&p, std::max<size_t>(need, 1) * sizeof(T)));
-  cap = std::max<size_t>(need, 1);
-  return 0;
-}
-
 // this rank's part of the copy: segment sizes (records) and where they sit (doubles)
 struct CopyPlan {
   std::vector<int64_t> tab;
@@ -1176,10 +1143,6 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
   const int words = rs::record_words(c->local[0].h);
   const size_t L = c->local.size();
   std::vector<rs::Args> args(L);
-  auto launched = [](sipnet_gpu_handle *h, cudaError_t e) {
-    h->launches++;
-    return e == cudaSuccess ? 0 : fail(SIPNET_GPU_ERR_NO_DEVICE, "resampling launch failed: %s", cudaGetErrorString(e));
-  };
   std::vector<int64_t> rankBase((size_t)R + 1, 0);
   for (int q = 0; q < R; ++q) rankBase[(size_t)q + 1] = rankBase[(size_t)q] + c->memberCounts[(size_t)q];
   for (size_t i = 0; i < L; ++i) {
@@ -1201,9 +1164,9 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
     a.nmembers = h->nmembers;
     a.ld = h->ld;
     a.nsites = (int32_t)S;
-    a.nchunks = (int32_t)h->asChunks;
-    a.chunk = h->asChunk;
-    a.siteChunks = h->asSiteChunks;
+    a.nchunks = (int32_t)h->nchunks;
+    a.chunk = h->chunk;
+    a.siteChunks = h->siteChunks;
     a.params = h->params;
     a.state = h->state;
     a.ringV = h->ringV;
@@ -1219,14 +1182,14 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
     a.nranks = R;
     a.rank = l.rank;
     a.idBase = rankBase[(size_t)l.rank];
-    a.part = reinterpret_cast<uint64_t *>(h->asPart);
+    a.part = h->rsPart;
     a.w = h->rsW;
     a.c = h->rsC;
     a.siteRec = h->rsSite;
     a.lmax = h->rsLmax;
     a.anc = h->rsAnc;
-    if (int rc = launched(h, rs::launch_weights(a, 0, h->stream))) return rc;
-    if (int rc = launched(h, rs::launch_site(a, 0, h->stream))) return rc;
+    if (int rc = launched(h, rs::launch_weights(a, 0, h->stream), "resampling")) return rc;
+    if (int rc = launched(h, rs::launch_site(a, 0, h->stream), "resampling")) return rc;
   }
   // pass a over the ranks: participants, members and the largest log-weight of every site
   std::vector<uint64_t> recA, recB;
@@ -1251,8 +1214,8 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
     sipnet_gpu_handle *h = c->local[i].h;
     CUDA_OK(cudaSetDevice(h->device));
     CUDA_OK(cudaMemcpyAsync(h->rsLmax, lmax.data(), (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    if (int rc = launched(h, rs::launch_weights(args[i], 1, h->stream))) return rc;
-    if (int rc = launched(h, rs::launch_site(args[i], 1, h->stream))) return rc;
+    if (int rc = launched(h, rs::launch_weights(args[i], 1, h->stream), "resampling")) return rc;
+    if (int rc = launched(h, rs::launch_site(args[i], 1, h->stream), "resampling")) return rc;
   }
   // pass b over the ranks: ESS, the decision and the slot ranges of every site (integer sums: any order, same bits)
   if (int rc = site_records(c, recB)) return rc;
@@ -1350,8 +1313,8 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
     a.src = reinterpret_cast<double *const *>(t + at[13]);
     a.sendBuf = h->rsSend;
     a.nOut = outPre[(size_t)S];
-    if (int rc = launched(h, rs::launch_prefix(a, h->stream))) return rc;
-    if (int rc = launched(h, rs::launch_pack(a, h->stream))) return rc;
+    if (int rc = launched(h, rs::launch_prefix(a, h->stream), "resampling")) return rc;
+    if (int rc = launched(h, rs::launch_pack(a, h->stream), "resampling")) return rc;
   }
   // the segments between ranks
   if (R > 1 && c->loopback) {
@@ -1386,7 +1349,7 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
   for (size_t i = 0; i < L; ++i) {
     sipnet_gpu_handle *h = c->local[i].h;
     CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = launched(h, rs::launch_unpack(args[i], h->stream))) return rc;
+    if (int rc = launched(h, rs::launch_unpack(args[i], h->stream), "resampling")) return rc;
   }
   // the ancestors of the whole team, and the distinct ancestors of every resampled site
   ancAll.assign((size_t)rankBase[(size_t)R], -1);
@@ -1420,10 +1383,7 @@ extern "C" int sipnet_gpu_resample(sipnet_gpu_handle *h, const double *u, double
                                    int64_t *ancestors, double *diag) {
   if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
   if (int rc = check_resample(h, u, h->nsites, ess_fraction, log_weights)) return rc;
-  sipnet_gpu_comm one;
-  one.local.resize(1);
-  one.local[0].h = h;
-  one.memberCounts.assign(1, h->nmembers);
+  sipnet_gpu_comm one = team_of_one(h);
   std::vector<int64_t> anc;
   if (int rc = run_resample(&one, u, ess_fraction, {log_weights}, diag, anc)) return rc;
   if (ancestors) memcpy(ancestors, anc.data(), anc.size() * sizeof(int64_t));
@@ -1436,16 +1396,7 @@ extern "C" int sipnet_gpu_comm_resample(sipnet_gpu_comm *c, const double *u, dou
   sipnet_gpu_handle *h = c->local[0].h;
   const int64_t S = h->nsites;
   const int bad = check_resample(h, u, S, ess_fraction, log_weights);
-  uint64_t hash = 0;
-  if (!bad) {
-    const int64_t words = rs::record_words(h);
-    hash = fnv1a(0xcbf29ce484222325ull, &S, sizeof S);
-    hash = fnv1a(hash, &words, sizeof words);
-    hash = fnv1a(hash, &ess_fraction, sizeof ess_fraction);
-    hash = fnv1a(hash, u, (size_t)S * sizeof(double));
-    hash = hash == 0 ? 1 : hash;
-  }
-  if (int rc = team_agree(c, bad, hash, "resampling arguments")) return rc;
+  if (int rc = team_agree(c, bad, bad ? 0 : resample_hash(h, u, ess_fraction), "resampling arguments")) return rc;
   std::vector<int64_t> anc;
   if (int rc = run_resample(c, u, ess_fraction, std::vector<const double *>(c->local.size(), log_weights), diag, anc))
     return rc;
@@ -1461,14 +1412,9 @@ extern "C" int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, d
   // configuration index of every device's members
   std::vector<std::vector<int64_t>> glob(D);
   for (size_t d = 0; d < D; ++d) {
-    const sipnet_gpu_multi::Part &p = m->parts[d];
     glob[d].resize((size_t)m->handles[d]->nmembers);
-    if (!m->split) {
-      std::iota(glob[d].begin(), glob[d].end(), p.member0);
-    } else {
-      for (size_t s = 0; s < p.siteCount.size(); ++s)
-        for (int64_t i = 0; i < p.siteCount[s]; ++i) glob[d][(size_t)(p.siteLocal0[s] + i)] = p.siteGlobal0[s] + i;
-    }
+    for (const sipnet_gpu_multi::Run &r : m->parts[d].runs)
+      std::iota(glob[d].begin() + r.local0, glob[d].begin() + r.local0 + r.count, r.global0);
   }
   // the log-weights per device, checked here: a device must not resample before another one rejects the call
   std::vector<double> all;
@@ -1515,10 +1461,7 @@ extern "C" int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, d
   }
   // whole sites: each device alone on its site range
   for (size_t d = 0; d < D; ++d) {
-    sipnet_gpu_comm one;
-    one.local.resize(1);
-    one.local[0].h = m->handles[d];
-    one.memberCounts.assign(1, m->handles[d]->nmembers);
+    sipnet_gpu_comm one = team_of_one(m->handles[d]);
     const size_t s0 = (size_t)m->parts[d].site0;
     if (int rc = run_resample(&one, u + s0, ess_fraction, {lw[d].data()}, diag ? diag + s0 * 4 : nullptr, anc)) return rc;
     if (ancestors)
@@ -1565,18 +1508,14 @@ int check_jitter(const sipnet_gpu_jitter_spec *sp, int64_t nsites, int64_t nmemb
 }
 
 uint64_t jitter_hash(const sipnet_gpu_jitter_spec *sp, int64_t nsites) {
-  uint64_t h = 0xcbf29ce484222325ull;
-  h = fnv1a(h, &nsites, sizeof nsites);
-  h = fnv1a(h, &sp->n_rows, sizeof sp->n_rows);
-  h = fnv1a(h, sp->rows, (size_t)sp->n_rows * sizeof(int32_t));
-  h = fnv1a(h, sp->transform, (size_t)sp->n_rows * sizeof(int32_t));
+  ArgHash h;
+  h.add(&nsites, sizeof nsites)
+      .add(&sp->n_rows, sizeof sp->n_rows)
+      .add(sp->rows, (size_t)sp->n_rows * sizeof(int32_t))
+      .add(sp->transform, (size_t)sp->n_rows * sizeof(int32_t));
   for (int j = 0; j < sp->n_rows; ++j)
-    if (sp->transform[j] == SIPNET_GPU_TF_LOGIT) {
-      h = fnv1a(h, &sp->lower[j], sizeof(double));
-      h = fnv1a(h, &sp->upper[j], sizeof(double));
-    }
-  h = fnv1a(h, sp->shrink, (size_t)nsites * sizeof(double));
-  return h == 0 ? 1 : h;
+    if (sp->transform[j] == SIPNET_GPU_TF_LOGIT) h.add(&sp->lower[j], sizeof(double)).add(&sp->upper[j], sizeof(double));
+  return h.add(sp->shrink, (size_t)nsites * sizeof(double)).value();
 }
 
 // Move every local rank of `c` (all ranks hold the same sites): shrink holds the handles' sites, z[i] local rank i's
@@ -1594,7 +1533,8 @@ int run_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *sp, const d
     if (h->nsites != S) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites");
     CUDA_OK(cudaSetDevice(h->device));
     if (int rc = jt::ensure_scratch(h)) return rc;
-    if (R > 1 && !l.jtAll) CUDA_OK(cudaMalloc((void **)&l.jtAll, (size_t)R * S * jt::kRec * sizeof(double)));
+    if (R > 1)
+      if (int rc = grow(l.xchg, l.xchgCap, (size_t)R * S * jt::kRec * sizeof(double), h->stream)) return rc;
     CUDA_OK(cudaMemcpyAsync(h->jtShrink, shrink, (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CUDA_OK(cudaMemcpyAsync(h->jtZ, z[i], (size_t)n * h->nmembers * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     jt::Args &a = args[i];
@@ -1605,9 +1545,9 @@ int run_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *sp, const d
     a.nmembers = h->nmembers;
     a.sites = h->sites;
     a.nsites = (int32_t)S;
-    a.nchunks = (int32_t)h->asChunks;
-    a.chunk = h->asChunk;
-    a.siteChunks = h->asSiteChunks;
+    a.nchunks = (int32_t)h->nchunks;
+    a.chunk = h->chunk;
+    a.siteChunks = h->siteChunks;
     a.nrows = n;
     a.nranks = R;
     a.rank = l.rank;
@@ -1623,26 +1563,22 @@ int run_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *sp, const d
     a.mom = h->jtMom;
     a.coef = h->jtCoef;
     a.diag = h->jtDiag;
-    a.rankRec = l.jtAll;
+    a.rankRec = reinterpret_cast<double *>(l.xchg);
   }
-  auto launched = [](sipnet_gpu_handle *h, cudaError_t e) {
-    h->launches++;
-    return e == cudaSuccess ? 0 : fail(SIPNET_GPU_ERR_NO_DEVICE, "rejuvenation launch failed: %s", cudaGetErrorString(e));
-  };
   for (int pass = 1; pass <= 3; ++pass) {
     for (size_t i = 0; i < c->local.size(); ++i) {
       sipnet_gpu_handle *h = c->local[i].h;
       CUDA_OK(cudaSetDevice(h->device));
-      if (int rc = launched(h, jt::launch_members(args[i], pass, h->stream))) return rc;
-      if (int rc = launched(h, jt::launch_site(args[i], pass, h->stream))) return rc;
+      if (int rc = launched(h, jt::launch_members(args[i], pass, h->stream), "rejuvenation")) return rc;
+      if (int rc = launched(h, jt::launch_site(args[i], pass, h->stream), "rejuvenation")) return rc;
     }
     if (R > 1) {
-      if (int rc = all_gather_bytes(c, (size_t)S * jt::kRec * sizeof(double), [](Local &l) -> void * { return l.jtAll; }))
+      if (int rc = all_gather_bytes(c, (size_t)S * jt::kRec * sizeof(double), [](Local &l) -> void * { return l.xchg; }))
         return rc;
       for (size_t i = 0; i < c->local.size(); ++i) {
         sipnet_gpu_handle *h = c->local[i].h;
         CUDA_OK(cudaSetDevice(h->device));
-        if (int rc = launched(h, jt::launch_combine(args[i], pass, h->stream))) return rc;
+        if (int rc = launched(h, jt::launch_combine(args[i], pass, h->stream), "rejuvenation")) return rc;
       }
     }
   }
@@ -1659,9 +1595,7 @@ int run_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *sp, const d
 extern "C" int sipnet_gpu_rejuvenate(sipnet_gpu_handle *h, const sipnet_gpu_jitter_spec *spec, double *diag) {
   if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
   if (int rc = check_jitter(spec, h->nsites, h->nmembers)) return rc;
-  sipnet_gpu_comm one;
-  one.local.resize(1);
-  one.local[0].h = h;
+  sipnet_gpu_comm one = team_of_one(h);
   return run_rejuvenate(&one, spec, spec->shrink, {spec->z}, diag);
 }
 
@@ -1681,18 +1615,11 @@ extern "C" int sipnet_gpu_multi_rejuvenate(sipnet_gpu_multi *m, const sipnet_gpu
   // every device's normals, [n_rows][its members], from the configuration-order z
   std::vector<std::vector<double>> zd(D);
   for (size_t d = 0; d < D; ++d) {
-    const sipnet_gpu_multi::Part &p = m->parts[d];
     const size_t nm = (size_t)m->handles[d]->nmembers;
     zd[d].resize(n * nm);
-    for (size_t j = 0; j < n; ++j) {
-      const double *zj = spec->z + j * M;
-      if (!m->split) {
-        memcpy(zd[d].data() + j * nm, zj + p.member0, nm * sizeof(double));
-      } else {
-        for (size_t s = 0; s < p.siteCount.size(); ++s)
-          memcpy(zd[d].data() + j * nm + p.siteLocal0[s], zj + p.siteGlobal0[s], (size_t)p.siteCount[s] * sizeof(double));
-      }
-    }
+    for (size_t j = 0; j < n; ++j)
+      for (const sipnet_gpu_multi::Run &r : m->parts[d].runs)
+        memcpy(zd[d].data() + j * nm + r.local0, spec->z + j * M + r.global0, (size_t)r.count * sizeof(double));
   }
   if (m->split) {  // every device ends with the same diagnostics: take device 0's
     std::vector<const double *> ptrs;
@@ -1701,9 +1628,7 @@ extern "C" int sipnet_gpu_multi_rejuvenate(sipnet_gpu_multi *m, const sipnet_gpu
   }
   // whole sites: each device alone on its site range
   for (size_t d = 0; d < D; ++d) {
-    sipnet_gpu_comm one;
-    one.local.resize(1);
-    one.local[0].h = m->handles[d];
+    sipnet_gpu_comm one = team_of_one(m->handles[d]);
     const size_t s0 = (size_t)m->parts[d].site0;
     if (int rc = run_rejuvenate(&one, spec, spec->shrink + s0, {zd[d].data()}, diag ? diag + s0 * 4 : nullptr)) return rc;
   }

@@ -56,13 +56,14 @@ struct sipnet_gpu_handle {
   std::vector<sip::SiteDev> hostSites;
   bool mixedBlocks = false;          // some block holds members of two sites
   sip::StepConsts kc = {};           // launch-lifetime constants of the step (device-evaluated at init)
+  // the chunk tables of the ensemble filters (sip::ensure_chunks), made by the first filter call
+  int64_t nchunks = 0;
+  int2 *chunk = nullptr, *siteChunks = nullptr;
   // ensemble adjustment Kalman filter scratch (sip_assim.cu), made by the first assimilation
-  int64_t asChunks = 0;
   int asObsCap = 0;
-  int2 *asChunk = nullptr, *asSiteChunks = nullptr;
   double *asPart = nullptr, *asMom = nullptr, *asCoef = nullptr, *asObs = nullptr, *asDiag = nullptr;
   // particle filter scratch (sip_resample.cu), made by the first resampling; the tables and the record buffers grow
-  uint64_t *rsW = nullptr, *rsC = nullptr, *rsSite = nullptr;
+  uint64_t *rsW = nullptr, *rsC = nullptr, *rsSite = nullptr, *rsPart = nullptr;
   double *rsLogw = nullptr, *rsLmax = nullptr, *rsSend = nullptr, *rsRecv = nullptr;
   int64_t *rsAnc = nullptr, *rsTab = nullptr;
   size_t rsSiteCap = 0, rsTabCap = 0, rsSendCap = 0, rsRecvCap = 0;  // elements
@@ -75,4 +76,13 @@ namespace sip {
 int fail(int code, const char *fmt, ...);
 // queue the local row summaries of the last run range (sipnet_gpu.cu)
 int ensure_summaries(sipnet_gpu_handle *h);
+
+// The ensemble filters (sip_assim.cu, sip_resample.cu, sip_jitter.cu) reduce over chunks of kChunk consecutive
+// SITE-LOCAL member indices, so their sums depend on a site's members and not on the handle's block layout.
+constexpr int kChunk = 128;
+// members no filter counts or changes
+constexpr uint32_t kExcluded = SIPNET_GPU_ST_BAD_ALLOCATION | SIPNET_GPU_ST_NONFINITE;
+// the handle's chunk tables, made once (sipnet_gpu.cu): chunk[nchunks] = (site, first site-local member),
+// siteChunks[nsites] = (first chunk, chunk count), sites in order and a site's chunks in member order
+int ensure_chunks(sipnet_gpu_handle *h);
 }  // namespace sip

@@ -252,9 +252,9 @@ __global__ void __launch_bounds__(kSiteThreads) combine_kernel(const Args a) {
 }  // namespace
 
 int ensure_scratch(sipnet_gpu_handle *h) {
-  if (int rc = as::ensure_scratch(h, 0)) return rc;  // the chunk tables
+  if (int rc = ensure_chunks(h)) return rc;
   if (h->jtPart) return 0;
-  const size_t S = (size_t)h->nsites, nc = (size_t)std::max<int64_t>(h->asChunks, 1);
+  const size_t S = (size_t)h->nsites, nc = (size_t)std::max<int64_t>(h->nchunks, 1);
   cudaError_t e = cudaMalloc((void **)&h->jtPart, nc * kRec * sizeof(double));
   if (e == cudaSuccess) e = cudaMalloc((void **)&h->jtMom, S * kRec * sizeof(double));
   if (e == cudaSuccess) e = cudaMalloc((void **)&h->jtCoef, S * kCoef * sizeof(double));

@@ -12,7 +12,7 @@
 //   site(3)         -> per site diagnostics {N, rank, moved, kept} (team: + combine)
 // Six launches on one GPU, whatever the number of sites.
 //
-// Reduction order: the EAKF's 128-member chunks of site-local indices (sipnet_gpu_handle::asChunk).  Inside a chunk,
+// Reduction order: the handle's 128-member chunks of site-local indices (sipnet_gpu_handle::chunk).  Inside a chunk,
 // a lane sums one quantity over the chunk's members in index order; a site sums its chunks in chunk order; a team
 // sums the ranks' partials in rank order.  No floating-point atomics: the same members of a site give the same bits
 // in any handle.
@@ -21,7 +21,6 @@
 
 #include <cstdint>
 
-#include "sip_assim.cuh"
 #include "sip_handle.h"
 
 namespace sip {
@@ -31,8 +30,6 @@ constexpr int kMaxRows = 16;
 constexpr int kTri = kMaxRows * (kMaxRows + 1) / 2;  // lower triangle of V (l <= j), row-major
 constexpr int kSum0 = 1 + kMaxRows;                  // first cross sum in a record
 constexpr int kRec = kSum0 + kTri;                   // doubles per chunk / site / rank record: N, sums of phi, cross sums
-constexpr int kChunk = as::kChunk;
-constexpr uint32_t kExcluded = as::kExcluded;
 
 // Coefficient record of a site (doubles): [0] 1 = the site moves  [1] a  [2] rank
 //   [3 + j] (1 - a) mean_j  [3 + kMaxRows + tri(j, m)] h L_jm
@@ -64,7 +61,7 @@ struct Args {
   double *rankRec;       // [nranks][nsites][kRec] (teams only)
 };
 
-// the handle's scratch (made once, by the first call)
+// the handle's chunk tables and scratch (made once, by the first call)
 int ensure_scratch(sipnet_gpu_handle *h);
 // pass 1 / 2 / 3
 cudaError_t launch_members(const Args &a, int pass, cudaStream_t stream);

@@ -67,7 +67,7 @@ __global__ void __launch_bounds__(kWarps * 32) weights_kernel(const Args a) {
       T += W;
     }
   }
-  uint64_t *p = a.part + (size_t)c * kPartStride;
+  uint64_t *p = a.part + (size_t)c * (kRec + 1);
   if (PASS == 0) {
     for (int off = 16; off > 0; off >>= 1) {
       n += shfl_xor(n, off);
@@ -111,7 +111,7 @@ __global__ void __launch_bounds__(kWarps * 32) site_kernel(const Args a) {
     uint64_t n = 0, inf = 0;
     double mx = -INFINITY;
     for (int c = lane; c < sc.y; c += 32) {
-      const uint64_t *p = a.part + (size_t)(sc.x + c) * kPartStride;
+      const uint64_t *p = a.part + (size_t)(sc.x + c) * (kRec + 1);
       n += p[0];
       mx = fmax(mx, __longlong_as_double((long long)p[1]));
       inf |= p[3];
@@ -135,7 +135,7 @@ __global__ void __launch_bounds__(kWarps * 32) site_kernel(const Args a) {
     const int c = c0 + lane;
     uint64_t t = 0;
     if (c < sc.y) {
-      uint64_t *p = a.part + (size_t)(sc.x + c) * kPartStride;
+      uint64_t *p = a.part + (size_t)(sc.x + c) * (kRec + 1);
       s1 += (u128)p[1] << 64 | p[0];
       s2 += (u128)p[3] << 64 | p[2];
       t = p[4];
@@ -145,7 +145,7 @@ __global__ void __launch_bounds__(kWarps * 32) site_kernel(const Args a) {
       const uint64_t o = __shfl_up_sync(kFull, incl, off);
       if (lane >= off) incl += o;
     }
-    if (c < sc.y) a.part[(size_t)(sc.x + c) * kPartStride + kRec] = carry + incl - t;
+    if (c < sc.y) a.part[(size_t)(sc.x + c) * (kRec + 1) + kRec] = carry + incl - t;
     carry += __shfl_sync(kFull, incl, 31);
   }
   uint64_t v[4] = {(uint64_t)s1, (uint64_t)(s1 >> 64), (uint64_t)s2, (uint64_t)(s2 >> 64)};
@@ -175,7 +175,7 @@ __global__ void __launch_bounds__(kWarps * 32) prefix_kernel(const Args a) {
   const int2 ch = a.chunk[c];
   if (!a.flag[ch.x]) return;
   const int32_t member0 = a.sites[ch.x].member0, count = a.sites[ch.x].memberCount;
-  uint64_t carry = (uint64_t)a.toff[ch.x] + a.part[(size_t)c * kPartStride + kRec];
+  uint64_t carry = (uint64_t)a.toff[ch.x] + a.part[(size_t)c * (kRec + 1) + kRec];
   for (int i = 0; i < kChunk / 32; ++i) {
     const int idx = ch.y + lane + 32 * i;
     const int64_t m = (int64_t)member0 + idx;
@@ -320,10 +320,11 @@ int record_words(const sipnet_gpu_handle *h) {
 }
 
 int ensure_scratch(sipnet_gpu_handle *h) {
-  if (int rc = as::ensure_scratch(h, 0)) return rc;
+  if (int rc = ensure_chunks(h)) return rc;
   if (h->rsW) return 0;
-  const size_t ld = (size_t)h->ld, S = (size_t)h->nsites;
+  const size_t ld = (size_t)h->ld, S = (size_t)h->nsites, nc = (size_t)std::max<int64_t>(h->nchunks, 1);
   cudaError_t e = cudaMalloc((void **)&h->rsW, ld * sizeof(uint64_t));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&h->rsPart, nc * (kRec + 1) * sizeof(uint64_t));
   if (e == cudaSuccess) e = cudaMalloc((void **)&h->rsC, ld * sizeof(uint64_t));
   if (e == cudaSuccess) e = cudaMalloc((void **)&h->rsLogw, ld * sizeof(double));
   if (e == cudaSuccess) e = cudaMalloc((void **)&h->rsAnc, ld * sizeof(int64_t));

@@ -20,20 +20,15 @@
 
 #include <cstdint>
 
-#include "sip_assim.cuh"
 #include "sip_handle.h"
 
 namespace sip {
 namespace rs {
 
-constexpr int kChunk = as::kChunk;  // site-local members per chunk: the EAKF's chunk tables (sipnet_gpu_handle::asChunk)
 constexpr int kRec = 6;             // uint64 words per (rank, site) record
-constexpr int kPartStride = as::kRec;  // chunk records live in the EAKF's chunk scratch (as::kRec doubles per chunk)
-static_assert(kRec + 1 <= kPartStride && sizeof(uint64_t) == sizeof(double), "a chunk record and its prefix fit the EAKF's chunk slot");
 constexpr int kFixBits = 100;     // w and w^2 are summed as floor(x 2^100)
 constexpr int kWeightBits = 40;   // W = floor(w 2^40)
 constexpr int64_t kMaxSiteMembers = int64_t(1) << 23;  // keeps T = sum W below 2^63
-constexpr uint32_t kExcluded = SIPNET_GPU_ST_BAD_ALLOCATION | SIPNET_GPU_ST_NONFINITE;
 
 // Record layouts (uint64 words):
 //   pass a  [0] participants N  [1] max l of the participants (double bits; -inf if none)  [2] members n
@@ -60,7 +55,7 @@ struct Args {
   int32_t nranks, rank;
   int64_t idBase;  // rank-major index of this rank's first member
   // scratch
-  uint64_t *part;     // [nchunks][kPartStride]: the record, then [kRec] the chunk's exclusive prefix of W in its site
+  uint64_t *part;     // [nchunks][kRec + 1]: the record, then [kRec] the chunk's exclusive prefix of W in its site
   uint64_t *w, *c;    // [ld]: W and C of every member
   uint64_t *siteRec;  // [nranks][nsites][kRec]: this rank writes its slot
   const double *lmax; // [nsites]
@@ -79,7 +74,7 @@ struct Args {
   int64_t nOut;            // outgoing records
 };
 
-// chunk tables (shared with the EAKF) and member scratch of the handle
+// the handle's chunk tables, chunk records and member scratch
 int ensure_scratch(sipnet_gpu_handle *h);
 // doubles of one member record
 int record_words(const sipnet_gpu_handle *h);

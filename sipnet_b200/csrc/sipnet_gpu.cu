@@ -343,8 +343,8 @@ static void free_handle(sipnet_gpu_handle *h) {
   void *ptrs[] = {h->params, h->state, h->ringV, h->ringW, h->status, h->memberSite, h->blocks, h->sites, h->out,
                   h->dbg,    h->counters, h->loglik, h->loglikN, h->recs, h->recCount, h->mean, h->var, h->quant,
                   h->stateBk, h->ringVBk, h->ringWBk, h->loglikBk, h->loglikNBk, h->statusBk,
-                  h->recCountBk, h->sched, h->asChunk, h->asSiteChunks, h->asPart, h->asMom, h->asCoef,
-                  h->asObs, h->asDiag, h->rsW, h->rsC, h->rsSite, h->rsLogw, h->rsLmax, h->rsSend, h->rsRecv,
+                  h->recCountBk, h->sched, h->chunk, h->siteChunks, h->asPart, h->asMom, h->asCoef,
+                  h->asObs, h->asDiag, h->rsW, h->rsC, h->rsSite, h->rsPart, h->rsLogw, h->rsLmax, h->rsSend, h->rsRecv,
                   h->rsAnc, h->rsTab, h->jtPart, h->jtMom, h->jtCoef, h->jtDiag, h->jtShrink, h->jtZ};
   for (void *p : ptrs)
     if (p) cudaFree(p);
@@ -921,6 +921,25 @@ int sip::ensure_summaries(sipnet_gpu_handle *h) {
     if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "summary launch failed: %s", cudaGetErrorString(e));
   }
   h->summariesValid = true;
+  return 0;
+}
+
+int sip::ensure_chunks(sipnet_gpu_handle *h) {
+  if (h->chunk) return 0;
+  const size_t S = (size_t)h->nsites;
+  std::vector<int2> chunk, siteChunks(S);
+  for (size_t s = 0; s < S; ++s) {
+    const int32_t cnt = h->hostSites[s].memberCount;
+    siteChunks[s] = make_int2((int)chunk.size(), (cnt + kChunk - 1) / kChunk);
+    for (int32_t i = 0; i < cnt; i += kChunk) chunk.push_back(make_int2((int)s, i));
+  }
+  cudaError_t e = cudaMalloc((void **)&h->chunk, std::max<size_t>(chunk.size(), 1) * sizeof(int2));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&h->siteChunks, S * sizeof(int2));
+  if (e == cudaSuccess && !chunk.empty())
+    e = cudaMemcpy(h->chunk, chunk.data(), chunk.size() * sizeof(int2), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(h->siteChunks, siteChunks.data(), S * sizeof(int2), cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "chunk tables: %s", cudaGetErrorString(e));
+  h->nchunks = (int64_t)chunk.size();
   return 0;
 }
 
