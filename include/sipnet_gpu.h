@@ -437,6 +437,46 @@ typedef struct sipnet_gpu_obs_spec {
 int sipnet_gpu_assimilate(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs, double *diag);
 
 /*
+ * sipnet_gpu_assimilate() with prior covariance inflation, fixed or adaptive per site (Anderson 2007, 2009).  A
+ * forecast without model error loses spread at every analysis; inflating the prior deviations keeps the filter from
+ * trusting its ensemble more than the observations.  The caller owns lambda (and lambda_sd) and carries them from
+ * call to call; the library keeps no per-site state.
+ *
+ * Participants and N are the EAKF's (above); lambda0_s is lambda[s] at the start of the call.
+ * Prior inflation, once, before observation 0, at every site with lambda0_s finite, != 1 and N >= 2 (observed or not):
+ *   xbar_j = (1/N) sum x_ji  (the EAKF's fixed-order sum);  x_ji <- xbar_j + sqrt(lambda0_s) * (x_ji - xbar_j)
+ * for every listed row j and participant i.  The EAKF then runs on the inflated state, and an inflated site counts as
+ * updated for the final floor (+0.0 and SIPNET_GPU_ST_ANALYSIS_FLOORED).  Other sites are not rewritten.
+ * Adaptive update (gamma = 1: a site's state is all local to it), at sites with lambda_sd != NULL, lambda_sd[s] > 0
+ * and lambda0_s finite, for every observation k the EAKF applies there (the pair is not skipped), in order, with
+ * ybar and s2 of that observation: d = y_obs - ybar, r its variance, sp2 = s2 / lambda0_s (the variance without this
+ * call's inflation), lp = lambda[s] and v = lambda_sd[s]^2 (current values), and
+ *   g(l) = -(l - lp)^2 / (2v) - log(l sp2 + r) / 2 - d^2 / (2 (l sp2 + r)),
+ * the log posterior of lambda under the prior N(lp, v) and the likelihood N(d; 0, l sp2 + r).  g'(l) = 0 is the cubic
+ *   2 (l - lp)(sp2 l + r)^2 + v sp2 (sp2 l + r) - v d^2 sp2 = 0.
+ *   lambda[s]    <- the argmax of g over [lambda_min, lambda_max] among the cubic's real roots inside it and the two
+ *                   bounds (a tie: the smaller l);
+ *   lambda_sd[s] <- max(sd_min, min(sd, sqrt(v / (2 D)))) with sd = lambda_sd[s], D = g(l_new) - g(l_new + sd), or
+ *                   sd where D <= 0 or D is not finite: the uncertainty never grows.
+ * Sites without the update (lambda_sd NULL or 0, lambda NaN, nothing applied) keep the bits of lambda and lambda_sd.
+ *
+ * diag is sipnet_gpu_assimilate()'s, taken after the inflation.  Rejected with SIPNET_GPU_ERR_BAD_ARGUMENT, nothing
+ * changed (state, status, lambda, lambda_sd): whatever sipnet_gpu_assimilate() rejects; a NULL infl or lambda; a
+ * lambda[s] neither NaN nor finite and > 0; bounds not finite or not 0 < lambda_min <= lambda_max; sd_min negative or
+ * not finite; a lambda_sd[s] NaN, infinite, negative, or > 0 and below sd_min; lambda_sd[s] > 0 with a finite
+ * lambda[s] outside [lambda_min, lambda_max].  A call without an inflated site takes sipnet_gpu_assimilate()'s
+ * launches; one with some lambda[s] finite and != 1 takes two more.
+ */
+typedef struct sipnet_gpu_inflation_spec {
+  double *lambda;                /* [nsites] in/out; NaN or 1 = no inflation at that site */
+  double *lambda_sd;             /* [nsites] in/out, or NULL (all fixed); 0 = fixed at that site */
+  double lambda_min, lambda_max; /* bounds of the adaptive estimate */
+  double sd_min;                 /* floor of lambda_sd where it is updated */
+} sipnet_gpu_inflation_spec;
+int sipnet_gpu_assimilate_inflated(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs,
+                                   sipnet_gpu_inflation_spec *infl, double *diag);
+
+/*
  * Sequential Monte Carlo: the bootstrap particle filter (Gordon, Salmond & Smith 1993), per site, between two run()
  * segments.  Members of a site are weighted by a log-weight and replaced by copies of well-weighted members, chosen by
  * systematic resampling.  A copy carries its parameters with its pools, so forecast -> resample cycles also filter the
@@ -618,6 +658,11 @@ int sipnet_gpu_comm_member_counts(const sipnet_gpu_comm *c, int64_t *counts /* [
  * all-gather per-site partial sums (2 x 128 B per site) and sum them in rank order, so every rank applies identical
  * coefficients; no member value leaves its GPU. */
 int sipnet_gpu_comm_assimilate(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, double *diag);
+/* Collective.  sipnet_gpu_assimilate_inflated() over the members of ALL ranks: the same spec and inflation arguments
+ * on every rank (lambda, lambda_sd and the three scalars join the compared hash); the ranks also all-gather the
+ * inflation's per-site partial sums, and every rank returns the same lambda / lambda_sd bits. */
+int sipnet_gpu_comm_assimilate_inflated(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs,
+                                        sipnet_gpu_inflation_spec *infl, double *diag);
 /* Collective.  sipnet_gpu_resample() over the members of ALL ranks, in site-local order rank by rank: u and
  * ess_fraction are the same on every rank (a mismatch, found through an all-gathered hash, fails on every rank),
  * log_weights holds the rank's own members.  ancestors receives the team's int64 [sum of member counts], rank-major
@@ -656,6 +701,9 @@ sipnet_gpu_handle *sipnet_gpu_multi_handle(sipnet_gpu_multi *m, int32_t i); /* d
 /* sipnet_gpu_assimilate() on the whole configuration (value / variance / diag in global site order): split sites go
  * through the team exchange, whole sites are updated by each device alone. */
 int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, double *diag);
+/* sipnet_gpu_assimilate_inflated() on the whole configuration (lambda / lambda_sd in global site order, as value). */
+int sipnet_gpu_multi_assimilate_inflated(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs,
+                                         sipnet_gpu_inflation_spec *infl, double *diag);
 /* sipnet_gpu_resample() on the whole configuration (u, log_weights, ancestors, diag in configuration order): split
  * sites go through the team exchange, whole sites are resampled by each device alone. */
 int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, double ess_fraction, const double *log_weights,

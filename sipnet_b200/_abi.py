@@ -201,6 +201,14 @@ class ObsSpec(C.Structure):
     ]
 
 
+class InflationSpec(C.Structure):
+    """sipnet_gpu_inflation_spec: the per-site prior inflation of sipnet_gpu_assimilate_inflated() (in/out arrays)."""
+    _fields_ = [
+        ("lambda_", C.POINTER(C.c_double)), ("lambda_sd", C.POINTER(C.c_double)),
+        ("lambda_min", C.c_double), ("lambda_max", C.c_double), ("sd_min", C.c_double),
+    ]
+
+
 class JitterSpec(C.Structure):
     """sipnet_gpu_jitter_spec: which parameter rows sipnet_gpu_rejuvenate() moves, how, and with which normals."""
     _fields_ = [

@@ -131,6 +131,10 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.sipnet_gpu_comm_assimilate.argtypes = [C.c_void_p, C.POINTER(A.ObsSpec), C.c_void_p]
     lib.sipnet_gpu_multi_assimilate.restype = C.c_int
     lib.sipnet_gpu_multi_assimilate.argtypes = [C.c_void_p, C.POINTER(A.ObsSpec), C.c_void_p]
+    for name in ("sipnet_gpu_assimilate_inflated", "sipnet_gpu_comm_assimilate_inflated",
+                 "sipnet_gpu_multi_assimilate_inflated"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [C.c_void_p, C.POINTER(A.ObsSpec), C.POINTER(A.InflationSpec), C.c_void_p]
     for name in ("sipnet_gpu_resample", "sipnet_gpu_comm_resample", "sipnet_gpu_multi_resample"):
         getattr(lib, name).restype = C.c_int
         getattr(lib, name).argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -421,11 +425,25 @@ class Ensemble:
         spec = A.ObsSpec(rows.size, _ip(rows), nobs, _dp(op), _dp(value), _dp(variance))
         return spec, (rows, op, value, variance), nobs
 
-    def _assimilate(self, fn, target, rows, op, value, variance) -> np.ndarray:
+    def _assimilate(self, fn, target, rows, op, value, variance, *infl) -> np.ndarray:
         spec, _keep, nobs = self.obs_spec(rows, op, value, variance)
         diag = np.empty((self.nsites, nobs, 4), np.float64)
-        self._check(fn(target, C.byref(spec), diag.ctypes.data))
+        self._check(fn(target, C.byref(spec), *infl, diag.ctypes.data))
         return diag
+
+    def inflation_spec(self, lam, lam_sd=None, lambda_bounds=(1.0, 100.0), sd_min=0.0):
+        """(A.InflationSpec, (lambda, lambda_sd)) for sipnet_gpu_*_assimilate_inflated: lam, lam_sd: [nsites] (lam NaN
+        or 1: no inflation; lam_sd None: all fixed, 0: fixed at that site), copied -- the call updates the copies."""
+        lam = np.array(np.broadcast_to(lam, (self.nsites,)), dtype=np.float64)
+        sd = None if lam_sd is None else np.array(np.broadcast_to(lam_sd, (self.nsites,)), dtype=np.float64)
+        lo, hi = lambda_bounds
+        spec = A.InflationSpec(_dp(lam), None if sd is None else _dp(sd), float(lo), float(hi), float(sd_min))
+        return spec, (lam, sd)
+
+    def _assimilate_inflated(self, fn, target, rows, op, value, variance, lam, lam_sd, lambda_bounds, sd_min):
+        spec, (lam, sd) = self.inflation_spec(lam, lam_sd, lambda_bounds, sd_min)
+        diag = self._assimilate(fn, target, rows, op, value, variance, C.byref(spec))
+        return diag, lam, sd
 
     def assimilate(self, rows, op, value, variance) -> np.ndarray:
         """Ensemble adjustment Kalman filter on the carried pools (sipnet_gpu_assimilate; see include/sipnet_gpu.h).
@@ -435,6 +453,19 @@ class Ensemble:
     def team_assimilate(self, rows, op, value, variance) -> np.ndarray:
         """Collective.  assimilate() over the members of every rank of the team (same arguments on every rank)."""
         return self._assimilate(self.lib.sipnet_gpu_comm_assimilate, self.comm, rows, op, value, variance)
+
+    def assimilate_inflated(self, rows, op, value, variance, lam, lam_sd=None, lambda_bounds=(1.0, 100.0), sd_min=0.0):
+        """assimilate() after a per-site prior inflation by lam, fixed or adaptive (sipnet_gpu_assimilate_inflated;
+        see include/sipnet_gpu.h).  Returns (diag, the updated lam, the updated lam_sd or None); the inputs are not
+        modified."""
+        return self._assimilate_inflated(self.lib.sipnet_gpu_assimilate_inflated, self.handle, rows, op, value,
+                                         variance, lam, lam_sd, lambda_bounds, sd_min)
+
+    def team_assimilate_inflated(self, rows, op, value, variance, lam, lam_sd=None, lambda_bounds=(1.0, 100.0),
+                                 sd_min=0.0):
+        """Collective.  assimilate_inflated() over the members of every rank (same arguments on every rank)."""
+        return self._assimilate_inflated(self.lib.sipnet_gpu_comm_assimilate_inflated, self.comm, rows, op, value,
+                                         variance, lam, lam_sd, lambda_bounds, sd_min)
 
     def _resample(self, fn, target, nmembers, u, ess_fraction, log_weights):
         u = np.ascontiguousarray(u, dtype=np.float64).reshape(-1)
@@ -678,6 +709,10 @@ class MultiEnsemble(Ensemble):
 
     def assimilate(self, rows, op, value, variance) -> np.ndarray:
         return self._assimilate(self.lib.sipnet_gpu_multi_assimilate, self.multi, rows, op, value, variance)
+
+    def assimilate_inflated(self, rows, op, value, variance, lam, lam_sd=None, lambda_bounds=(1.0, 100.0), sd_min=0.0):
+        return self._assimilate_inflated(self.lib.sipnet_gpu_multi_assimilate_inflated, self.multi, rows, op, value,
+                                         variance, lam, lam_sd, lambda_bounds, sd_min)
 
     def resample(self, u, ess_fraction: float = math.inf, log_weights=None):
         return self._resample(self.lib.sipnet_gpu_multi_resample, self.multi, self.nmembers, u, ess_fraction, log_weights)

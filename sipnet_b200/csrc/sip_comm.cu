@@ -923,25 +923,72 @@ uint64_t spec_hash(const sipnet_gpu_obs_spec *o, int64_t nsites) {
       .value();
 }
 
-// Queue the analysis on every local rank of `c`: value / variance hold the handles' sites (all ranks hold the same
-// sites).  A team of one needs no exchange and no host round trip; a larger team all-gathers each pass's per-site
-// partial sums and sums them in rank order on every rank.
-int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const double *value, const double *variance) {
+// the inflation arguments against `nsites` sites: 0, or SIPNET_GPU_ERR_BAD_ARGUMENT with the reason
+int check_inflation(const sipnet_gpu_inflation_spec *f, int64_t nsites) {
+  if (!f || !f->lambda) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL inflation spec or lambda");
+  if (!(std::isfinite(f->lambda_min) && std::isfinite(f->lambda_max) && f->lambda_min > 0.0 &&
+        f->lambda_min <= f->lambda_max))
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "lambda bounds must be finite with 0 < lambda_min <= lambda_max");
+  if (!(std::isfinite(f->sd_min) && f->sd_min >= 0.0))
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "sd_min must be finite and >= 0");
+  for (int64_t s = 0; s < nsites; ++s) {
+    const double l = f->lambda[s];
+    if (!std::isnan(l) && !(std::isfinite(l) && l > 0.0))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "lambda[%lld] = %g is neither NaN nor finite and > 0", (long long)s, l);
+    if (!f->lambda_sd) continue;
+    const double sd = f->lambda_sd[s];
+    if (!(std::isfinite(sd) && sd >= 0.0))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "lambda_sd[%lld] = %g is not finite and >= 0", (long long)s, sd);
+    if (sd > 0.0 && sd < f->sd_min)
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "lambda_sd[%lld] = %g is below sd_min", (long long)s, sd);
+    if (sd > 0.0 && std::isfinite(l) && (l < f->lambda_min || l > f->lambda_max))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "lambda[%lld] = %g is adaptive but outside the bounds", (long long)s, l);
+  }
+  return 0;
+}
+
+// the inflation arguments of sites [site0, ...): the multi-GPU partition's slice
+sipnet_gpu_inflation_spec inflation_slice(const sipnet_gpu_inflation_spec *f, int64_t site0) {
+  sipnet_gpu_inflation_spec g = *f;
+  g.lambda += site0;
+  if (g.lambda_sd) g.lambda_sd += site0;
+  return g;
+}
+
+// Queue the analysis on every local rank of `c`: value / variance (and infl, NULL = no inflation) hold the handles'
+// sites (all ranks hold the same sites).  A team of one needs no exchange and no host round trip; a larger team
+// all-gathers each pass's per-site partial sums and sums them in rank order on every rank.
+int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const double *value, const double *variance,
+                     const sipnet_gpu_inflation_spec *infl) {
   const int R = c->nranks, nobs = o->n_obs, nr = o->n_rows;
+  const int64_t S = c->local[0].h->nsites;
   std::vector<as::Args> args(c->local.size());
+  std::vector<double> f0;  // {λ0, λ, σ} per site
+  bool inflate = false;    // some site may be inflated: run the moment pass
+  if (infl) {
+    f0.resize((size_t)S * 3);
+    for (int64_t s = 0; s < S; ++s) {
+      const double l = infl->lambda[s];
+      f0[3 * s] = f0[3 * s + 1] = l;
+      f0[3 * s + 2] = infl->lambda_sd ? infl->lambda_sd[s] : 0.0;
+      inflate = inflate || (std::isfinite(l) && l != 1.0);
+    }
+  }
   for (size_t i = 0; i < c->local.size(); ++i) {
     Local &l = c->local[i];
     sipnet_gpu_handle *h = l.h;
-    if (h->nsites != c->local[0].h->nsites)
-      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites");
+    if (h->nsites != S) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites");
     CUDA_OK(cudaSetDevice(h->device));
     if (int rc = as::ensure_scratch(h, nobs)) return rc;
+    if (infl)
+      if (int rc = as::ensure_inflation(h)) return rc;
     if (R > 1)
       if (int rc = grow(l.xchg, l.xchgCap, (size_t)R * h->nsites * as::kRec * sizeof(double), h->stream)) return rc;
     const size_t nv = (size_t)h->nsites * nobs;
     CUDA_OK(cudaMemcpyAsync(h->asObs, value, nv * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CUDA_OK(cudaMemcpyAsync(h->asObs + nv, variance, nv * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CUDA_OK(cudaMemsetAsync(h->asCoef, 0, (size_t)h->nsites * as::kRec * sizeof(double), h->stream));
+    if (infl) CUDA_OK(cudaMemcpyAsync(h->asInfl, f0.data(), f0.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     as::Args &a = args[i];
     memset(&a, 0, sizeof a);
     a.state = h->state;
@@ -964,62 +1011,95 @@ int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const dou
     a.variance = h->asObs + nv;
     a.diag = h->asDiag;
     a.rankRec = reinterpret_cast<double *>(l.xchg);
+    if (infl) {
+      a.infl = h->asInfl;
+      a.lamMin = infl->lambda_min;
+      a.lamMax = infl->lambda_max;
+      a.sdMin = infl->sd_min;
+    }
   }
+  // one members pass and its site reduction on every rank; a team then exchanges and combines the site partials
+  auto run_pass = [&](int pass, bool apply, bool inflatePass) -> int {
+    for (size_t i = 0; i < c->local.size(); ++i) {
+      sipnet_gpu_handle *h = c->local[i].h;
+      CUDA_OK(cudaSetDevice(h->device));
+      if (int rc = launched(h, as::launch_members(args[i], pass, apply, false, inflatePass, h->stream), "assimilation"))
+        return rc;
+      if (int rc = launched(h, as::launch_site_reduce(args[i], pass, h->stream), "assimilation")) return rc;
+    }
+    if (R == 1) return 0;
+    const size_t bytes = (size_t)S * as::kRec * sizeof(double);
+    if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.xchg; })) return rc;
+    for (size_t i = 0; i < c->local.size(); ++i) {
+      sipnet_gpu_handle *h = c->local[i].h;
+      CUDA_OK(cudaSetDevice(h->device));
+      if (int rc = launched(h, as::launch_site_combine(args[i], pass, h->stream), "assimilation")) return rc;
+    }
+    return 0;
+  };
+  if (inflate)  // the means the inflation centres on
+    if (int rc = run_pass(as::kInflPass, false, false)) return rc;
   for (int k = 0; k < nobs; ++k) {
-    for (int pass = 1; pass <= 2; ++pass) {
-      for (size_t i = 0; i < c->local.size(); ++i) {
-        as::Args &a = args[i];
-        sipnet_gpu_handle *h = c->local[i].h;
-        a.k = k;
-        for (int j = 0; j < nr; ++j) {
-          a.opCur[j] = o->op[(size_t)k * nr + j];
-          a.opPrev[j] = k > 0 ? o->op[(size_t)(k - 1) * nr + j] : 0.0;
-        }
-        CUDA_OK(cudaSetDevice(h->device));
-        // pass 1 of observation k first applies observation k - 1
-        if (int rc = launched(h, as::launch_members(a, pass, pass == 1 && k > 0, false, h->stream), "assimilation"))
-          return rc;
-        if (int rc = launched(h, as::launch_site_reduce(a, pass, h->stream), "assimilation")) return rc;
-      }
-      if (R > 1) {
-        const size_t bytes = (size_t)args[0].nsites * as::kRec * sizeof(double);
-        if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.xchg; })) return rc;
-        for (size_t i = 0; i < c->local.size(); ++i) {
-          sipnet_gpu_handle *h = c->local[i].h;
-          CUDA_OK(cudaSetDevice(h->device));
-          if (int rc = launched(h, as::launch_site_combine(args[i], pass, h->stream), "assimilation")) return rc;
-        }
+    for (as::Args &a : args) {
+      a.k = k;
+      for (int j = 0; j < nr; ++j) {
+        a.opCur[j] = o->op[(size_t)k * nr + j];
+        a.opPrev[j] = k > 0 ? o->op[(size_t)(k - 1) * nr + j] : 0.0;
       }
     }
+    // pass 1 of observation k first applies observation k - 1, or (k = 0) the inflation
+    if (int rc = run_pass(1, k > 0, k == 0 && inflate)) return rc;
+    if (int rc = run_pass(2, false, false)) return rc;
   }
   for (size_t i = 0; i < c->local.size(); ++i) {  // the last observation's update and the floor
     as::Args &a = args[i];
     sipnet_gpu_handle *h = c->local[i].h;
     for (int j = 0; j < nr; ++j) a.opPrev[j] = o->op[(size_t)(nobs - 1) * nr + j];
     CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = launched(h, as::launch_members(a, 0, true, true, h->stream), "assimilation")) return rc;
+    if (int rc = launched(h, as::launch_members(a, 0, true, true, false, h->stream), "assimilation")) return rc;
   }
   return 0;
 }
 
-// wait for the analysis of `h`; diag (may be NULL) gets its [nsites][nobs][4] diagnostics
-int finish_assimilation(sipnet_gpu_handle *h, double *diag, int nobs) {
+// wait for the analysis of `h`; diag (may be NULL) gets its [nsites][nobs][4] diagnostics, infl (may be NULL) the
+// updated lambda / lambda_sd of its sites
+int finish_assimilation(sipnet_gpu_handle *h, double *diag, int nobs, const sipnet_gpu_inflation_spec *infl) {
   CUDA_OK(cudaSetDevice(h->device));
   if (diag)
     CUDA_OK(cudaMemcpyAsync(diag, h->asDiag, (size_t)h->nsites * nobs * 4 * sizeof(double), cudaMemcpyDeviceToHost,
                             h->stream));
+  std::vector<double> f(infl ? (size_t)h->nsites * 3 : 0);
+  if (infl) CUDA_OK(cudaMemcpyAsync(f.data(), h->asInfl, f.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CUDA_OK(cudaStreamSynchronize(h->stream));
+  for (int64_t s = 0; infl && s < h->nsites; ++s) {
+    infl->lambda[s] = f[3 * s + 1];
+    if (infl->lambda_sd) infl->lambda_sd[s] = f[3 * s + 2];
+  }
   return 0;
+}
+
+// sipnet_gpu_assimilate(), with the inflation unless infl is NULL (the same for the comm and multi variants below)
+int assimilate_handle(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs, sipnet_gpu_inflation_spec *infl,
+                      double *diag) {
+  if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  if (int rc = check_obs(obs, h->nsites)) return rc;
+  if (infl)
+    if (int rc = check_inflation(infl, h->nsites)) return rc;
+  sipnet_gpu_comm one = team_of_one(h);
+  if (int rc = run_assimilation(&one, obs, obs->value, obs->variance, infl)) return rc;
+  return finish_assimilation(h, diag, obs->n_obs, infl);
 }
 
 }  // namespace
 
 extern "C" int sipnet_gpu_assimilate(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs, double *diag) {
-  if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
-  if (int rc = check_obs(obs, h->nsites)) return rc;
-  sipnet_gpu_comm one = team_of_one(h);
-  if (int rc = run_assimilation(&one, obs, obs->value, obs->variance)) return rc;
-  return finish_assimilation(h, diag, obs->n_obs);
+  return assimilate_handle(h, obs, nullptr, diag);
+}
+
+extern "C" int sipnet_gpu_assimilate_inflated(sipnet_gpu_handle *h, const sipnet_gpu_obs_spec *obs,
+                                              sipnet_gpu_inflation_spec *infl, double *diag) {
+  if (!infl) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL inflation spec");
+  return assimilate_handle(h, obs, infl, diag);
 }
 
 // Collective: every rank sees every rank's argument hash (`mine`; 0 = this rank's arguments are invalid, with the
@@ -1047,37 +1127,82 @@ static int team_agree(sipnet_gpu_comm *c, int bad, uint64_t mine, const char *wh
   return bad;
 }
 
-extern "C" int sipnet_gpu_comm_assimilate(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, double *diag) {
+namespace {
+
+// the spec's hash, extended by the inflation arguments (infl NULL: spec_hash)
+uint64_t assim_hash(const sipnet_gpu_obs_spec *o, const sipnet_gpu_inflation_spec *f, int64_t nsites) {
+  const uint64_t h0 = spec_hash(o, nsites);
+  if (!f) return h0;
+  const uint8_t hasSd = f->lambda_sd != nullptr;
+  ArgHash h;
+  h.add(&h0, sizeof h0).add(f->lambda, (size_t)nsites * sizeof(double)).add(&hasSd, 1);
+  if (hasSd) h.add(f->lambda_sd, (size_t)nsites * sizeof(double));
+  return h.add(&f->lambda_min, sizeof(double)).add(&f->lambda_max, sizeof(double)).add(&f->sd_min, sizeof(double))
+      .value();
+}
+
+int assimilate_comm(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, sipnet_gpu_inflation_spec *infl,
+                    double *diag) {
   if (!c) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL comm");
   const int64_t S = c->local[0].h->nsites;
-  const int bad = check_obs(obs, S);
-  if (int rc = team_agree(c, bad, bad ? 0 : spec_hash(obs, S), "observation specs")) return rc;
-  if (int rc = run_assimilation(c, obs, obs->value, obs->variance)) return rc;
+  int bad = check_obs(obs, S);
+  if (!bad && infl) bad = check_inflation(infl, S);
+  if (int rc = team_agree(c, bad, bad ? 0 : assim_hash(obs, infl, S), "observation specs")) return rc;
+  if (int rc = run_assimilation(c, obs, obs->value, obs->variance, infl)) return rc;
   for (Local &l : c->local)
-    if (int rc = finish_assimilation(l.h, diag, obs->n_obs)) return rc;
+    if (int rc = finish_assimilation(l.h, diag, obs->n_obs, infl)) return rc;
   return 0;
 }
 
-extern "C" int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, double *diag) {
+int assimilate_multi(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, sipnet_gpu_inflation_spec *infl,
+                     double *diag) {
   if (!m) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
   if (int rc = check_obs(obs, m->nsites)) return rc;
+  if (infl)
+    if (int rc = check_inflation(infl, m->nsites)) return rc;
   const int nobs = obs->n_obs;
-  if (m->split) {  // every device ends with the same diagnostics: take device 0's
-    if (int rc = run_assimilation(m->comm, obs, obs->value, obs->variance)) return rc;
+  if (m->split) {  // every device ends with the same diagnostics and inflation: take device 0's
+    if (int rc = run_assimilation(m->comm, obs, obs->value, obs->variance, infl)) return rc;
     for (size_t d = 0; d < m->handles.size(); ++d)
-      if (int rc = finish_assimilation(m->handles[d], d == 0 ? diag : nullptr, nobs)) return rc;
+      if (int rc = finish_assimilation(m->handles[d], d == 0 ? diag : nullptr, nobs, d == 0 ? infl : nullptr)) return rc;
     return 0;
   }
   // whole sites: each device alone on its site range, all devices side by side
+  std::vector<sipnet_gpu_inflation_spec> slice(m->handles.size());
   for (size_t d = 0; d < m->handles.size(); ++d) {
     const size_t off = (size_t)m->parts[d].site0 * nobs;
+    if (infl) slice[d] = inflation_slice(infl, m->parts[d].site0);
     sipnet_gpu_comm one = team_of_one(m->handles[d]);
-    if (int rc = run_assimilation(&one, obs, obs->value + off, obs->variance + off)) return rc;
+    if (int rc = run_assimilation(&one, obs, obs->value + off, obs->variance + off, infl ? &slice[d] : nullptr))
+      return rc;
   }
   for (size_t d = 0; d < m->handles.size(); ++d)
-    if (int rc = finish_assimilation(m->handles[d], diag ? diag + (size_t)m->parts[d].site0 * nobs * 4 : nullptr, nobs))
+    if (int rc = finish_assimilation(m->handles[d], diag ? diag + (size_t)m->parts[d].site0 * nobs * 4 : nullptr, nobs,
+                                     infl ? &slice[d] : nullptr))
       return rc;
   return 0;
+}
+
+}  // namespace
+
+extern "C" int sipnet_gpu_comm_assimilate(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, double *diag) {
+  return assimilate_comm(c, obs, nullptr, diag);
+}
+
+extern "C" int sipnet_gpu_comm_assimilate_inflated(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs,
+                                                   sipnet_gpu_inflation_spec *infl, double *diag) {
+  if (!infl) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL inflation spec");
+  return assimilate_comm(c, obs, infl, diag);
+}
+
+extern "C" int sipnet_gpu_multi_assimilate(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, double *diag) {
+  return assimilate_multi(m, obs, nullptr, diag);
+}
+
+extern "C" int sipnet_gpu_multi_assimilate_inflated(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs,
+                                                    sipnet_gpu_inflation_spec *infl, double *diag) {
+  if (!infl) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL inflation spec");
+  return assimilate_multi(m, obs, infl, diag);
 }
 
 // ---- the particle filter: per-site systematic resampling (sip_resample.cuh) ---------------------------------------

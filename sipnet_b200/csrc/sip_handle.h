@@ -62,6 +62,7 @@ struct sipnet_gpu_handle {
   // ensemble adjustment Kalman filter scratch (sip_assim.cu), made by the first assimilation
   int asObsCap = 0;
   double *asPart = nullptr, *asMom = nullptr, *asCoef = nullptr, *asObs = nullptr, *asDiag = nullptr;
+  double *asInfl = nullptr;  // [nsites][3] {λ0, λ, σ} of the prior inflation, made by the first inflated call
   // particle filter scratch (sip_resample.cu), made by the first resampling; the tables and the record buffers grow
   uint64_t *rsW = nullptr, *rsC = nullptr, *rsSite = nullptr, *rsPart = nullptr;
   double *rsLogw = nullptr, *rsLmax = nullptr, *rsSend = nullptr, *rsRecv = nullptr;

@@ -344,7 +344,7 @@ static void free_handle(sipnet_gpu_handle *h) {
                   h->dbg,    h->counters, h->loglik, h->loglikN, h->recs, h->recCount, h->mean, h->var, h->quant,
                   h->stateBk, h->ringVBk, h->ringWBk, h->loglikBk, h->loglikNBk, h->statusBk,
                   h->recCountBk, h->sched, h->chunk, h->siteChunks, h->asPart, h->asMom, h->asCoef,
-                  h->asObs, h->asDiag, h->rsW, h->rsC, h->rsSite, h->rsPart, h->rsLogw, h->rsLmax, h->rsSend, h->rsRecv,
+                  h->asObs, h->asDiag, h->asInfl, h->rsW, h->rsC, h->rsSite, h->rsPart, h->rsLogw, h->rsLmax, h->rsSend, h->rsRecv,
                   h->rsAnc, h->rsTab, h->jtPart, h->jtMom, h->jtCoef, h->jtDiag, h->jtShrink, h->jtZ};
   for (void *p : ptrs)
     if (p) cudaFree(p);

@@ -1,7 +1,11 @@
 """Device time of sipnet_gpu_assimilate (the ensemble adjustment Kalman filter, sip_assim.cu) on one GPU's share of
 the C4 and C3 workloads, beside the forecast pass of the same handle.
 
-    python tools/assimilate_timing.py [--calls 20] [--warmup 3] [--out FILE.json]
+    python tools/assimilate_timing.py [--calls 20] [--warmup 3] [--inflation none,fixed,adaptive] [--out FILE.json]
+
+--inflation times sipnet_gpu_assimilate_inflated as well, on the same handle after the same forecast: `fixed` inflates
+every site by lambda = 1.5 (two more launches), `adaptive` also updates lambda (sd 0.5, bounds [1, 100]); every call
+gets the same inputs.  `none` is the plain call.
 
 Shapes: C4 share = 1 site x 131 072 members (the bench workload per GPU, 10-year forecast); C3 share = 2 500 sites x
 100 members (1-year forecast); synthetic forcing without an event schedule (its harvest would leave the plant pools
@@ -64,53 +68,75 @@ def observations(state, ms, nsites, op):
     return value, var
 
 
-def measure(name, sites, P, ms, calls, warmup) -> dict:
+MODES = ("none", "fixed", "adaptive")
+
+
+def analysis(e, mode, rows, op, value, var):
+    """One call of the mode, as a function of nothing."""
+    n = e.nsites
+    if mode == "none":
+        return lambda: e.assimilate(rows, op, value, var)
+    sd = np.full(n, 0.5) if mode == "adaptive" else None
+    return lambda: e.assimilate_inflated(rows, op, value, var, np.full(n, 1.5), sd)
+
+
+def measure(name, sites, P, ms, calls, warmup, modes) -> list:
     nsites = len(sites)
+    lines = []
     with api.Ensemble(sites, P, ms, synth.SYNTH_FLAGS, outputs=0, math=A.MATH_FAST) as e:
         e.run()
         forecast_ms = e.last_run_ms()
         op = operator()
         value, var = observations(e.state(), ms, nsites, op)
         rows = list(range(NROWS))
-        times = []
-        launches = e.launch_count()
-        for i in range(warmup + calls):
-            e.timer_start()
-            e.assimilate(rows, op, value, var)
-            ms_ = e.timer_stop_ms()
-            if i >= warmup:
-                times.append(ms_)
-        launches = (e.launch_count() - launches) // (warmup + calls)
         M = e.nmembers
-    per_member_read = NROWS * 8 + 4
-    read = (2 * NOBS + 1) * per_member_read * M
-    written = NOBS * NROWS * 8 * M
-    med = float(np.median(times))
-    return {"shape": name, "sites": nsites, "members": M, "rows": NROWS, "observations": NOBS,
-            "assimilate_ms_median": med, "assimilate_ms_min": float(np.min(times)),
-            "assimilate_ms_max": float(np.max(times)), "calls": calls, "warmup": warmup,
-            "launches_per_call": int(launches), "forecast_pass_ms": forecast_ms,
-            "forecast_steps": int(max(s.nsteps for s in sites)),
-            "analysis_over_forecast": med / forecast_ms if forecast_ms > 0 else None,
-            "rows_bytes": NROWS * 8 * M, "bytes_read": read, "bytes_written": written,
-            "note": "rows L2-resident after the forecast; bytes computed from the shapes"}
+        for mode in modes:
+            call = analysis(e, mode, rows, op, value, var)
+            times = []
+            launches = e.launch_count()
+            for i in range(warmup + calls):
+                e.timer_start()
+                call()
+                ms_ = e.timer_stop_ms()
+                if i >= warmup:
+                    times.append(ms_)
+            launches = (e.launch_count() - launches) // (warmup + calls)
+            passes = 2 * NOBS + 1 + (1 if mode != "none" else 0)     # members passes; the inflation adds one
+            per_member_read = NROWS * 8 + 4
+            read = passes * per_member_read * M
+            written = (NOBS + (1 if mode != "none" else 0)) * NROWS * 8 * M
+            med = float(np.median(times))
+            lines.append({"shape": name, "inflation": mode, "sites": nsites, "members": M, "rows": NROWS,
+                          "observations": NOBS, "assimilate_ms_median": med, "assimilate_ms_min": float(np.min(times)),
+                          "assimilate_ms_max": float(np.max(times)), "calls": calls, "warmup": warmup,
+                          "launches_per_call": int(launches), "forecast_pass_ms": forecast_ms,
+                          "forecast_steps": int(max(s.nsteps for s in sites)),
+                          "analysis_over_forecast": med / forecast_ms if forecast_ms > 0 else None,
+                          "rows_bytes": NROWS * 8 * M, "bytes_read": read, "bytes_written": written,
+                          "note": "rows L2-resident after the forecast; bytes computed from the shapes"})
+    return lines
 
 
 def main() -> None:
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--calls", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--inflation", default="none",
+                    help="comma-separated modes to time, each of none, fixed, adaptive (default: none)")
     ap.add_argument("--out", default=None, help="also write the lines to this file")
     args = ap.parse_args()
+    modes = args.inflation.split(",")
+    if not modes or any(m not in MODES for m in modes):
+        ap.error(f"--inflation takes a comma-separated list of {', '.join(MODES)}")
     info = gpu_info()
     lines = []
     site = synth.synth_site(0, 10, "half-daily")
     M = 131072
-    lines.append(measure("c4_share", [site], synth.synth_params(M, stream=1), np.zeros(M, np.int32), args.calls,
-                         args.warmup))
+    lines += measure("c4_share", [site], synth.synth_params(M, stream=1), np.zeros(M, np.int32), args.calls,
+                     args.warmup, modes)
     sites = [synth.synth_site(s, 1, "half-daily") for s in range(2500)]
     P, ms = synth.synth_params(250000, stream=1), np.repeat(np.arange(2500, dtype=np.int32), 100)
-    lines.append(measure("c3_share", sites, P, ms, args.calls, args.warmup))
+    lines += measure("c3_share", sites, P, ms, args.calls, args.warmup, modes)
     for line in lines:
         line.update(info)
         print(json.dumps(line))
