@@ -131,6 +131,8 @@ struct Local {
   gs::GsTie *tieAll = nullptr;
   uint64_t *emitAll = nullptr;
   int32_t *flags = nullptr;
+  double *list = nullptr;  // candidate lists (only where they are worth their memory, see ensure_scratch)
+  int32_t *listN = nullptr;
   // [nranks][bytes per rank] of one all-gather at a time: argument hashes, the filters' per-site partials, member words
   unsigned char *xchg = nullptr;
   size_t xchgCap = 0;
@@ -153,7 +155,7 @@ namespace {
 // all scratch of `l`: the rank keeps its handle, communicator and rank
 void free_local(Local &l) {
   if (l.h) cudaSetDevice(l.h->device);
-  void *ptrs[] = {l.statAll, l.q2All, l.hist, l.state, l.tieAll, l.emitAll, l.flags, l.xchg};
+  void *ptrs[] = {l.statAll, l.q2All, l.hist, l.state, l.tieAll, l.emitAll, l.flags, l.list, l.listN, l.xchg};
   for (void *p : ptrs)
     if (p) cudaFree(p);
   l = Local{l.h, l.comm, l.rank};
@@ -235,8 +237,11 @@ int all_reduce_hist(sipnet_gpu_comm *c, size_t words) {
   return g.end();
 }
 
-int ensure_scratch(sipnet_gpu_comm *c, Local &l, int64_t rows) {
-  if (rows <= l.rowsCap) return 0;
+// Candidate lists are kept when the rank's members per site are at least 4 x kGsListCap: then a list costs at most a
+// quarter of the memory of the summary columns themselves and saves the later scans most of a row.  Whether a rank
+// keeps lists is its own choice (each rank scans its own list or row); what it compacts is decided from global counts.
+int ensure_scratch(sipnet_gpu_comm *c, Local &l, int64_t rows, bool lists) {
+  if (rows <= l.rowsCap && (!lists || l.list)) return 0;
   const int R = c->nranks;
   sipnet_gpu_handle *h = l.h;
   CUDA_OK(cudaSetDevice(h->device));
@@ -249,6 +254,10 @@ int ensure_scratch(sipnet_gpu_comm *c, Local &l, int64_t rows) {
   CUDA_OK(cudaMalloc((void **)&l.tieAll, (size_t)R * rows * gs::kGsMaxStat * sizeof(gs::GsTie)));
   CUDA_OK(cudaMalloc((void **)&l.emitAll, (size_t)R * rows * gs::kGsMaxStat * gs::kGsEmit * sizeof(uint64_t)));
   CUDA_OK(cudaMalloc((void **)&l.flags, 16));
+  if (lists) {
+    CUDA_OK(cudaMalloc((void **)&l.list, (size_t)rows * gs::kGsListCap * sizeof(double)));
+    CUDA_OK(cudaMalloc((void **)&l.listN, (size_t)rows * sizeof(int32_t)));
+  }
   l.rowsCap = rows;
   return 0;
 }
@@ -269,7 +278,8 @@ int team_summaries(sipnet_gpu_comm *c) {
     sipnet_gpu_handle *h = l.h;
     if (h->lastEnd - h->lastBegin != n || h->nsites != h0->nsites || (int)h->summaryCols.size() != ncols)
       return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites, columns and run range");
-    if (int rc = ensure_scratch(c, l, rows)) return rc;
+    const bool lists = nqTotal > 0 && h->ld >= 4 * (int64_t)gs::kGsListCap * h->nsites;
+    if (int rc = ensure_scratch(c, l, rows, lists)) return rc;
   }
   std::vector<gs::GsArgs> args(c->local.size());
   for (size_t i = 0; i < c->local.size(); ++i) {
@@ -294,6 +304,8 @@ int team_summaries(sipnet_gpu_comm *c) {
     a.tieAll = l.tieAll;
     a.emitAll = l.emitAll;
     a.flags = l.flags;
+    a.list = l.list;
+    a.listN = l.listN;
     a.mean = h->mean;
     a.var = h->var;
     a.quant = h->quant;

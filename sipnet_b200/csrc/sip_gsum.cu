@@ -13,7 +13,12 @@ namespace sip {
 namespace gs {
 
 constexpr int kThreads = 512;
-constexpr int kUnroll = 4;
+constexpr int kUnroll = 4;       // loads in flight per thread: emit and the 64-bit levels (more would spill)
+// Levels 1-2 read whole rows at 2 blocks x 512 threads per SM, where 4 loads of 8 B in flight per thread are too
+// few bytes in flight for HBM latency (level 1 on the C4 share: 4.9 -> 4.3 ms with 8; pass 0, at 3 blocks per SM,
+// takes the same loop and stays at 3.0 ms).  Element i of a row is still handled by thread i % kThreads in
+// ascending i for any unroll, so the per-thread sums -- and the moments -- are the same bits.
+constexpr int kUnrollWide = 8;
 constexpr uint64_t kSent = kGsNoKey;
 
 __host__ __device__ constexpr int bits_after(int level) { return level < 7 ? 11 + 8 * level : 64; }
@@ -31,15 +36,13 @@ __device__ __forceinline__ double val_of(uint64_t k) {
 }
 __device__ __forceinline__ bool finite_hi(double x) { return (((unsigned int)__double2hiint(x) >> 20) & 0x7ffu) != 0x7ffu; }
 
-// histogram update for all 32 lanes (code < 0: nothing to count); the lanes agreeing with lane 0 add once
+// histogram update for all 32 lanes (code < 0: nothing to count); the lanes agreeing with lane 0 add once.  One
+// predicated atomic per lane: lane 0 and the lanes that differ from it do not take separate paths.
 __device__ __forceinline__ void hist_add(unsigned int *hist, int code) {
   const int lead = __shfl_sync(0xffffffffu, code, 0);
   const unsigned same = __ballot_sync(0xffffffffu, code == lead);
-  if ((threadIdx.x & 31) == 0) {
-    if (lead >= 0) atomicAdd(&hist[lead], (unsigned)__popc(same));
-  } else if (code >= 0 && code != lead) {
-    atomicAdd(&hist[code], 1u);
-  }
+  const bool first = (threadIdx.x & 31) == 0;
+  if (code >= 0 && (first || code != lead)) atomicAdd(&hist[code], first ? (unsigned)__popc(same) : 1u);
 }
 
 __device__ __forceinline__ double block_sum(double v, double *sh) {  // fixed order
@@ -90,15 +93,15 @@ __global__ void __launch_bounds__(kThreads, 2) gs_pass0_kernel(const GsArgs a) {
   double s = 0.0, c = 0.0;
   uint64_t first = 0, diff = 0;
   bool have = false;
-  for (int i0 = 0; i0 < r.count; i0 += kUnroll * kThreads) {
-    double x[kUnroll];
+  for (int i0 = 0; i0 < r.count; i0 += kUnrollWide * kThreads) {
+    double x[kUnrollWide];
 #pragma unroll
-    for (int u = 0; u < kUnroll; ++u) {
+    for (int u = 0; u < kUnrollWide; ++u) {
       const int i = i0 + u * kThreads + tid;
       x[u] = i < r.count ? r.p[i] : __longlong_as_double(0x7ff8000000000000ll);
     }
 #pragma unroll
-    for (int u = 0; u < kUnroll; ++u) {  // per thread the elements are accumulated in index order
+    for (int u = 0; u < kUnrollWide; ++u) {  // per thread the elements are accumulated in index order
       const bool fin = finite_hi(x[u]);
       int code = -1;
       if (fin) {
@@ -163,6 +166,7 @@ __device__ void init_state(const GsArgs &a, int64_t row, int64_t rows, GsRow &S)
   S.mean = n > 0 ? sum / n : __longlong_as_double(0x7ff8000000000000ll);
   S.bits = 0;
   S.nslots = 1;
+  S.listed = 0;
   for (int i = 0; i < kGsMaxStat; ++i) {
     S.prefix[i] = 0;
     S.k[i] = 0;
@@ -256,6 +260,9 @@ __global__ void __launch_bounds__(kThreads, 2) gs_level_kernel(const GsArgs a, c
   __shared__ uint64_t slotTop[kGsMaxStat];
   __shared__ unsigned long long tieRep[kGsMaxStat];
   __shared__ unsigned int tieLo[kGsMaxStat], tieHi[kGsMaxStat];
+  __shared__ uint64_t xTop[kGsMaxStat];  // the compacting pass: bins of the statistics waiting for the emit
+  __shared__ int xSh[kGsMaxStat], nx;
+  __shared__ unsigned int listFill;
   const int tid = threadIdx.x;
   const RowRef r = row_ref(a);
   const int64_t rows = gridDim.x;
@@ -294,12 +301,42 @@ __global__ void __launch_bounds__(kThreads, 2) gs_level_kernel(const GsArgs a, c
   const bool pass = S.done == 0 && level < kGsLevels;
   const bool needSS = level == 1 && a.wantMoments && S.n > 0;
   if (tid == 0) {
+    // compact when the filter -- every slot in play and every bin waiting for the emit, each counted once -- holds
+    // at most kGsListCap keys over all ranks (the same decision on every rank: it reads exchanged data only)
+    nx = 0;
+    listFill = 0;
+    if (pass && a.list && S.listed == 0) {
+      uint64_t popSum = 0;
+      for (int q = 0; q < 2 * a.nq; ++q) {
+        bool first = true;
+        if (S.rbits[q] == 0) {
+          for (int e = 0; e < q; ++e) first = first && !(S.rbits[e] == 0 && S.slotOf[e] == S.slotOf[q]);
+          if (first) popSum += S.pop[q];
+        } else if (S.rbits[q] < 64) {
+          const int shv = 64 - (int)S.rbits[q];
+          for (int e = 0; e < nx; ++e) first = first && !(xSh[e] == shv && xTop[e] == S.prefix[q] >> shv);
+          if (first) {
+            popSum += S.pop[q];
+            xTop[nx] = S.prefix[q] >> shv;
+            xSh[nx++] = shv;
+          }
+        }
+      }
+      if (popSum <= (uint64_t)kGsListCap) S.listed = (uint8_t)level;
+    }
     a.state[r.row] = S;
     if (pass) a.flags[0] = 1;
   }
+  __syncthreads();  // S.listed
   if (!pass && !needSS) return;
 
   const int nslots = S.nslots;
+  // a row compacted by an earlier level scans its list; the compacting pass (listed == level) reads the row
+  const bool fromList = S.listed != 0 && S.listed < level;
+  const bool listing = pass && S.listed == level;
+  const double *src = fromList ? a.list + r.row * kGsListCap : r.p;
+  const int count = fromList ? a.listN[r.row] : r.count;
+  double *dstList = a.list + r.row * kGsListCap;
   if (pass) {
     for (int i = tid; i < nslots * 256; i += kThreads) hist[i] = 0;
     if (tid < 2 * a.nq && S.slotOf[tid] != 0xff) slotTop[S.slotOf[tid]] = S.prefix[tid] >> shift_of(level - 1);
@@ -329,18 +366,23 @@ __global__ void __launch_bounds__(kThreads, 2) gs_level_kernel(const GsArgs a, c
       if (S.slotOf[r2] != 0xff && S.pop[r2] > 1024u) trackMask |= 1u << S.slotOf[r2];
   // The scan of the row, instantiated for the number of slots an element has to be matched against: most rows have one
   // or two bins in play, and eight compare + select pairs per element are most of what the later levels execute.
-  const auto scan = [&](auto nsTag) {
+  const int nxs = nx;
+  // LIST: the compacting pass (its own instantiation: the other passes keep the loop without the append)
+  const auto scan = [&](auto nsTag, auto listTag) {
   constexpr int NS = decltype(nsTag)::value;
-  for (int i0 = 0; i0 < r.count; i0 += kUnroll * kThreads) {
-    double x[kUnroll];
+  constexpr bool LIST = decltype(listTag)::value;
+  constexpr int UN = HI32 ? kUnrollWide : kUnroll;
+  for (int i0 = 0; i0 < count; i0 += UN * kThreads) {
+    double x[UN];
 #pragma unroll
-    for (int u = 0; u < kUnroll; ++u) {
+    for (int u = 0; u < UN; ++u) {
       const int i = i0 + u * kThreads + tid;
-      x[u] = i < r.count ? r.p[i] : __longlong_as_double(0x7ff8000000000000ll);
+      x[u] = i < count ? src[i] : __longlong_as_double(0x7ff8000000000000ll);
     }
 #pragma unroll
-    for (int u = 0; u < kUnroll; ++u) {
+    for (int u = 0; u < UN; ++u) {
       int code = -1;
+      bool keep = false;
       if (finite_hi(x[u])) {
         if (needSS) {
           const double d = x[u] - mu;
@@ -365,6 +407,13 @@ __global__ void __launch_bounds__(kThreads, 2) gs_level_kernel(const GsArgs a, c
               if (top[s] == t) slot = s;
             bin = (int)((k >> sh1) & (uint64_t)bmask);
           }
+          if (LIST) {
+            keep = slot >= 0;
+            if (nxs > 0) {  // rare: a statistic already waits for the emit while others are open
+              const uint64_t k = key_of(x[u]);
+              for (int j = 0; j < nxs; ++j) keep = keep || (k >> xSh[j]) == xTop[j];
+            }
+          }
           if (slot >= 0) {
             code = slot * 256 + bin;
             if ((trackMask >> slot) & 1u) {  // one representative (first come) and the OR of the differences
@@ -385,20 +434,37 @@ __global__ void __launch_bounds__(kThreads, 2) gs_level_kernel(const GsArgs a, c
         }
       }
       // (warps in which no lane holds a candidate -- most of them from the second refinement on -- skip the update)
-      if (pass && __any_sync(0xffffffffu, code >= 0)) hist_add(hist, code);
+      if (!LIST) {
+        if (pass && __any_sync(0xffffffffu, code >= 0)) hist_add(hist, code);
+      } else {  // keep >= (code >= 0); one shared atomic per warp, and a warp's keys land side by side in the list
+        const unsigned m = __ballot_sync(0xffffffffu, keep);
+        if (m) {
+          hist_add(hist, code);
+          const int lane = tid & 31;
+          unsigned base = 0;
+          if (lane == 0) base = atomicAdd(&listFill, (unsigned)__popc(m));
+          base = __shfl_sync(0xffffffffu, base, 0) + (unsigned)__popc(m & ((1u << lane) - 1u));
+          if (keep && base < (unsigned)kGsListCap) dstList[base] = x[u];  // (the global bound keeps base below)
+        }
+      }
     }
   }
   };
-  if (nslots <= 1) scan(std::integral_constant<int, 1>{});
-  else if (nslots <= 2) scan(std::integral_constant<int, 2>{});
-  else if (nslots <= 4) scan(std::integral_constant<int, 4>{});
-  else scan(std::integral_constant<int, kGsMaxStat>{});
+  const auto slots = [&](auto listTag) {
+    if (nslots <= 1) scan(std::integral_constant<int, 1>{}, listTag);
+    else if (nslots <= 2) scan(std::integral_constant<int, 2>{}, listTag);
+    else if (nslots <= 4) scan(std::integral_constant<int, 4>{}, listTag);
+    else scan(std::integral_constant<int, kGsMaxStat>{}, listTag);
+  };
+  if (listing) slots(std::true_type{});
+  else slots(std::false_type{});
   if (needSS) {
     const double ss = block_sum(q2, red);
     if (tid == 0) a.q2All[(int64_t)a.rank * rows + r.row] = ss;
   }
   if (pass) {
     __syncthreads();
+    if (listing && tid == 0) a.listN[r.row] = (int)min(listFill, (unsigned)kGsListCap);
     unsigned int *g = a.hist + r.row * kGsHistWords;
     for (int i = tid; i < nslots * 256; i += kThreads) g[i] = hist[i];
     if (tid < kGsMaxStat) {
@@ -452,6 +518,9 @@ __global__ void __launch_bounds__(kThreads, 2) gs_emit_kernel(const GsArgs a) {
   }
   __syncthreads();
   if (nemit == 0) return;
+  const bool fromList = S.listed != 0;  // every emit bin lies inside the filter the list was cut with
+  const double *src = fromList ? a.list + r.row * kGsListCap : r.p;
+  const int count = fromList ? a.listN[r.row] : r.count;
   // the ACTIVE emit slots in registers, compacted (most rows have one to three): a key belongs to slot at[j] when
   // (key >> shv[j]) == tp[j].  When every slot was resolved within the key's high word (<= 32 bits: the usual case)
   // the test is a 32-bit shift and compare.  The scan is instantiated for the number of active slots.
@@ -487,12 +556,12 @@ __global__ void __launch_bounds__(kThreads, 2) gs_emit_kernel(const GsArgs a) {
   }
   const auto scan = [&](auto neTag) {
     constexpr int NE = decltype(neTag)::value;
-    for (int i0 = 0; i0 < r.count; i0 += kUnroll * kThreads) {
+    for (int i0 = 0; i0 < count; i0 += kUnroll * kThreads) {
       double x[kUnroll];
 #pragma unroll
       for (int u = 0; u < kUnroll; ++u) {
         const int i = i0 + u * kThreads + tid;
-        x[u] = i < r.count ? r.p[i] : __longlong_as_double(0x7ff8000000000000ll);
+        x[u] = i < count ? src[i] : __longlong_as_double(0x7ff8000000000000ll);
       }
 #pragma unroll
       for (int u = 0; u < kUnroll; ++u) {

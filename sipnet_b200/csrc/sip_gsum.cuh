@@ -27,6 +27,7 @@ constexpr int kGsEmit = 16;             // a bin with at most this many keys (ov
 constexpr int kGsHistWords = 2048;      // per row and level: 2^11 bins (level 0) or kGsMaxStat slots x 2^8 bins
 constexpr int kGsLevels = 8;            // key bits per level: 11, 8, 8, 8, 8, 8, 8, 5
 constexpr int kGsMaxCols = 8;           // summary columns per pass
+constexpr int kGsListCap = 4096;        // candidate list of a row (see GsArgs::list): at most this many keys, all ranks
 
 struct GsStat {  // per row and rank, pass 0
   double count, sum;
@@ -51,7 +52,7 @@ struct GsRow {  // selection state of a row; identical on every rank after each 
   uint8_t bits;                 // leading key bits resolved so far (same for every statistic of the row)
   uint8_t done;                 // 0 = needs another level, 1 = every statistic is resolved or ready to emit,
                                 // 2 = constant row (value in prefix[0]), 3 = no finite member
-  uint8_t pad;
+  uint8_t listed;               // level whose pass copied this rank's candidates into GsArgs::list (0 = none)
   double n, mean;
 };
 
@@ -77,6 +78,12 @@ struct GsArgs {
                        // large group of equal values -- exact zeros -- would otherwise need every key bit)
   uint64_t *emitAll;   // [nranks][rows][kGsMaxStat][kGsEmit]
   int32_t *flags;      // [0] = some row needs the next level
+  // Candidate lists (nullptr: never compact).  A level pass whose filter -- the slots in play plus the bins of the
+  // statistics waiting for the emit -- holds at most kGsListCap keys over ALL ranks copies this rank's finite members
+  // inside it to list[row]; later levels and the emit scan that list instead of the row.  Later prefixes only extend
+  // the filter's, so the list holds every key they look for; the global bound keeps every rank's share in the list.
+  double *list;        // [rows][kGsListCap]
+  int32_t *listN;      // [rows]: members in list[row]
   // results, in the handle's layout: mean/var [site][col][n], quant [site][col][q][n]
   double *mean, *var, *quant;
   int32_t nqTotal;  // quantiles per column (quant rows are [nqTotal] per column)
