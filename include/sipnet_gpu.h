@@ -622,7 +622,10 @@ int sipnet_gpu_rows_summary(int device, const double *d_rows, int64_t nrows, int
  * reference's host libm (glibc) -- see sipnet_b200/csrc/sip_libm.cuh.
  * ops 2..5 evaluate the optimistic policy of the production kernel (sip_num.cuh FastNum): 2 = exp(x),
  * 3 = pow(x, y), 4 = pow(x, y) through the cached log of x, 5 = x / y.  An input outside the policy's guards
- * (the member would be replayed by the general kernel) yields SIPNET_GPU_EVAL_FLAGGED instead of a value. */
+ * (the member would be replayed by the general kernel) yields SIPNET_GPU_EVAL_FLAGGED instead of a value.
+ * ops 6, 7 evaluate the throughput policy's divisions (ThroughNum): 6 = x / y as one multiplication by the refined
+ * reciprocal of y, 7 = x / y of the soil-water balance (the reciprocal plus one residual step); they are flagged by
+ * the divisor check only.  op 8 = the refined reciprocal of x itself (y unused, never flagged). */
 #define SIPNET_GPU_EVAL_FLAGGED 0x7ff8bad0bad0bad0ull
 int sipnet_gpu_eval_libm(int device, int op, const double *x, const double *y, double *out, int64_t n);
 

@@ -220,17 +220,19 @@ def flags_array(flags: dict) -> np.ndarray:
 
 
 EVAL_FLAGGED = 0x7ff8bad0bad0bad0     # sipnet_gpu.h SIPNET_GPU_EVAL_FLAGGED
-_EVAL_OPS = {"exp": 0, "pow": 1, "fast_exp": 2, "fast_pow": 3, "fast_powc": 4, "fast_div": 5}
+_EVAL_OPS = {"exp": 0, "pow": 1, "fast_exp": 2, "fast_pow": 3, "fast_powc": 4, "fast_div": 5, "thr_div": 6,
+             "thr_divw": 7, "seed": 8}
 
 
 def device_libm(op: str, x: np.ndarray, y: Optional[np.ndarray] = None, device: int = 0) -> np.ndarray:
     """Evaluate the DEVICE exp/pow (glibc-exact restatement) on arrays (validation hook).  The fast_* ops run the
-    production kernel's optimistic policy; inputs outside its guards come back as the bit pattern EVAL_FLAGGED."""
+    production kernel's optimistic policy; inputs outside its guards come back as the bit pattern EVAL_FLAGGED.
+    thr_div / thr_divw are the throughput policy's divisions, seed the refined reciprocal of x (sip_num.cuh)."""
     lib = load_library()
     x = np.ascontiguousarray(x, dtype=np.float64)
     out = np.empty_like(x)
     yp = None
-    if op not in ("exp", "fast_exp"):
+    if op not in ("exp", "fast_exp", "seed"):
         y = np.ascontiguousarray(y, dtype=np.float64)
         yp = y.ctypes.data
     rc = lib.sipnet_gpu_eval_libm(device, _EVAL_OPS[op], x.ctypes.data, yp, out.ctypes.data, x.size)

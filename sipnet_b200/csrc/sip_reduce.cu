@@ -589,6 +589,10 @@ cudaError_t measure_fp64_peak(int device, double *tflops) {
 // ops 0, 1: the general restatement (libm::exp, libm::pow).  ops 2..5: the optimistic policy of the production
 // kernel (FastNum: exp, pow with a varying base, pow with a cached log of the base, a / b); an input outside its
 // guards yields kFlagged instead of a value -- "FastNum never has to be right outside its guards, only to notice".
+// ops 6, 7: the throughput policy's divisions (ThroughNum::div, ThroughNum::divw, flagged by the divisor check
+// only); op 8: the refined reciprocal FastNum::seed(x) both policies start from (never flagged).  Their arithmetic
+// is written with explicit intrinsics (__dmul_rn, __fma_rn, rcp.approx), so this translation unit's -fmad=false
+// evaluates them exactly as the -fmad=true throughput kernels do.
 constexpr unsigned long long kFlagged = 0x7ff8bad0bad0bad0ull;
 __global__ void eval_libm_kernel(int op, const double *x, const double *y, double *out, int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -608,8 +612,14 @@ __global__ void eval_libm_kernel(int op, const double *x, const double *y, doubl
   } else if (op == 4) {
     const libm::LogHL l = libm::pow_log(x[i]);
     v = nm.powc(x[i], l.hi, l.lo, y[i]);
-  } else {
+  } else if (op == 5) {
     v = nm.div(x[i], y[i]);
+  } else if (op == 8) {
+    v = nm.seed(x[i]);
+  } else {
+    ThroughNum tn;
+    v = op == 6 ? tn.div(x[i], y[i]) : tn.divw(x[i], y[i]);
+    nm.bad = tn.bad;
   }
   out[i] = nm.bad ? __longlong_as_double((long long)kFlagged) : v;
 }

@@ -1074,7 +1074,7 @@ extern "C" int sipnet_gpu_measure_fp64_peak(int device, double *tflops) {
 }
 
 extern "C" int sipnet_gpu_eval_libm(int device, int op, const double *x, const double *y, double *out, int64_t n) {
-  if (!x || !out || n <= 0 || op < 0 || op > 5 || (op != 0 && op != 2 && !y))
+  if (!x || !out || n <= 0 || op < 0 || op > 8 || (op != 0 && op != 2 && op != 8 && !y))
     return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "bad eval_libm arguments");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev)

@@ -53,6 +53,41 @@ def assert_close(a, b, scale, names, rtol=RTOL, what=""):
     return float(np.nanmax(e)) if e.size else 0.0
 
 
+# the pool columns: their empty / non-empty pattern is a clamp or mortality decision
+POOL_COLS = [A.O[n] for n in ("plantWoodC", "plantLeafC", "soilC", "coarseRootC", "fineRootC", "litterC", "soilWater", "snow",
+                              "minN", "soilOrgN", "litterN", "plantStorageN")]
+
+
+def check_throughput(got, o_out, got_recs, o_recs, tag, cols=None):
+    """The throughput policy's bar (tests/test_gpu_throughput.py): `got` [T'][len(cols)] holds one member's values of
+    the output columns `cols` (all 32 by default) from a MATH_THROUGHPUT run, `o_out` [T][32] the oracle's.
+      * every column within RTOL, except nLeaching (the drainage of a nearly saturated soil) within 10 * RTOL;
+      * the empty / non-empty pattern of the pool columns exact ("empty" = below 1e-12 of the column's magnitude);
+      * event records (when `o_recs` is not None): steps, types, variants exact, values within RTOL.
+    Returns (worst error of the RTOL columns, worst nLeaching error)."""
+    cols = list(range(A.NOUT)) if cols is None else list(cols)
+    T = o_out.shape[0]
+    g, ref = got[:T], o_out[:, cols]
+    scale = out_scales(o_out)[cols]
+    names = [A.OUT_NAMES[c] for c in cols]
+    keep = [i for i, c in enumerate(cols) if c != A.O["nLeaching"]]
+    nl = [i for i, c in enumerate(cols) if c == A.O["nLeaching"]]
+    err = assert_close(g[:, keep], ref[:, keep], scale[keep], [names[i] for i in keep], RTOL, tag) if keep else 0.0
+    err_nl = assert_close(g[:, nl], ref[:, nl], scale[nl], ["nLeaching"], 10 * RTOL, tag) if nl else 0.0
+    pools = [i for i, c in enumerate(cols) if c in POOL_COLS]
+    if pools:
+        tiny = 1e-12 * np.maximum(np.nanmax(np.abs(ref[:, pools]), axis=0), 1e-300)
+        assert np.array_equal(np.abs(g[:, pools]) <= tiny, np.abs(ref[:, pools]) <= tiny), \
+            f"{tag}: pool clamp / mortality pattern differs"
+    if o_recs is not None:
+        assert [(r.step, r.type, r.variant, r.nval) for r in got_recs] == [(r.step, r.type, r.variant, r.nval) for r in o_recs], \
+            f"{tag}: event rows differ"
+        for a, b in zip(got_recs, o_recs):
+            for k in range(b.nval):
+                assert abs(a.val[k] - b.val[k]) <= RTOL * max(abs(a.val[k]), abs(b.val[k]), 1e-6), (tag, b.type, k)
+    return err, err_nl
+
+
 def random_flag_cases(ntrials=30, members=6, seed=2026):
     """Seeded random combinations of the 12 model flags that pass validateContext() (context.c:195-223), each with a
     synthetic two-year site (alternating step patterns, event schedule when EVENTS is on) and a few wide-prior members."""

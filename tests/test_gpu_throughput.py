@@ -20,13 +20,11 @@ import numpy as np
 import pytest
 
 from conftest import Golden, golden_names
-from gpu_util import RTOL, assert_close, out_scales, random_flag_cases
+from gpu_util import RTOL, check_throughput, random_flag_cases
 from sipnet_b200 import _abi as A, api, synth
 
 pytestmark = pytest.mark.gpu
 
-POOL_COLS = [A.O[n] for n in ("plantWoodC", "plantLeafC", "soilC", "coarseRootC", "fineRootC", "litterC", "soilWater", "snow",
-                              "minN", "soilOrgN", "litterN", "plantStorageN")]
 WORST = {"err": 0.0, "nLeaching": 0.0}
 
 
@@ -38,23 +36,9 @@ def run_throughput(sites, params, ms, flags, **kw):
 
 
 def check(res, m, o_out, o_recs, tag):
-    T = o_out.shape[0]
-    g = res["out"][:, :T, m].T
-    keep = [i for i in range(A.NOUT) if i != A.O["nLeaching"]]
-    names = [A.OUT_NAMES[i] for i in keep]
-    WORST["err"] = max(WORST["err"], assert_close(g[:, keep], o_out[:, keep], out_scales(o_out)[keep], names, RTOL, tag))
-    nl = [A.O["nLeaching"]]
-    WORST["nLeaching"] = max(WORST["nLeaching"], assert_close(g[:, nl], o_out[:, nl], out_scales(o_out)[nl], ["nLeaching"],
-                                                              10 * RTOL, tag))
-    tiny = 1e-12 * np.maximum(np.nanmax(np.abs(o_out[:, POOL_COLS]), axis=0), 1e-300)
-    assert np.array_equal(np.abs(g[:, POOL_COLS]) <= tiny, np.abs(o_out[:, POOL_COLS]) <= tiny), \
-        f"{tag}: pool clamp / mortality pattern differs"
-    got = res["recs"][m]
-    assert [(r.step, r.type, r.variant, r.nval) for r in got] == [(r.step, r.type, r.variant, r.nval) for r in o_recs], \
-        f"{tag}: event rows differ"
-    for a, b in zip(got, o_recs):
-        for k in range(b.nval):
-            assert abs(a.val[k] - b.val[k]) <= RTOL * max(abs(a.val[k]), abs(b.val[k]), 1e-6), (tag, b.type, k)
+    err, err_nl = check_throughput(res["out"][:, :, m].T, o_out, res["recs"][m], o_recs, tag)
+    WORST["err"] = max(WORST["err"], err)
+    WORST["nLeaching"] = max(WORST["nLeaching"], err_nl)
 
 
 @pytest.mark.parametrize("name", golden_names())

@@ -9,6 +9,8 @@ import os
 import subprocess
 import tempfile
 
+from fractions import Fraction
+
 import numpy as np
 import pytest
 
@@ -68,6 +70,15 @@ def test_device_libm_is_bit_exact():
     assert np.array_equal(gotp[idx][ok].view(np.uint64), wantp[ok].view(np.uint64))
 
 
+# the edges of every guard of the optimistic policy (sip_num.cuh FastNum) and the special values of exp / pow / division
+SPECIALS = np.array([0.0, -0.0, 5e-324, -5e-324, 1e-320, 2.0 ** -1022, 2.0 ** -1000, -2.0 ** -970, 2.0 ** -969, 2.0 ** -901,
+                     2.0 ** -900, -2.0 ** -899, 2.0 ** -65, 2.0 ** -64, 2.0 ** -63, 2.0 ** -55, -2.0 ** -55, 2.0 ** -54,
+                     np.nextafter(2.0 ** -54, 0), -np.nextafter(2.0 ** -54, 0), 2.0 ** -53, 1e-17, -1e-17, 0.5, 1.0,
+                     -1.0, np.nextafter(1.0, 2), np.nextafter(1.0, 0), 1.5, 2.0, 3.0, 10.0, 511.9999, np.nextafter(512.0, 0),
+                     512.0, -512.0, 709.0, -745.0, 1024.0, 2.0 ** 62, 2.0 ** 63, 2.0 ** 64, np.nextafter(2.0 ** 64, 0),
+                     2.0 ** 899, 2.0 ** 900, 2.0 ** 964, 1e300, 1.7e308, np.inf, -np.inf, np.nan])
+
+
 def _glibc():
     import ctypes
     libm = ctypes.CDLL("libm.so.6")
@@ -90,12 +101,7 @@ def test_optimistic_policy_is_exact_or_flags():
     libm = _glibc()
     rng = np.random.default_rng(2024)
     flagged = np.uint64(api.EVAL_FLAGGED)
-    specials = np.array([0.0, -0.0, 5e-324, -5e-324, 1e-320, 2.0 ** -1022, 2.0 ** -1000, -2.0 ** -970, 2.0 ** -969, 2.0 ** -901,
-                         2.0 ** -900, -2.0 ** -899, 2.0 ** -65, 2.0 ** -64, 2.0 ** -63, 2.0 ** -55, -2.0 ** -55, 2.0 ** -54,
-                         np.nextafter(2.0 ** -54, 0), -np.nextafter(2.0 ** -54, 0), 2.0 ** -53, 1e-17, -1e-17, 0.5, 1.0,
-                         -1.0, np.nextafter(1.0, 2), np.nextafter(1.0, 0), 1.5, 2.0, 3.0, 10.0, 511.9999, np.nextafter(512.0, 0),
-                         512.0, -512.0, 709.0, -745.0, 1024.0, 2.0 ** 62, 2.0 ** 63, 2.0 ** 64, np.nextafter(2.0 ** 64, 0),
-                         2.0 ** 899, 2.0 ** 900, 2.0 ** 964, 1e300, 1.7e308, np.inf, -np.inf, np.nan])
+    specials = SPECIALS
 
     # ---- exp
     xs = np.concatenate([rng.uniform(-60, 20, 200000), rng.uniform(-511, 511, 100000), rng.uniform(-1e-15, 1e-15, 20000),
@@ -155,3 +161,88 @@ def test_optimistic_policy_is_exact_or_flags():
     q = np.abs(want[ordinary])
     inside = (q == 0) | ((q >= 2.0 ** -900) & (q < 2.0 ** 900))
     assert np.array_equal(~fl[ordinary], inside)          # the guard is exactly "zero or 2^-900 <= |q| < 2^900"
+
+
+def _exponent(x):
+    """floor(log2 |x|) of a nonzero Fraction"""
+    n, d = abs(x.numerator), x.denominator
+    e = n.bit_length() - d.bit_length()
+    return e if (n >= d << e if e >= 0 else n << -e >= d) else e - 1
+
+
+def _significand(x):
+    """|x| / 2^floor(log2 |x|), in [1, 2)"""
+    return abs(x) / Fraction(2) ** _exponent(x)
+
+
+@pytest.mark.gpu
+def test_throughput_quotients_against_exact_rationals():
+    """The throughput policy's divisions (sip_num.cuh ThroughNum), op by op against fractions.Fraction.
+
+    div(a, b) = RN(a * y) with y = seed(b), the refined reciprocal.  Write Q = a / b = m_q 2^e_q and 1/b = m_r 2^e_r
+    (m in [1, 2)).  Then |q - Q| <= |RN(a y) - a y| + |a| |y - 1/b|, and |a| = m_q 2^e_q / (m_r 2^e_r), so in ulps of Q
+    (2^(e_q - 52)):
+      * y correctly rounded, |y - 1/b| <= 2^(e_r - 53):  |q - Q| <= 1/2 + m_q / (2 m_r) < 1.5 ulp.  (When a y crosses
+        into the next binade, RN(a y) is that power of two, no farther from Q than a y is; the bound stands.)
+      * y only faithful, |y - 1/b| < 2^(e_r - 52):  |q - Q| < m_q / m_r + 1 (the rounding may then be a full ulp of Q).
+    The test checks which of the two the seed is for every sampled divisor, against RN(1/b), and asserts the bound that
+    follows for that element."""
+    from sipnet_b200 import api
+    rng = np.random.default_rng(2026)
+    n = 100000
+    b = np.concatenate([rng.uniform(1, 2, n // 4), np.exp(rng.uniform(-44, 44, n // 4)),
+                        rng.integers(2 ** 52, 2 ** 53, n // 4).astype(np.float64) * 2.0 ** rng.integers(-116, 11, n // 4),
+                        rng.uniform(0.1, 50, n // 4)])
+    a = np.concatenate([rng.normal(0, 100, n // 2), np.exp(rng.uniform(-40, 40, n // 2)) * rng.choice([-1.0, 1.0], n // 2)])
+    a[: n // 8] = rng.integers(2 ** 52, 2 ** 53, n // 8).astype(np.float64) * 2.0 ** -52   # both significands random
+
+    # ---- op 8: the refined reciprocal against RN(1/b)
+    y = api.device_libm("seed", b)
+    rn = 1.0 / b
+    cr = y == rn
+    for i in np.flatnonzero(~cr):                      # faithful: y and RN(1/b) are the two neighbours of 1/b
+        r = 1 / Fraction(float(b[i]))
+        lo, hi = sorted((Fraction(float(y[i])), Fraction(float(rn[i]))))
+        assert np.nextafter(rn[i], y[i]) == y[i] and lo < r < hi, (b[i].hex(), y[i].hex())
+
+    # ---- op 6: the quotient, in ulps of the exact quotient
+    q = api.device_libm("thr_div", a, b)
+    assert not (q.view(np.uint64) == np.uint64(api.EVAL_FLAGGED)).any()
+    worst, worst_bound = 0.0, 0.0
+    for i in range(a.size):
+        Q = Fraction(float(a[i])) / Fraction(float(b[i]))
+        ulp = Fraction(2) ** (_exponent(Q) - 52)
+        err = abs(Fraction(float(q[i])) - Q) / ulp
+        ratio = _significand(Q) / _significand(1 / Fraction(float(b[i])))
+        bound = Fraction(1, 2) + ratio / 2 if cr[i] else 1 + ratio
+        assert err <= bound, (a[i].hex(), b[i].hex(), float(err), float(bound), bool(cr[i]))
+        worst, worst_bound = max(worst, float(err)), max(worst_bound, float(bound))
+    if cr.all():
+        assert worst_bound < 1.5                        # sip_num.cuh: "<= 1.5 ulp instead of correctly rounded"
+    print(f"throughput division: seed correctly rounded for {int(cr.sum())} of {cr.size} divisors; worst error "
+          f"{worst:.4f} ulp of the exact quotient, largest proved bound of the sample {worst_bound:.4f} ulp")
+
+    # ---- flags: the divisor check and nothing else (no quotient-range guard); op 7 = IEEE a / b where op 5 is unflagged
+    sa = np.concatenate([np.repeat(SPECIALS, SPECIALS.size), np.repeat(-SPECIALS, SPECIALS.size), a[:2000]])
+    sb = np.concatenate([np.tile(SPECIALS, SPECIALS.size), np.tile(SPECIALS, SPECIALS.size), b[:2000]])
+    ordinary = (sb >= 2.0 ** -64) & (sb < 2.0 ** 64)
+    flag = np.uint64(api.EVAL_FLAGGED)
+    f5, f6, f7 = ((api.device_libm(op, sa, sb).view(np.uint64) == flag) for op in ("fast_div", "thr_div", "thr_divw"))
+    assert np.array_equal(f6, ~ordinary) and np.array_equal(f7, ~ordinary)
+    assert (f5 | ~f6).all() and (f5 & ordinary).any()   # op 5 flags more: its quotient-range guard
+    for x, z in ((a, b), (sa[~f5], sb[~f5])):
+        with np.errstate(all="ignore"):
+            assert _same_bits(api.device_libm("thr_divw", x, z), x / z)
+
+    # ---- edges, unflagged: quotients in the subnormal range and past DBL_MAX
+    m1, m2 = rng.uniform(1, 2, 2000), rng.uniform(1, 2, 2000)
+    sub_a, sub_b = m1 * 2.0 ** -1000 * rng.choice([-1.0, 1.0], 2000), m2 * 2.0 ** rng.integers(23, 64, 2000)
+    q6, q7 = api.device_libm("thr_div", sub_a, sub_b), api.device_libm("thr_divw", sub_a, sub_b)
+    assert not (q6.view(np.uint64) == flag).any() and not (q7.view(np.uint64) == flag).any() and np.isfinite(q7).all()
+    tiny = Fraction(2) ** -1074
+    for i in range(sub_a.size):   # rounding to the subnormal grid (<= 2^-1075) + the seed's share (< |Q| 2^-52 < 2^-1074)
+        assert abs(Fraction(float(q6[i])) - Fraction(float(sub_a[i])) / Fraction(float(sub_b[i]))) < Fraction(3, 2) * tiny
+    big_a, big_b = m1 * 2.0 ** 1000 * rng.choice([-1.0, 1.0], 2000), m2 * 2.0 ** -rng.integers(26, 64, 2000)
+    q6, q7 = api.device_libm("thr_div", big_a, big_b), api.device_libm("thr_divw", big_a, big_b)
+    assert np.array_equal(q6, np.copysign(np.inf, big_a))   # a y > DBL_MAX: RN(a y) overflows
+    assert np.isnan(q7).all() and not (q7.view(np.uint64) == flag).any()   # q0 = inf, r = -inf: q0 + y r = NaN
