@@ -566,6 +566,69 @@ typedef struct sipnet_gpu_jitter_spec {
 } sipnet_gpu_jitter_spec;
 int sipnet_gpu_rejuvenate(sipnet_gpu_handle *h, const sipnet_gpu_jitter_spec *spec, double *diag);
 
+/*
+ * Parameter calibration: a tempered random-walk Metropolis-Hastings move of listed parameter rows, per site, that
+ * re-runs every member over the window [0, s) (s = the next step, s >= 1) and keeps or restores each member's
+ * proposal.  It leaves the tempered posterior  p(theta) L(theta)^tau  of each site invariant, so a caller's
+ * resample-move loop (temper, resample(), mh_move()) reaches the parameter posterior of a fixed calibration window.
+ * L is the step kernel's Gaussian NEE likelihood (SIPNET_GPU_OUT_LOGLIK, nee_sigma).  Units as in rejuvenate().
+ *
+ * rows, transform, lower, upper: exactly as in sipnet_gpu_jitter_spec (same checks).  prior[j] of row j:
+ *   SIPNET_GPU_PRIOR_FLAT    uniform in theta on [prior_a, prior_b] (prior_a < prior_b, either may be infinite: an
+ *                            improper flat prior; on a LOGIT row lower <= prior_a and prior_b <= upper)
+ *   SIPNET_GPU_PRIOR_NORMAL  normal in phi with mean prior_a (finite) and sd prior_b (finite, > 0): a lognormal
+ *                            prior on theta for a LOG row, a logit-normal one for a LOGIT row
+ * Its log density in phi (constants dropped): FLAT log|dtheta/dphi| = 0 (IDENTITY), phi (LOG),
+ * log((theta - lo)(hi - theta) / (hi - lo)) (LOGIT), and -inf outside [prior_a, prior_b];
+ * NORMAL -(phi - prior_a)^2 / (2 prior_b^2).  lp(phi) = sum over the rows.
+ * scale[nsites] is the random-walk scale h per site (finite, > 0; NaN = leave the site alone); tempering[nsites] is
+ * tau in [0, 1].  current_loglik[nmembers] is the members' log-likelihood over [0, s) (the handle's own is zeroed by
+ * resample(), so the caller carries it); z[n_rows][nmembers] standard normals; log_u[nmembers] <= 0 (-inf allowed).
+ *
+ * Member i takes part at its site iff it would take part in rejuvenate(), current_loglik[i] is finite and lp(phi_i)
+ * is finite.  A site with scale[s] not NaN and N >= 2 participants is moved: mean, population covariance V and its
+ * semidefinite Cholesky factor L exactly as in rejuvenate(), and
+ *   phi'_ij = phi_ij + h sum_{m<=j} L_jm z_mi   (rejuvenate() with a = 1, a symmetric proposal)
+ * A proposal is invalid when some theta' is not finite or not inside its domain, fails ensureAllocation, or has
+ * lp(phi') = -inf.  Every member with a valid proposal gets theta' and its derived rows (as rejuvenate()); then every
+ * member is reset and run over [0, s) (reset(), run(0, s) in pieces of out_steps_capacity when outputs are kept),
+ * giving its log-likelihood L'_i.  With
+ *   delta_i = tau_s (L'_i - current_loglik[i]) + sum_j [lp_j(phi'_i) - lp_j(phi_i)]   (the tau term is 0 at tau = 0)
+ * member i is accepted iff its proposal was valid, L'_i is finite (0 without SIPNET_GPU_OUT_LOGLIK), its status after
+ * the run has neither SIPNET_GPU_ST_BAD_ALLOCATION nor SIPNET_GPU_ST_NONFINITE, and log_u[i] < delta_i.  An accepted
+ * member keeps what the run produced.  Every other member -- non-participants, sites left alone, invalid and rejected
+ * proposals -- gets back, bit for bit, everything it had before the call: parameter rows, state, rings, status, event
+ * count and records, message counters, log-likelihood and observation count.
+ *
+ * Afterwards every member is at step s and there is no last run range: the per-step outputs and summaries of
+ * [0, s) are gone, as after reset() (run again to get them).  Only windows that start at step 0 are supported.
+ *
+ * diag (may be NULL) receives double [nsites][4] = {N, rank (-1 where the site was left alone), invalid, accepted}.
+ * A call whose scale is NaN at every site launches nothing and changes nothing; its diag rows are {NaN, -1, 0, 0}.
+ *
+ * Rejected with SIPNET_GPU_ERR_BAD_ARGUMENT, nothing changed: everything rejuvenate() rejects for rows, transforms
+ * and z; NULL spec arrays; an unknown prior or out-of-range prior bounds or sd; a scale neither NaN nor finite > 0;
+ * a tempering outside [0, 1]; a log_u entry NaN or > 0; s = 0; tau > 0 at a site with a scale on a handle without
+ * SIPNET_GPU_OUT_LOGLIK.  Every call returns when the move is complete.
+ */
+#define SIPNET_GPU_PRIOR_FLAT 0   /* uniform in theta on [prior_a, prior_b] */
+#define SIPNET_GPU_PRIOR_NORMAL 1 /* normal in phi, mean prior_a, sd prior_b */
+typedef struct sipnet_gpu_mh_spec {
+  int32_t n_rows;               /* 1 .. 16 */
+  const int32_t *rows;          /* as sipnet_gpu_jitter_spec */
+  const int32_t *transform;     /* [n_rows] SIPNET_GPU_TF_* */
+  const double *lower, *upper;  /* [n_rows] bounds of LOGIT rows (read only for those; may be NULL without one) */
+  const int32_t *prior;         /* [n_rows] SIPNET_GPU_PRIOR_* */
+  const double *prior_a;        /* [n_rows] FLAT: lower bound on theta; NORMAL: mean of phi */
+  const double *prior_b;        /* [n_rows] FLAT: upper bound on theta; NORMAL: sd of phi */
+  const double *scale;          /* [nsites] random-walk scale h > 0; NaN = leave the site alone */
+  const double *tempering;      /* [nsites] tau in [0, 1] */
+  const double *current_loglik; /* [nmembers] the members' log-likelihood over [0, s) (host) */
+  const double *z;              /* [n_rows][nmembers] standard normals (host) */
+  const double *log_u;          /* [nmembers] log of uniforms, <= 0, -inf allowed (host) */
+} sipnet_gpu_mh_spec;
+int sipnet_gpu_mh_move(sipnet_gpu_handle *h, const sipnet_gpu_mh_spec *spec, double *diag);
+
 /* Slots of the mean-NPP ring this handle uses (config ring_slots, or the automatic choice). */
 int32_t sipnet_gpu_ring_slots(const sipnet_gpu_handle *h);
 
@@ -678,6 +741,11 @@ int sipnet_gpu_comm_resample(sipnet_gpu_comm *c, const double *u, double ess_fra
  * rank); every rank gets the same diag.  The ranks all-gather two per-site partial sums (N and the sums of phi, then
  * the centred cross sums) and add them in rank order, so every rank applies identical coefficients. */
 int sipnet_gpu_comm_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *spec, double *diag);
+/* Collective.  sipnet_gpu_mh_move() over the members of ALL ranks: current_loglik, z and log_u hold the rank's own
+ * members, everything else (and the next step) is the same on every rank (a mismatch, found through an all-gathered
+ * hash, fails on every rank); every rank gets the same diag.  The ranks exchange the two moment passes' partial sums
+ * as rejuvenate() does and then the integer counts; each rank resets and runs its own members, with no exchange. */
+int sipnet_gpu_comm_mh_move(sipnet_gpu_comm *c, const sipnet_gpu_mh_spec *spec, double *diag);
 
 /* (b) one process, one host thread, several GPUs: the single-GPU configuration, partitioned by the library --
  *     whole sites per device when there are at least as many sites as devices, otherwise an even contiguous share
@@ -714,6 +782,9 @@ int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, double ess_f
 /* sipnet_gpu_rejuvenate() on the whole configuration (shrink, z [n_rows][nmembers] and diag in configuration order):
  * split sites go through the team exchange, whole sites are moved by each device alone. */
 int sipnet_gpu_multi_rejuvenate(sipnet_gpu_multi *m, const sipnet_gpu_jitter_spec *spec, double *diag);
+/* sipnet_gpu_mh_move() on the whole configuration (current_loglik, z [n_rows][nmembers], log_u in configuration
+ * order; scale, tempering and diag in global site order), over [0, the multi handle's next step). */
+int sipnet_gpu_multi_mh_move(sipnet_gpu_multi *m, const sipnet_gpu_mh_spec *spec, double *diag);
 void sipnet_gpu_multi_destroy(sipnet_gpu_multi *m);
 
 #ifdef __cplusplus

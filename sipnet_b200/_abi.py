@@ -135,6 +135,7 @@ MATH_VALIDATION, MATH_FAST, MATH_THROUGHPUT = 0, 1, 2
  GATHER_EVENT_RECORDS, GATHER_LOGLIK_N, GATHER_RING_VALUES, GATHER_RING_WEIGHTS, GATHER_BALANCE, GATHER_COUNTERS,
  GATHER_PARAMS) = range(1, 17)
 TF_IDENTITY, TF_LOG, TF_LOGIT = 0, 1, 2      # sipnet_gpu_jitter_spec transforms
+PRIOR_FLAT, PRIOR_NORMAL = 0, 1              # sipnet_gpu_mh_spec priors
 
 ST_BAD_ALLOCATION, ST_RING_OVERFLOW, ST_CLAMPED, ST_DIED, ST_EVREC_OVERFLOW, \
     ST_NONFINITE, ST_REPLAY = 0x1, 0x2, 0x4, 0x8, 0x10, 0x20, 0x40
@@ -215,4 +216,16 @@ class JitterSpec(C.Structure):
         ("n_rows", C.c_int32), ("rows", C.POINTER(C.c_int32)), ("transform", C.POINTER(C.c_int32)),
         ("lower", C.POINTER(C.c_double)), ("upper", C.POINTER(C.c_double)),
         ("shrink", C.POINTER(C.c_double)), ("z", C.POINTER(C.c_double)),
+    ]
+
+
+class MHSpec(C.Structure):
+    """sipnet_gpu_mh_spec: the rows, priors, per-site scale and tempering, and the caller's random numbers of
+    sipnet_gpu_mh_move()."""
+    _fields_ = [
+        ("n_rows", C.c_int32), ("rows", C.POINTER(C.c_int32)), ("transform", C.POINTER(C.c_int32)),
+        ("lower", C.POINTER(C.c_double)), ("upper", C.POINTER(C.c_double)),
+        ("prior", C.POINTER(C.c_int32)), ("prior_a", C.POINTER(C.c_double)), ("prior_b", C.POINTER(C.c_double)),
+        ("scale", C.POINTER(C.c_double)), ("tempering", C.POINTER(C.c_double)),
+        ("current_loglik", C.POINTER(C.c_double)), ("z", C.POINTER(C.c_double)), ("log_u", C.POINTER(C.c_double)),
     ]

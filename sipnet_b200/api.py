@@ -141,6 +141,9 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     for name in ("sipnet_gpu_rejuvenate", "sipnet_gpu_comm_rejuvenate", "sipnet_gpu_multi_rejuvenate"):
         getattr(lib, name).restype = C.c_int
         getattr(lib, name).argtypes = [C.c_void_p, C.POINTER(A.JitterSpec), C.c_void_p]
+    for name in ("sipnet_gpu_mh_move", "sipnet_gpu_comm_mh_move", "sipnet_gpu_multi_mh_move"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [C.c_void_p, C.POINTER(A.MHSpec), C.c_void_p]
     lib.sipnet_gpu_eval_libm.restype = C.c_int
     lib.sipnet_gpu_eval_libm.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
     if path is None:
@@ -533,6 +536,59 @@ class Ensemble:
         holds this rank's members)."""
         return self._rejuvenate(self.lib.sipnet_gpu_comm_rejuvenate, self.comm, rows, transform, shrink, z, lower, upper)
 
+    def mh_spec(self, rows, transform, prior, prior_a, prior_b, scale, tempering, current_loglik, z, log_u,
+                lower=None, upper=None):
+        """(A.MHSpec, the arrays it points into) for sipnet_gpu_*_mh_move.  rows, transform, lower, upper: as
+        jitter_spec; prior: A.PRIOR_* per row with prior_a / prior_b (FLAT: bounds on theta; NORMAL: mean and sd of
+        phi); scale, tempering: [nsites] (scale NaN = leave the site alone); current_loglik, log_u: [nmembers];
+        z: [n_rows][nmembers]."""
+        M = self.nmembers
+        rows = np.ascontiguousarray(rows, dtype=np.int32).reshape(-1)
+        n = rows.size
+
+        def per_row(v, dt=np.float64):
+            return np.ascontiguousarray(np.broadcast_to(v, rows.shape), dtype=dt)
+
+        tf, pr, pa, pb = per_row(transform, np.int32), per_row(prior, np.int32), per_row(prior_a), per_row(prior_b)
+        scale = np.ascontiguousarray(np.broadcast_to(scale, (self.nsites,)), dtype=np.float64)
+        tau = np.ascontiguousarray(np.broadcast_to(tempering, (self.nsites,)), dtype=np.float64)
+        cl = np.ascontiguousarray(current_loglik, dtype=np.float64).reshape(-1)
+        lu = np.ascontiguousarray(log_u, dtype=np.float64).reshape(-1)
+        z = np.ascontiguousarray(z, dtype=np.float64)
+        if z.shape != (n, M) or cl.size != M or lu.size != M:
+            raise ValueError(f"z must be [{n}][{M}], current_loglik and log_u [{M}]")
+        lo = None if lower is None else per_row(lower)
+        hi = None if upper is None else per_row(upper)
+        spec = A.MHSpec(n, _ip(rows), _ip(tf), None if lo is None else _dp(lo), None if hi is None else _dp(hi),
+                        _ip(pr), _dp(pa), _dp(pb), _dp(scale), _dp(tau), _dp(cl), _dp(z), _dp(lu))
+        return spec, (rows, tf, lo, hi, pr, pa, pb, scale, tau, cl, z, lu)
+
+    def _mh_move(self, fn, target, args, kw) -> np.ndarray:
+        spec, keep = self.mh_spec(*args, **kw)
+        diag = np.empty((self.nsites, 4), np.float64)
+        self._check(fn(target, C.byref(spec), diag.ctypes.data))
+        if not np.isnan(keep[7]).all():            # every member was re-run: no run range is left
+            self.last_range = (self.last_range[1], self.last_range[1])
+        return diag
+
+    def mh_move(self, rows, transform, prior, prior_a, prior_b, scale, tempering, current_loglik, z, log_u,
+                lower=None, upper=None) -> np.ndarray:
+        """Tempered random-walk Metropolis-Hastings move of the listed parameter rows over the window [0, next step),
+        per site (sipnet_gpu_mh_move; see include/sipnet_gpu.h).  Every member is re-run; rejected ones get back
+        everything they had.  Afterwards there is no last run range.  Returns diag [nsites][4] =
+        (N, rank (-1: site left alone), invalid, accepted)."""
+        return self._mh_move(self.lib.sipnet_gpu_mh_move, self.handle,
+                             (rows, transform, prior, prior_a, prior_b, scale, tempering, current_loglik, z, log_u),
+                             dict(lower=lower, upper=upper))
+
+    def team_mh_move(self, rows, transform, prior, prior_a, prior_b, scale, tempering, current_loglik, z, log_u,
+                     lower=None, upper=None) -> np.ndarray:
+        """Collective.  mh_move() over the members of every rank (same arguments on every rank except
+        current_loglik, z and log_u, which hold this rank's members)."""
+        return self._mh_move(self.lib.sipnet_gpu_comm_mh_move, self.comm,
+                             (rows, transform, prior, prior_a, prior_b, scale, tempering, current_loglik, z, log_u),
+                             dict(lower=lower, upper=upper))
+
     def mean(self) -> np.ndarray:
         return self._gather(A.GATHER_MEAN, np.float64, (self.nsites, self.n_summary_cols, self.nrun))
 
@@ -721,6 +777,12 @@ class MultiEnsemble(Ensemble):
 
     def rejuvenate(self, rows, transform, shrink, z, lower=None, upper=None) -> np.ndarray:
         return self._rejuvenate(self.lib.sipnet_gpu_multi_rejuvenate, self.multi, rows, transform, shrink, z, lower, upper)
+
+    def mh_move(self, rows, transform, prior, prior_a, prior_b, scale, tempering, current_loglik, z, log_u,
+                lower=None, upper=None) -> np.ndarray:
+        return self._mh_move(self.lib.sipnet_gpu_multi_mh_move, self.multi,
+                             (rows, transform, prior, prior_a, prior_b, scale, tempering, current_loglik, z, log_u),
+                             dict(lower=lower, upper=upper))
 
     def sync(self) -> None:
         self.lib.sipnet_gpu_multi_sync(self.multi)

@@ -1612,15 +1612,12 @@ namespace {
 
 bool derived_row(int32_t r) { return r == SIPNET_P_psnTMax || r == SIPNET_P_coarseRootAllocation; }
 
-// the spec against `nsites` sites and `nmembers` members (z): 0, or SIPNET_GPU_ERR_BAD_ARGUMENT with the reason
-int check_jitter(const sipnet_gpu_jitter_spec *sp, int64_t nsites, int64_t nmembers) {
-  if (!sp || !sp->rows || !sp->transform || !sp->shrink || !sp->z)
-    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL jitter spec or array");
-  if (sp->n_rows < 1 || sp->n_rows > jt::kMaxRows)
-    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "n_rows must be 1..%d", jt::kMaxRows);
+// the moved rows of a spec (both moves): 0, or SIPNET_GPU_ERR_BAD_ARGUMENT with the reason
+int check_rows(int32_t nRows, const int32_t *rows, const int32_t *transform, const double *lower, const double *upper) {
+  if (nRows < 1 || nRows > jt::kMaxRows) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "n_rows must be 1..%d", jt::kMaxRows);
   bool seen[SIPNET_GPU_NPARAMS] = {};
-  for (int j = 0; j < sp->n_rows; ++j) {
-    const int32_t r = sp->rows[j], tf = sp->transform[j];
+  for (int j = 0; j < nRows; ++j) {
+    const int32_t r = rows[j], tf = transform[j];
     if (r < 0 || r >= SIPNET_GPU_NPARAMS) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "parameter row %d out of range", r);
     if (derived_row(r)) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "parameter row %d is derived by setupModel()", r);
     if (seen[r]) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "parameter row %d listed twice", r);
@@ -1628,20 +1625,32 @@ int check_jitter(const sipnet_gpu_jitter_spec *sp, int64_t nsites, int64_t nmemb
     if (tf != SIPNET_GPU_TF_IDENTITY && tf != SIPNET_GPU_TF_LOG && tf != SIPNET_GPU_TF_LOGIT)
       return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "unknown transform %d of row %d", tf, r);
     if (tf == SIPNET_GPU_TF_LOGIT) {
-      if (!sp->lower || !sp->upper) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "LOGIT row %d without lower / upper", r);
-      const double lo = sp->lower[j], hi = sp->upper[j];
+      if (!lower || !upper) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "LOGIT row %d without lower / upper", r);
+      const double lo = lower[j], hi = upper[j];
       if (!std::isfinite(lo) || !std::isfinite(hi) || !(lo < hi))
         return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "LOGIT bounds of row %d must be finite with lower < upper", r);
     }
   }
+  return 0;
+}
+
+int check_normals(const double *z, int32_t nRows, int64_t nmembers) {
+  for (size_t i = 0; i < (size_t)nRows * (size_t)nmembers; ++i)
+    if (!std::isfinite(z[i])) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "z[%zu] is not finite", i);
+  return 0;
+}
+
+// the spec against `nsites` sites and `nmembers` members (z): 0, or SIPNET_GPU_ERR_BAD_ARGUMENT with the reason
+int check_jitter(const sipnet_gpu_jitter_spec *sp, int64_t nsites, int64_t nmembers) {
+  if (!sp || !sp->rows || !sp->transform || !sp->shrink || !sp->z)
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL jitter spec or array");
+  if (int rc = check_rows(sp->n_rows, sp->rows, sp->transform, sp->lower, sp->upper)) return rc;
   for (int64_t s = 0; s < nsites; ++s) {
     const double a = sp->shrink[s];
     if (!std::isnan(a) && !(a > 0.0 && a < 1.0))
       return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "shrink[%lld] = %g is neither NaN nor in (0, 1)", (long long)s, a);
   }
-  for (size_t i = 0; i < (size_t)sp->n_rows * (size_t)nmembers; ++i)
-    if (!std::isfinite(sp->z[i])) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "z[%zu] is not finite", i);
-  return 0;
+  return check_normals(sp->z, sp->n_rows, nmembers);
 }
 
 uint64_t jitter_hash(const sipnet_gpu_jitter_spec *sp, int64_t nsites) {
@@ -1655,76 +1664,96 @@ uint64_t jitter_hash(const sipnet_gpu_jitter_spec *sp, int64_t nsites) {
   return h.add(sp->shrink, (size_t)nsites * sizeof(double)).value();
 }
 
+// The arguments of the move's kernels on local rank `l` (scratch made, rows checked): the handle, the rows, the
+// chunk records and a team's exchange buffer (grown here); the caller sets the per-site move arguments.
+int jitter_args(sipnet_gpu_comm *c, Local &l, int32_t n, const int32_t *rows, const int32_t *transform,
+                const double *lower, const double *upper, jt::Args &a) {
+  sipnet_gpu_handle *h = l.h;
+  const int R = c->nranks;
+  const int64_t S = h->nsites;
+  if (S != c->local[0].h->nsites) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites");
+  CUDA_OK(cudaSetDevice(h->device));
+  if (int rc = jt::ensure_scratch(h)) return rc;
+  if (R > 1)
+    if (int rc = grow(l.xchg, l.xchgCap, (size_t)R * S * jt::kRec * sizeof(double), h->stream)) return rc;
+  memset(&a, 0, sizeof a);
+  a.params = h->params;
+  a.status = h->status;
+  a.ld = h->ld;
+  a.nmembers = h->nmembers;
+  a.sites = h->sites;
+  a.nsites = (int32_t)S;
+  a.nchunks = (int32_t)h->nchunks;
+  a.chunk = h->chunk;
+  a.siteChunks = h->siteChunks;
+  a.nrows = n;
+  a.nranks = R;
+  a.rank = l.rank;
+  for (int j = 0; j < n; ++j) {
+    a.rows[j] = rows[j];
+    a.transform[j] = transform[j];
+    a.lower[j] = transform[j] == SIPNET_GPU_TF_LOGIT ? lower[j] : 0.0;
+    a.upper[j] = transform[j] == SIPNET_GPU_TF_LOGIT ? upper[j] : 0.0;
+  }
+  a.z = h->jtZ;
+  a.part = h->jtPart;
+  a.mom = h->jtMom;
+  a.coef = h->jtCoef;
+  a.diag = h->jtDiag;
+  a.rankRec = reinterpret_cast<double *>(l.xchg);
+  return 0;
+}
+
+// One pass of the move on every local rank: members(pass) (unless the chunk records are already written), site(pass),
+// and for a team the exchange of the per-site partials and combine(pass).
+int jitter_pass(sipnet_gpu_comm *c, std::vector<jt::Args> &args, int pass, bool members, const char *what) {
+  for (size_t i = 0; i < c->local.size(); ++i) {
+    sipnet_gpu_handle *h = c->local[i].h;
+    CUDA_OK(cudaSetDevice(h->device));
+    if (members)
+      if (int rc = launched(h, jt::launch_members(args[i], pass, h->stream), what)) return rc;
+    if (int rc = launched(h, jt::launch_site(args[i], pass, h->stream), what)) return rc;
+  }
+  if (c->nranks > 1) {
+    const size_t bytes = (size_t)c->local[0].h->nsites * jt::kRec * sizeof(double);
+    if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.xchg; })) return rc;
+    for (size_t i = 0; i < c->local.size(); ++i) {
+      sipnet_gpu_handle *h = c->local[i].h;
+      CUDA_OK(cudaSetDevice(h->device));
+      if (int rc = launched(h, jt::launch_combine(args[i], pass, h->stream), what)) return rc;
+    }
+  }
+  return 0;
+}
+
+// local rank 0's diagnostics into diag (may be NULL), and every local stream finished
+int jitter_diag(sipnet_gpu_comm *c, double *diag) {
+  if (diag) {
+    sipnet_gpu_handle *h = c->local[0].h;
+    CUDA_OK(cudaSetDevice(h->device));
+    CUDA_OK(cudaMemcpyAsync(diag, h->jtDiag, (size_t)h->nsites * 4 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  }
+  return sync_all(c);
+}
+
 // Move every local rank of `c` (all ranks hold the same sites): shrink holds the handles' sites, z[i] local rank i's
 // members.  A team of one needs no exchange and no host round trip; a larger team all-gathers the per-site partial
 // sums of the two moment passes and of the counts, and sums them in rank order on every rank.  diag (may be NULL)
 // gets local rank 0's [nsites][4].
 int run_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *sp, const double *shrink,
                    const std::vector<const double *> &z, double *diag) {
-  const int R = c->nranks, n = sp->n_rows;
-  const int64_t S = c->local[0].h->nsites;
+  const int n = sp->n_rows;
   std::vector<jt::Args> args(c->local.size());
   for (size_t i = 0; i < c->local.size(); ++i) {
-    Local &l = c->local[i];
-    sipnet_gpu_handle *h = l.h;
-    if (h->nsites != S) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the ranks of a team must hold the same sites");
-    CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = jt::ensure_scratch(h)) return rc;
-    if (R > 1)
-      if (int rc = grow(l.xchg, l.xchgCap, (size_t)R * S * jt::kRec * sizeof(double), h->stream)) return rc;
-    CUDA_OK(cudaMemcpyAsync(h->jtShrink, shrink, (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    sipnet_gpu_handle *h = c->local[i].h;
+    if (int rc = jitter_args(c, c->local[i], n, sp->rows, sp->transform, sp->lower, sp->upper, args[i])) return rc;
+    CUDA_OK(cudaMemcpyAsync(h->jtShrink, shrink, (size_t)h->nsites * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CUDA_OK(cudaMemcpyAsync(h->jtZ, z[i], (size_t)n * h->nmembers * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    jt::Args &a = args[i];
-    memset(&a, 0, sizeof a);
-    a.params = h->params;
-    a.status = h->status;
-    a.ld = h->ld;
-    a.nmembers = h->nmembers;
-    a.sites = h->sites;
-    a.nsites = (int32_t)S;
-    a.nchunks = (int32_t)h->nchunks;
-    a.chunk = h->chunk;
-    a.siteChunks = h->siteChunks;
-    a.nrows = n;
-    a.nranks = R;
-    a.rank = l.rank;
-    for (int j = 0; j < n; ++j) {
-      a.rows[j] = sp->rows[j];
-      a.transform[j] = sp->transform[j];
-      a.lower[j] = sp->transform[j] == SIPNET_GPU_TF_LOGIT ? sp->lower[j] : 0.0;
-      a.upper[j] = sp->transform[j] == SIPNET_GPU_TF_LOGIT ? sp->upper[j] : 0.0;
-    }
-    a.shrink = h->jtShrink;
-    a.z = h->jtZ;
-    a.part = h->jtPart;
-    a.mom = h->jtMom;
-    a.coef = h->jtCoef;
-    a.diag = h->jtDiag;
-    a.rankRec = reinterpret_cast<double *>(l.xchg);
+    args[i].shrink = h->jtShrink;
   }
-  for (int pass = 1; pass <= 3; ++pass) {
-    for (size_t i = 0; i < c->local.size(); ++i) {
-      sipnet_gpu_handle *h = c->local[i].h;
-      CUDA_OK(cudaSetDevice(h->device));
-      if (int rc = launched(h, jt::launch_members(args[i], pass, h->stream), "rejuvenation")) return rc;
-      if (int rc = launched(h, jt::launch_site(args[i], pass, h->stream), "rejuvenation")) return rc;
-    }
-    if (R > 1) {
-      if (int rc = all_gather_bytes(c, (size_t)S * jt::kRec * sizeof(double), [](Local &l) -> void * { return l.xchg; }))
-        return rc;
-      for (size_t i = 0; i < c->local.size(); ++i) {
-        sipnet_gpu_handle *h = c->local[i].h;
-        CUDA_OK(cudaSetDevice(h->device));
-        if (int rc = launched(h, jt::launch_combine(args[i], pass, h->stream), "rejuvenation")) return rc;
-      }
-    }
-  }
-  if (diag) {
-    sipnet_gpu_handle *h = c->local[0].h;
-    CUDA_OK(cudaSetDevice(h->device));
-    CUDA_OK(cudaMemcpyAsync(diag, h->jtDiag, (size_t)S * 4 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  }
-  return sync_all(c);
+  for (int pass = 1; pass <= 3; ++pass)
+    if (int rc = jitter_pass(c, args, pass, true, "rejuvenation")) return rc;
+  return jitter_diag(c, diag);
 }
 
 }  // namespace
@@ -1768,6 +1797,225 @@ extern "C" int sipnet_gpu_multi_rejuvenate(sipnet_gpu_multi *m, const sipnet_gpu
     sipnet_gpu_comm one = team_of_one(m->handles[d]);
     const size_t s0 = (size_t)m->parts[d].site0;
     if (int rc = run_rejuvenate(&one, spec, spec->shrink + s0, {zd[d].data()}, diag ? diag + s0 * 4 : nullptr)) return rc;
+  }
+  return 0;
+}
+
+// ---- parameter calibration: the Metropolis-Hastings move (sip_jitter.cuh proposes, sip_resample.cuh decides) ------
+namespace {
+
+// the spec against `nsites` sites, `nmembers` members, the next step and whether the handles keep a log-likelihood
+int check_mh(const sipnet_gpu_mh_spec *sp, int64_t nsites, int64_t nmembers, int64_t step, bool hasLoglik) {
+  if (!sp || !sp->rows || !sp->transform || !sp->prior || !sp->prior_a || !sp->prior_b || !sp->scale || !sp->tempering ||
+      !sp->current_loglik || !sp->z || !sp->log_u)
+    return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL Metropolis-Hastings spec or array");
+  if (int rc = check_rows(sp->n_rows, sp->rows, sp->transform, sp->lower, sp->upper)) return rc;
+  for (int j = 0; j < sp->n_rows; ++j) {
+    const double a = sp->prior_a[j], b = sp->prior_b[j];
+    if (sp->prior[j] == SIPNET_GPU_PRIOR_FLAT) {
+      if (std::isnan(a) || std::isnan(b) || !(a < b))
+        return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "FLAT prior of row %d needs prior_a < prior_b", sp->rows[j]);
+      if (sp->transform[j] == SIPNET_GPU_TF_LOGIT && !(a >= sp->lower[j] && b <= sp->upper[j]))
+        return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "FLAT prior of LOGIT row %d must lie inside [lower, upper]", sp->rows[j]);
+    } else if (sp->prior[j] == SIPNET_GPU_PRIOR_NORMAL) {
+      if (!std::isfinite(a) || !std::isfinite(b) || !(b > 0.0))
+        return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NORMAL prior of row %d needs a finite mean and a finite sd > 0",
+                    sp->rows[j]);
+    } else {
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "unknown prior %d of row %d", sp->prior[j], sp->rows[j]);
+    }
+  }
+  for (int64_t s = 0; s < nsites; ++s) {
+    const double h = sp->scale[s], t = sp->tempering[s];
+    if (!std::isnan(h) && !(std::isfinite(h) && h > 0.0))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "scale[%lld] = %g is neither NaN nor finite > 0", (long long)s, h);
+    if (!(t >= 0.0 && t <= 1.0))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "tempering[%lld] = %g is not in [0, 1]", (long long)s, t);
+    if (!std::isnan(h) && t > 0.0 && !hasLoglik)
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "tempering[%lld] > 0 on a handle without SIPNET_GPU_OUT_LOGLIK", (long long)s);
+  }
+  if (int rc = check_normals(sp->z, sp->n_rows, nmembers)) return rc;
+  for (int64_t i = 0; i < nmembers; ++i)
+    if (!(sp->log_u[i] <= 0.0))
+      return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "log_u[%lld] = %g is not <= 0", (long long)i, sp->log_u[i]);
+  if (step < 1) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "the window [0, s) is empty: run at least one step first");
+  return 0;
+}
+
+// everything the ranks of a team must agree on (all but the per-member arrays)
+uint64_t mh_hash(const sipnet_gpu_mh_spec *sp, int64_t nsites, int64_t step, bool hasLoglik) {
+  const size_t n = (size_t)sp->n_rows;
+  const uint8_t ll = hasLoglik;
+  ArgHash h;
+  h.add(&nsites, sizeof nsites).add(&step, sizeof step).add(&ll, 1).add(&sp->n_rows, sizeof sp->n_rows)
+      .add(sp->rows, n * sizeof(int32_t)).add(sp->transform, n * sizeof(int32_t)).add(sp->prior, n * sizeof(int32_t))
+      .add(sp->prior_a, n * sizeof(double)).add(sp->prior_b, n * sizeof(double));
+  for (size_t j = 0; j < n; ++j)
+    if (sp->transform[j] == SIPNET_GPU_TF_LOGIT) h.add(&sp->lower[j], sizeof(double)).add(&sp->upper[j], sizeof(double));
+  return h.add(sp->scale, (size_t)nsites * sizeof(double)).add(sp->tempering, (size_t)nsites * sizeof(double)).value();
+}
+
+// reset() and run(0, s) of one handle, in pieces its output buffers hold
+int rerun_window(sipnet_gpu_handle *h, int64_t s) {
+  if (int rc = sipnet_gpu_reset(h)) return rc;
+  const int64_t piece = (h->out || h->dbg) && h->outCap > 0 ? h->outCap : s;
+  for (int64_t b = 0; b < s; b += piece)
+    if (int rc = sipnet_gpu_run(h, b, std::min(s, b + piece))) return rc;
+  return 0;
+}
+
+// Move every local rank of `c` (all ranks hold the same sites): scale and tau hold the handles' sites, curL[i], z[i]
+// and logU[i] local rank i's members.  The sequence: the two moment passes (a team exchanges their partials), the
+// snapshot, the proposal, reset and run of every local handle over its window (no exchange), the accept pass, and the
+// site pass of the counts (a team exchanges them).  diag (may be NULL) gets local rank 0's [nsites][4].
+int run_mh(sipnet_gpu_comm *c, const sipnet_gpu_mh_spec *sp, const double *scale, const double *tau,
+           const std::vector<const double *> &curL, const std::vector<const double *> &z,
+           const std::vector<const double *> &logU, double *diag) {
+  const int n = sp->n_rows;
+  const int64_t S = c->local[0].h->nsites;
+  const size_t L = c->local.size();
+  if (std::all_of(scale, scale + S, [](double v) { return std::isnan(v); })) {  // no site moves: nothing to launch
+    if (diag)
+      for (int64_t s = 0; s < S; ++s) {
+        double *d = diag + s * 4;
+        d[0] = __builtin_nan("");
+        d[1] = -1.0;
+        d[2] = d[3] = 0.0;
+      }
+    return 0;
+  }
+  std::vector<jt::Args> args(L);
+  std::vector<rs::Args> acc(L);
+  std::vector<int64_t> window(L);
+  for (size_t i = 0; i < L; ++i) {
+    sipnet_gpu_handle *h = c->local[i].h;
+    if (int rc = jitter_args(c, c->local[i], n, sp->rows, sp->transform, sp->lower, sp->upper, args[i])) return rc;
+    if (int rc = rs::ensure_mh_scratch(h)) return rc;
+    const size_t M = (size_t)h->nmembers;
+    CUDA_OK(cudaMemcpyAsync(h->mhScale, scale, (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(cudaMemcpyAsync(h->mhTau, tau, (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(cudaMemcpyAsync(h->jtZ, z[i], (size_t)n * M * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(cudaMemcpyAsync(h->mhCurL, curL[i], M * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(cudaMemcpyAsync(h->mhLogU, logU[i], M * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    jt::Args &a = args[i];
+    a.scale = h->mhScale;
+    a.curLoglik = h->mhCurL;
+    for (int j = 0; j < n; ++j) {
+      a.prior[j] = sp->prior[j];
+      a.priorA[j] = sp->prior_a[j];
+      a.priorB[j] = sp->prior_b[j];
+    }
+    a.valid = h->mhValid;
+    a.dlp = h->mhDlp;
+    rs::Args &r = acc[i];
+    memset(&r, 0, sizeof r);
+    r.status = h->status;
+    r.sites = h->sites;
+    r.nmembers = h->nmembers;
+    r.ld = h->ld;
+    r.nsites = (int32_t)S;
+    r.nchunks = (int32_t)h->nchunks;
+    r.chunk = h->chunk;
+    r.params = h->params;
+    r.state = h->state;
+    r.ringV = h->ringV;
+    r.ringW = h->ringW;
+    r.loglik = h->loglik;
+    r.loglikN = h->loglikN;
+    r.counters = h->counters;
+    r.recs = h->recs;
+    r.recCount = h->recCount;
+    r.ringCap = h->ringCap;
+    r.maxRecs = h->maxRecs;
+    r.words = rs::record_words(h);
+    r.snap = h->mhSnap;
+    r.valid = h->mhValid;
+    r.dlp = h->mhDlp;
+    r.curLoglik = h->mhCurL;
+    r.logU = h->mhLogU;
+    r.tau = h->mhTau;
+    r.count = h->jtPart;
+    r.countStride = jt::kRec;
+    window[i] = h->stepsDone;
+  }
+  for (int pass = 1; pass <= 2; ++pass)
+    if (int rc = jitter_pass(c, args, pass, true, "Metropolis-Hastings")) return rc;
+  for (size_t i = 0; i < L; ++i) {
+    sipnet_gpu_handle *h = c->local[i].h;
+    CUDA_OK(cudaSetDevice(h->device));
+    if (int rc = launched(h, rs::launch_snapshot(acc[i], h->stream), "Metropolis-Hastings")) return rc;
+    if (int rc = launched(h, jt::launch_members(args[i], 3, h->stream), "Metropolis-Hastings")) return rc;
+  }
+  for (size_t i = 0; i < L; ++i)  // asynchronous: the devices run side by side
+    if (int rc = rerun_window(c->local[i].h, window[i])) return rc;
+  for (size_t i = 0; i < L; ++i) {
+    sipnet_gpu_handle *h = c->local[i].h;
+    CUDA_OK(cudaSetDevice(h->device));
+    if (int rc = launched(h, rs::launch_accept(acc[i], h->stream), "Metropolis-Hastings")) return rc;
+    h->lastBegin = h->lastEnd = window[i];  // no run range: its outputs are the proposals' (or are gone)
+    h->summariesValid = false;
+  }
+  if (int rc = jitter_pass(c, args, 3, false, "Metropolis-Hastings")) return rc;
+  return jitter_diag(c, diag);
+}
+
+}  // namespace
+
+extern "C" int sipnet_gpu_mh_move(sipnet_gpu_handle *h, const sipnet_gpu_mh_spec *spec, double *diag) {
+  if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  if (int rc = check_mh(spec, h->nsites, h->nmembers, h->stepsDone, h->loglik != nullptr)) return rc;
+  sipnet_gpu_comm one = team_of_one(h);
+  return run_mh(&one, spec, spec->scale, spec->tempering, {spec->current_loglik}, {spec->z}, {spec->log_u}, diag);
+}
+
+extern "C" int sipnet_gpu_comm_mh_move(sipnet_gpu_comm *c, const sipnet_gpu_mh_spec *spec, double *diag) {
+  if (!c) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL comm");
+  sipnet_gpu_handle *h = c->local[0].h;
+  const int64_t S = h->nsites;
+  const bool ll = h->loglik != nullptr;
+  const int bad = check_mh(spec, S, h->nmembers, h->stepsDone, ll);
+  if (int rc = team_agree(c, bad, bad ? 0 : mh_hash(spec, S, h->stepsDone, ll), "Metropolis-Hastings specs")) return rc;
+  const size_t L = c->local.size();
+  return run_mh(c, spec, spec->scale, spec->tempering, std::vector<const double *>(L, spec->current_loglik),
+                std::vector<const double *>(L, spec->z), std::vector<const double *>(L, spec->log_u), diag);
+}
+
+extern "C" int sipnet_gpu_multi_mh_move(sipnet_gpu_multi *m, const sipnet_gpu_mh_spec *spec, double *diag) {
+  if (!m) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
+  int64_t step = 0;
+  for (const sipnet_gpu_handle *h : m->handles) step = std::max(step, h->stepsDone);
+  if (int rc = check_mh(spec, m->nsites, m->nmembers, step, m->handles[0]->loglik != nullptr)) return rc;
+  const size_t D = m->handles.size(), n = (size_t)spec->n_rows, M = (size_t)m->nmembers;
+  // every device's normals [n_rows][its members], log-likelihoods and log u, from the configuration-order arrays
+  std::vector<std::vector<double>> zd(D), cl(D), lu(D);
+  for (size_t d = 0; d < D; ++d) {
+    const size_t nm = (size_t)m->handles[d]->nmembers;
+    zd[d].resize(n * nm);
+    cl[d].resize(nm);
+    lu[d].resize(nm);
+    for (const sipnet_gpu_multi::Run &r : m->parts[d].runs) {
+      for (size_t j = 0; j < n; ++j)
+        memcpy(zd[d].data() + j * nm + r.local0, spec->z + j * M + r.global0, (size_t)r.count * sizeof(double));
+      memcpy(cl[d].data() + r.local0, spec->current_loglik + r.global0, (size_t)r.count * sizeof(double));
+      memcpy(lu[d].data() + r.local0, spec->log_u + r.global0, (size_t)r.count * sizeof(double));
+    }
+  }
+  if (m->split) {  // every device ends with the same diagnostics: take device 0's
+    std::vector<const double *> zp, cp, up;
+    for (size_t d = 0; d < D; ++d) {
+      zp.push_back(zd[d].data());
+      cp.push_back(cl[d].data());
+      up.push_back(lu[d].data());
+    }
+    return run_mh(m->comm, spec, spec->scale, spec->tempering, cp, zp, up, diag);
+  }
+  // whole sites: each device alone on its site range
+  for (size_t d = 0; d < D; ++d) {
+    sipnet_gpu_comm one = team_of_one(m->handles[d]);
+    const size_t s0 = (size_t)m->parts[d].site0;
+    if (int rc = run_mh(&one, spec, spec->scale + s0, spec->tempering + s0, {cl[d].data()}, {zd[d].data()},
+                        {lu[d].data()}, diag ? diag + s0 * 4 : nullptr))
+      return rc;
   }
   return 0;
 }

@@ -70,6 +70,11 @@ struct sipnet_gpu_handle {
   size_t rsSiteCap = 0, rsTabCap = 0, rsSendCap = 0, rsRecvCap = 0;  // elements
   // parameter move scratch (sip_jitter.cu), made by the first rejuvenation
   double *jtPart = nullptr, *jtMom = nullptr, *jtCoef = nullptr, *jtDiag = nullptr, *jtShrink = nullptr, *jtZ = nullptr;
+  // Metropolis-Hastings move scratch (sip_resample.cu), made by the first move: the members' snapshot
+  // ([rs::snapshot_words][ld]), the proposal's verdict and log-prior difference, the uploaded per-member and per-site
+  // arguments
+  double *mhSnap = nullptr, *mhDlp = nullptr, *mhCurL = nullptr, *mhLogU = nullptr, *mhScale = nullptr, *mhTau = nullptr;
+  int8_t *mhValid = nullptr;
 };
 
 namespace sip {
@@ -83,6 +88,8 @@ int ensure_summaries(sipnet_gpu_handle *h);
 constexpr int kChunk = 128;
 // members no filter counts or changes
 constexpr uint32_t kExcluded = SIPNET_GPU_ST_BAD_ALLOCATION | SIPNET_GPU_ST_NONFINITE;
+// a member's Metropolis-Hastings proposal, from the proposal pass (sip_jitter.cu) to the accept pass (sip_resample.cu)
+constexpr int8_t kMhNone = 0, kMhInvalid = 1, kMhValid = 2;
 // the handle's chunk tables, made once (sipnet_gpu.cu): chunk[nchunks] = (site, first site-local member),
 // siteChunks[nsites] = (first chunk, chunk count), sites in order and a site's chunks in member order
 int ensure_chunks(sipnet_gpu_handle *h);

@@ -1,4 +1,4 @@
-// sip_jitter.cu -- kernels of the Liu-West parameter move (see sip_jitter.cuh for the sequence of launches and the
+// sip_jitter.cu -- kernels of the Liu-West parameter move and of the Metropolis-Hastings proposal (see sip_jitter.cuh for the sequence of launches and the
 // reduction order).  Compiled with -fmad=false like the rest of the model path: every product and sum below is rounded
 // on its own, and the re-derivation of the dependent rows is setupModel()'s own (sip_derive.cuh).
 #include <cuda_runtime.h>
@@ -36,7 +36,20 @@ __device__ __forceinline__ double inverse(double p, int tf, double lo, double hi
   return p;
 }
 
-// member m's transformed rows; false when it does not take part
+// log density of row j's prior in phi at theta = t, phi = p, constants dropped (include/sipnet_gpu.h mh_move)
+__device__ __forceinline__ double log_prior(const Args &a, int j, double t, double p) {
+  if (a.prior[j] == SIPNET_GPU_PRIOR_NORMAL) {
+    const double d = p - a.priorA[j];
+    return -(d * d) / (2.0 * (a.priorB[j] * a.priorB[j]));
+  }
+  if (!(t >= a.priorA[j] && t <= a.priorB[j])) return -INFINITY;
+  if (a.transform[j] == SIPNET_GPU_TF_LOG) return p;  // log |dtheta / dphi|
+  if (a.transform[j] == SIPNET_GPU_TF_LOGIT) return log((t - a.lower[j]) * (a.upper[j] - t) / (a.upper[j] - a.lower[j]));
+  return 0.0;
+}
+
+// member m's transformed rows; false when it does not take part (the MH move also needs a finite current
+// log-likelihood and log prior)
 __device__ __forceinline__ bool load_phi(const Args &a, int64_t m, double (&phi)[kMaxRows]) {
   bool in = (a.status[m] & kExcluded) == 0;
 #pragma unroll
@@ -45,8 +58,18 @@ __device__ __forceinline__ bool load_phi(const Args &a, int64_t m, double (&phi)
       const double t = a.params[(int64_t)a.rows[j] * a.ld + m];
       in = in && in_domain(t, a.transform[j], a.lower[j], a.upper[j]);
       phi[j] = in ? forward(t, a.transform[j], a.lower[j], a.upper[j]) : 0.0;
+      if (a.scale) in = in && log_prior(a, j, t, phi[j]) > -INFINITY;
     }
+  if (a.scale) in = in && isfinite(a.curLoglik[m]);
   return in;
+}
+
+// the move's (a, h) at site s: Liu-West (a = shrink, h = sqrt(1 - a^2)) or Metropolis-Hastings (a = 1, h = scale);
+// h NaN: the site stays
+__device__ __forceinline__ double2 move_ah(const Args &a, int s) {
+  if (a.scale) return make_double2(1.0, a.scale[s]);
+  const double sa = a.shrink[s];
+  return make_double2(sa, sqrt(1.0 - sa * sa));
 }
 
 // the quantities of a pass inside a record: [q0, q0 + count)
@@ -70,7 +93,10 @@ __global__ void __launch_bounds__(kWarps * 32) members_kernel(const Args a) {
   const int n = a.nrows;
   if (PASS == 3) {
     const double *cf = a.coef + (size_t)ch.x * kCoef;
+    const bool mh = a.scale != nullptr;
     if (cf[0] == 0.0) {  // the site does not move
+      if (mh)
+        for (int i = lane; i < cnt; i += 32) a.valid[(int64_t)member0 + ch.y + i] = kMhNone;
       if (lane == 0) a.part[(size_t)c * kRec] = a.part[(size_t)c * kRec + 1] = 0.0;
       return;
     }
@@ -79,8 +105,12 @@ __global__ void __launch_bounds__(kWarps * 32) members_kernel(const Args a) {
     for (int i = lane; i < cnt; i += 32) {
       const int64_t m = (int64_t)member0 + ch.y + i;
       double phi[kMaxRows], zz[kMaxRows], th[kMaxRows];
-      if (!load_phi(a, m, phi)) continue;
+      if (!load_phi(a, m, phi)) {
+        if (mh) a.valid[m] = kMhNone;
+        continue;
+      }
       bool ok = true;
+      double dl = 0.0;  // MH: sum_j lp_j(phi') - lp_j(phi)
 #pragma unroll
       for (int j = 0; j < kMaxRows; ++j)
         if (j < n) zz[j] = a.z[(int64_t)j * a.nmembers + m];
@@ -93,6 +123,11 @@ __global__ void __launch_bounds__(kWarps * 32) members_kernel(const Args a) {
           const double p = (sa * phi[j] + cf[3 + j]) + s;
           th[j] = inverse(p, a.transform[j], a.lower[j], a.upper[j]);
           ok = ok && in_domain(th[j], a.transform[j], a.lower[j], a.upper[j]);
+          if (mh && ok) {
+            const double l1 = log_prior(a, j, th[j], p);
+            ok = l1 > -INFINITY;
+            dl += l1 - log_prior(a, j, a.params[(int64_t)a.rows[j] * a.ld + m], phi[j]);
+          }
         }
       auto P = [&](int k) -> double & { return a.params[(int64_t)k * a.ld + m]; };
       if (ok) {  // ensureAllocation on the proposed fractions, before anything is written
@@ -107,6 +142,7 @@ __global__ void __launch_bounds__(kWarps * 32) members_kernel(const Args a) {
       }
       if (!ok) {
         ++kept;
+        if (mh) a.valid[m] = kMhInvalid;
         continue;
       }
 #pragma unroll
@@ -114,6 +150,10 @@ __global__ void __launch_bounds__(kWarps * 32) members_kernel(const Args a) {
         if (j < n) P(a.rows[j]) = th[j];
       derive_dependent(P);
       ++moved;
+      if (mh) {
+        a.valid[m] = kMhValid;
+        a.dlp[m] = dl;
+      }
     }
     moved = __reduce_add_sync(kFull, moved);
     kept = __reduce_add_sync(kFull, kept);
@@ -179,9 +219,10 @@ __device__ void finish(const Args &a, int s, const double *r) {
     }
     return;
   }
-  const double N = mom[0], sa = a.shrink[s];
+  const double N = mom[0];
+  const double2 ah = move_ah(a, s);
   cf[0] = 0.0;
-  if (isnan(sa) || N < 2.0) return;
+  if (isnan(ah.y) || N < 2.0) return;
   // V (population covariance) and its semidefinite Cholesky factor, column by column
   double L[kTri];
   int rank = 0;
@@ -203,7 +244,7 @@ __device__ void finish(const Args &a, int s, const double *r) {
       for (int i = j; i < n; ++i) L[tri(i, j)] = 0.0;
     }
   }
-  const double h = sqrt(1.0 - sa * sa);
+  const double sa = ah.x, h = ah.y;
   cf[0] = 1.0;
   cf[1] = sa;
   cf[2] = (double)rank;

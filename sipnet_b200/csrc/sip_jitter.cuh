@@ -11,6 +11,9 @@
 //   members(3)      propose, invert, re-derive (sip_derive.cuh), accept or keep; moved / kept per chunk
 //   site(3)         -> per site diagnostics {N, rank, moved, kept} (team: + combine)
 // Six launches on one GPU, whatever the number of sites.
+// The Metropolis-Hastings move (Args::scale set) runs the same passes with a = 1, h = scale and its own participants;
+// members(3) also records each member's verdict, and site(3) runs after the accept pass of sip_resample.cu, whose
+// per-chunk counts {invalid, accepted} it turns into diag (sip_comm.cu run_mh).
 //
 // Reduction order: the handle's 128-member chunks of site-local indices (sipnet_gpu_handle::chunk).  Inside a chunk,
 // a lane sums one quantity over the chunk's members in index order; a site sums its chunks in chunk order; a team
@@ -59,6 +62,15 @@ struct Args {
   double *coef;          // [nsites][kCoef]
   double *diag;          // [nsites][4]
   double *rankRec;       // [nranks][nsites][kRec] (teams only)
+  // The Metropolis-Hastings proposal (sipnet_gpu_mh_move) when scale != NULL: a = 1 and h = scale[s] per site (the
+  // Liu-West move: a = shrink[s], h = sqrt(1 - a^2)); a participant also needs a finite current log-likelihood and
+  // log prior; members(3) writes every member's verdict (kMh*) and, for a valid proposal, lp(phi') - lp(phi).
+  const double *scale;      // [nsites]
+  const double *curLoglik;  // [nmembers]
+  int32_t prior[kMaxRows];  // SIPNET_GPU_PRIOR_*
+  double priorA[kMaxRows], priorB[kMaxRows];
+  int8_t *valid;            // [nmembers]
+  double *dlp;              // [nmembers]
 };
 
 // the handle's chunk tables and scratch (made once, by the first call)

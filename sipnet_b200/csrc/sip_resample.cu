@@ -310,6 +310,64 @@ __global__ void __launch_bounds__(128) unpack_kernel(const Args a) {
   }
 }
 
+// word w of member m's snapshot: LOAD reads the member into v, else v goes back into the member
+template <bool LOAD>
+__device__ __forceinline__ void snapshot_word(const Args &a, int w, int64_t m, double &v) {
+  const int rec = a.words - 1;  // the record without the ancestor's index
+  if (w < rec) return record_word<LOAD>(a, w, m, v);
+  double *p = w == rec ? a.loglik : a.loglikN;
+  if (!p) {
+    if (LOAD) v = 0.0;
+  } else if (LOAD) {
+    v = p[m];
+  } else {
+    p[m] = v;
+  }
+}
+
+// one thread per member (x) and group of snapshot words (y)
+__global__ void __launch_bounds__(128) snapshot_kernel(const Args a) {
+  const int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (m >= a.nmembers) return;
+  const int k0 = blockIdx.y * kWordsPerY, k1 = min(k0 + kWordsPerY, a.words + 1);
+  for (int w = k0; w < k1; ++w) {
+    double v;
+    snapshot_word<true>(a, w, m, v);
+    a.snap[(int64_t)w * a.ld + m] = v;
+  }
+}
+
+// One CTA per chunk, thread i = the chunk's member i.  A member is accepted iff its proposal was valid, the run left
+// it a finite log-likelihood and no excluded status bit, and log u < delta; every other member gets its snapshot back.
+__global__ void __launch_bounds__(kChunk) accept_kernel(const Args a) {
+  const int c = blockIdx.x;
+  if (c >= a.nchunks) return;  // block-uniform
+  const int2 ch = a.chunk[c];
+  const int idx = ch.y + (int)threadIdx.x;
+  const bool here = idx < a.sites[ch.x].memberCount;
+  const int64_t m = (int64_t)a.sites[ch.x].member0 + idx;
+  int8_t v = kMhNone;
+  bool acc = false;
+  if (here) {
+    v = a.valid[m];
+    if (v == kMhValid) {
+      const double l = a.loglik ? a.loglik[m] : 0.0, t = a.tau[ch.x];
+      const double delta = (t == 0.0 ? 0.0 : t * (l - a.curLoglik[m])) + a.dlp[m];
+      acc = isfinite(l) && (a.status[m] & kExcluded) == 0 && a.logU[m] < delta;
+    }
+    if (!acc)
+      for (int w = 0; w <= a.words; ++w) {
+        double x = a.snap[(int64_t)w * a.ld + m];
+        snapshot_word<false>(a, w, m, x);
+      }
+  }
+  const int invalid = __syncthreads_count(v == kMhInvalid), accepted = __syncthreads_count(acc);
+  if (threadIdx.x == 0) {
+    a.count[(size_t)c * a.countStride] = (double)invalid;
+    a.count[(size_t)c * a.countStride + 1] = (double)accepted;
+  }
+}
+
 unsigned blocks_for(int64_t units, int per) { return (unsigned)std::max<int64_t>((units + per - 1) / per, 1); }
 
 }  // namespace
@@ -331,6 +389,34 @@ int ensure_scratch(sipnet_gpu_handle *h) {
   if (e == cudaSuccess) e = cudaMalloc((void **)&h->rsLmax, S * sizeof(double));
   if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "resampling scratch: %s", cudaGetErrorString(e));
   return 0;
+}
+
+int snapshot_words(const sipnet_gpu_handle *h) { return record_words(h) + 1; }
+
+int ensure_mh_scratch(sipnet_gpu_handle *h) {
+  if (int rc = ensure_chunks(h)) return rc;
+  if (h->mhSnap) return 0;
+  const size_t ld = (size_t)h->ld, S = (size_t)h->nsites;
+  cudaError_t e = cudaMalloc((void **)&h->mhSnap, (size_t)snapshot_words(h) * ld * sizeof(double));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&h->mhValid, ld * sizeof(int8_t));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&h->mhDlp, ld * sizeof(double));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&h->mhCurL, ld * sizeof(double));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&h->mhLogU, ld * sizeof(double));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&h->mhScale, S * sizeof(double));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&h->mhTau, S * sizeof(double));
+  if (e != cudaSuccess) return fail(SIPNET_GPU_ERR_NO_DEVICE, "Metropolis-Hastings scratch: %s", cudaGetErrorString(e));
+  return 0;
+}
+
+cudaError_t launch_snapshot(const Args &a, cudaStream_t stream) {
+  const dim3 g(blocks_for(a.nmembers, 128), (unsigned)((a.words + 1 + kWordsPerY - 1) / kWordsPerY));
+  snapshot_kernel<<<g, 128, 0, stream>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_accept(const Args &a, cudaStream_t stream) {
+  accept_kernel<<<blocks_for(a.nchunks, 1), kChunk, 0, stream>>>(a);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_weights(const Args &a, int pass, cudaStream_t stream) {

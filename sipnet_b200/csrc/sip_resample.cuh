@@ -72,6 +72,15 @@ struct Args {
   double *const *src;      // [nranks]: where the segment from p is read (this rank's own: in sendBuf)
   double *sendBuf;
   int64_t nOut;            // outgoing records
+  // the Metropolis-Hastings move (sip_comm.cu run_mh): the snapshot of every member and the accept pass
+  double *snap;               // [snapshot_words][ld]: the record's words but the ancestor's, log-likelihood, count
+  const int8_t *valid;        // [ld] the proposal's verdict (kMh*, from sip_jitter.cu members(3))
+  const double *dlp;          // [ld] lp(phi') - lp(phi) of a valid proposal
+  const double *curLoglik;    // [ld] the caller's log-likelihood over the window
+  const double *logU;         // [ld]
+  const double *tau;          // [nsites]
+  double *count;              // [nchunks][countStride]: {invalid, accepted} per chunk (sip_jitter.cu's chunk records)
+  int32_t countStride;
 };
 
 // the handle's chunk tables, chunk records and member scratch
@@ -83,6 +92,15 @@ cudaError_t launch_site(const Args &a, int pass, cudaStream_t stream);
 cudaError_t launch_prefix(const Args &a, cudaStream_t stream);
 cudaError_t launch_pack(const Args &a, cudaStream_t stream);
 cudaError_t launch_unpack(const Args &a, cudaStream_t stream);
+
+// The Metropolis-Hastings move keeps a snapshot of every member in the resampler's record layout:
+//   snapshot     one thread per member and group of words: member m's record into column m of `snap`
+//   accept       one CTA per chunk, one thread per member: delta, the decision, a rejected member back from the
+//                snapshot; the chunk's invalid and accepted counts (integers: any order of summation, same value)
+int snapshot_words(const sipnet_gpu_handle *h);
+int ensure_mh_scratch(sipnet_gpu_handle *h);  // the snapshot and the move's member / site buffers
+cudaError_t launch_snapshot(const Args &a, cudaStream_t stream);
+cudaError_t launch_accept(const Args &a, cudaStream_t stream);
 
 }  // namespace rs
 }  // namespace sip

@@ -345,7 +345,8 @@ static void free_handle(sipnet_gpu_handle *h) {
                   h->stateBk, h->ringVBk, h->ringWBk, h->loglikBk, h->loglikNBk, h->statusBk,
                   h->recCountBk, h->sched, h->chunk, h->siteChunks, h->asPart, h->asMom, h->asCoef,
                   h->asObs, h->asDiag, h->asInfl, h->rsW, h->rsC, h->rsSite, h->rsPart, h->rsLogw, h->rsLmax, h->rsSend, h->rsRecv,
-                  h->rsAnc, h->rsTab, h->jtPart, h->jtMom, h->jtCoef, h->jtDiag, h->jtShrink, h->jtZ};
+                  h->rsAnc, h->rsTab, h->jtPart, h->jtMom, h->jtCoef, h->jtDiag, h->jtShrink, h->jtZ,
+                  h->mhSnap, h->mhDlp, h->mhCurL, h->mhLogU, h->mhScale, h->mhTau, h->mhValid};
   for (void *p : ptrs)
     if (p) cudaFree(p);
   for (void *p : h->siteAllocs)
