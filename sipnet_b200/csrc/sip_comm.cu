@@ -145,9 +145,7 @@ struct sipnet_gpu_comm {
   bool loopback = false;                 // every rank on one device: the collectives are device copies, not NCCL
   std::vector<Local> local;              // the ranks this process drives (1 with one process per GPU)
   std::vector<int64_t> memberCounts;     // [nranks]
-  float lastExchangeMs = 0.f, lastSummaryMs = 0.f;
   int lastLevels = 0;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
 
 namespace {
@@ -185,13 +183,22 @@ struct Group {
   }
 };
 
-// the local streams, all finished (the loopback collectives copy between the ranks' buffers on one device)
-int sync_all(sipnet_gpu_comm *c) {
-  for (Local &l : c->local) {
-    CUDA_OK(cudaSetDevice(l.h->device));
-    CUDA_OK(cudaStreamSynchronize(l.h->stream));
+// f(i, local rank i) on every local rank, with its device current; stops at the first non-zero return
+template <class F>
+int each_rank(sipnet_gpu_comm *c, F f) {
+  for (size_t i = 0; i < c->local.size(); ++i) {
+    CUDA_OK(cudaSetDevice(c->local[i].h->device));
+    if (int rc = f(i, c->local[i])) return rc;
   }
   return 0;
+}
+
+// the local streams, all finished (the loopback collectives copy between the ranks' buffers on one device)
+int sync_all(sipnet_gpu_comm *c) {
+  return each_rank(c, [](size_t, Local &l) {
+    CUDA_OK(cudaStreamSynchronize(l.h->stream));
+    return 0;
+  });
 }
 
 int all_gather_bytes(sipnet_gpu_comm *c, size_t bytesPerRank, void *(*buf)(Local &)) {
@@ -209,11 +216,13 @@ int all_gather_bytes(sipnet_gpu_comm *c, size_t bytesPerRank, void *(*buf)(Local
   }
   const Group g(c);
   if (int rc = g.begin()) return rc;
-  for (Local &l : c->local) {
-    CUDA_OK(cudaSetDevice(l.h->device));
-    char *base = static_cast<char *>(buf(l));
-    NCCL_OK(nccl_api()->AllGather(base + (size_t)l.rank * bytesPerRank, base, bytesPerRank, ncclUint8, l.comm, l.h->stream));
-  }
+  if (int rc = each_rank(c, [&](size_t, Local &l) {
+        char *base = static_cast<char *>(buf(l));
+        NCCL_OK(nccl_api()->AllGather(base + (size_t)l.rank * bytesPerRank, base, bytesPerRank, ncclUint8, l.comm,
+                                      l.h->stream));
+        return 0;
+      }))
+    return rc;
   return g.end();
 }
 
@@ -230,10 +239,11 @@ int all_reduce_hist(sipnet_gpu_comm *c, size_t words) {
   }
   const Group g(c);
   if (int rc = g.begin()) return rc;
-  for (Local &l : c->local) {
-    CUDA_OK(cudaSetDevice(l.h->device));
-    NCCL_OK(nccl_api()->AllReduce(l.hist, l.hist, words, ncclUint32, ncclSum, l.comm, l.h->stream));
-  }
+  if (int rc = each_rank(c, [&](size_t, Local &l) {
+        NCCL_OK(nccl_api()->AllReduce(l.hist, l.hist, words, ncclUint32, ncclSum, l.comm, l.h->stream));
+        return 0;
+      }))
+    return rc;
   return g.end();
 }
 
@@ -319,28 +329,26 @@ int team_summaries(sipnet_gpu_comm *c) {
   // quantiles in groups of kGsMaxQ; the moments ride with the first group
   for (int q0 = 0; q0 < std::max(nqTotal, 1); q0 += gs::kGsMaxQ) {
     const int nq = std::min(gs::kGsMaxQ, nqTotal - q0);
-    for (size_t i = 0; i < c->local.size(); ++i) {
-      Local &l = c->local[i];
-      gs::GsArgs &a = args[i];
-      a.nq = std::max(nq, 0);
-      for (int k = 0; k < a.nq; ++k) {
-        a.qOut[k] = order[(size_t)(q0 + k)];
-        a.probs[k] = l.h->quantiles[(size_t)a.qOut[k]];
-      }
-      a.wantMoments = (l.h->mean != nullptr && q0 == 0) ? 1 : 0;
-      CUDA_OK(cudaSetDevice(l.h->device));
-      if (int rc = launched(l.h, gs::launch_pass0(a, l.h->stream), "summary")) return rc;
-    }
+    if (int rc = each_rank(c, [&](size_t i, Local &l) {
+          gs::GsArgs &a = args[i];
+          a.nq = std::max(nq, 0);
+          for (int k = 0; k < a.nq; ++k) {
+            a.qOut[k] = order[(size_t)(q0 + k)];
+            a.probs[k] = l.h->quantiles[(size_t)a.qOut[k]];
+          }
+          a.wantMoments = (l.h->mean != nullptr && q0 == 0) ? 1 : 0;
+          return launched(l.h, gs::launch_pass0(a, l.h->stream), "summary");
+        }))
+      return rc;
     if (int rc = all_gather_bytes(c, (size_t)rows * sizeof(gs::GsStat), [](Local &l) -> void * { return l.statAll; })) return rc;
     if (args[0].nq > 0)
       if (int rc = all_reduce_hist(c, (size_t)rows * gs::kGsHistWords)) return rc;
     for (int level = 1; level <= gs::kGsLevels; ++level) {
-      for (size_t i = 0; i < c->local.size(); ++i) {
-        Local &l = c->local[i];
-        CUDA_OK(cudaSetDevice(l.h->device));
-        CUDA_OK(cudaMemsetAsync(l.flags, 0, 16, l.h->stream));
-        if (int rc = launched(l.h, gs::launch_level(args[i], level, l.h->stream), "summary")) return rc;
-      }
+      if (int rc = each_rank(c, [&](size_t i, Local &l) {
+            CUDA_OK(cudaMemsetAsync(l.flags, 0, 16, l.h->stream));
+            return launched(l.h, gs::launch_level(args[i], level, l.h->stream), "summary");
+          }))
+        return rc;
       // the flag is a function of exchanged data only: every rank reads the same value
       int32_t flag = 0;
       {
@@ -358,20 +366,18 @@ int team_summaries(sipnet_gpu_comm *c) {
         return rc;
     }
     if (args[0].nq > 0) {
-      for (size_t i = 0; i < c->local.size(); ++i) {
-        Local &l = c->local[i];
-        CUDA_OK(cudaSetDevice(l.h->device));
-        if (int rc = launched(l.h, gs::launch_emit(args[i], l.h->stream), "summary")) return rc;
-      }
+      if (int rc = each_rank(c, [&](size_t i, Local &l) {
+            return launched(l.h, gs::launch_emit(args[i], l.h->stream), "summary");
+          }))
+        return rc;
       if (int rc = all_gather_bytes(c, (size_t)rows * gs::kGsMaxStat * gs::kGsEmit * sizeof(uint64_t),
                                     [](Local &l) -> void * { return l.emitAll; }))
         return rc;
     }
-    for (size_t i = 0; i < c->local.size(); ++i) {
-      Local &l = c->local[i];
-      CUDA_OK(cudaSetDevice(l.h->device));
-      if (int rc = launched(l.h, gs::launch_finish(args[i], l.h->stream), "summary")) return rc;
-    }
+    if (int rc = each_rank(c, [&](size_t i, Local &l) {
+          return launched(l.h, gs::launch_finish(args[i], l.h->stream), "summary");
+        }))
+      return rc;
   }
   for (Local &l : c->local) l.h->summariesValid = true;
   return 0;
@@ -391,6 +397,25 @@ extern "C" int sipnet_gpu_comm_unique_id(void *id) {
   return 0;
 }
 
+// mine[i] of every local rank i, all-gathered through xchg: every rank's word, rank-major, on the host
+static int gather_words(sipnet_gpu_comm *c, const std::vector<uint64_t> &mine, std::vector<uint64_t> &all) {
+  if (int rc = each_rank(c, [&](size_t i, Local &l) {
+        if (int rc = grow(l.xchg, l.xchgCap, (size_t)c->nranks * sizeof(uint64_t), l.h->stream)) return rc;
+        CUDA_OK(cudaMemcpyAsync(l.xchg + l.rank * sizeof(uint64_t), &mine[i], sizeof(uint64_t), cudaMemcpyHostToDevice,
+                                l.h->stream));
+        CUDA_OK(cudaStreamSynchronize(l.h->stream));
+        return 0;
+      }))
+    return rc;
+  if (int rc = all_gather_bytes(c, sizeof(uint64_t), [](Local &l) -> void * { return l.xchg; })) return rc;
+  all.resize((size_t)c->nranks);
+  Local &l0 = c->local[0];
+  CUDA_OK(cudaSetDevice(l0.h->device));
+  CUDA_OK(cudaMemcpyAsync(all.data(), l0.xchg, all.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, l0.h->stream));
+  CUDA_OK(cudaStreamSynchronize(l0.h->stream));
+  return 0;
+}
+
 static int finish_comm(sipnet_gpu_comm *c) {
   // member counts of all ranks (for the log-likelihood gather's layout); no exchange when this process drives them all
   c->memberCounts.assign((size_t)c->nranks, 0);
@@ -398,31 +423,10 @@ static int finish_comm(sipnet_gpu_comm *c) {
     for (const Local &l : c->local) c->memberCounts[(size_t)l.rank] = l.h->nmembers;
     return 0;
   }
-  std::vector<int64_t *> dev(c->local.size(), nullptr);
-  const Group g(c);
-  for (size_t i = 0; i < c->local.size(); ++i) {
-    Local &l = c->local[i];
-    CUDA_OK(cudaSetDevice(l.h->device));
-    CUDA_OK(cudaMalloc((void **)&dev[i], (size_t)c->nranks * sizeof(int64_t)));
-    const int64_t mine = l.h->nmembers;
-    CUDA_OK(cudaMemcpyAsync(dev[i] + l.rank, &mine, sizeof mine, cudaMemcpyHostToDevice, l.h->stream));
-    CUDA_OK(cudaStreamSynchronize(l.h->stream));
-  }
-  if (int rc = g.begin()) return rc;
-  for (size_t i = 0; i < c->local.size(); ++i) {
-    Local &l = c->local[i];
-    CUDA_OK(cudaSetDevice(l.h->device));
-    NCCL_OK(nccl_api()->AllGather(dev[i] + l.rank, dev[i], sizeof(int64_t), ncclUint8, l.comm, l.h->stream));
-  }
-  if (int rc = g.end()) return rc;
-  for (size_t i = 0; i < c->local.size(); ++i) {
-    Local &l = c->local[i];
-    CUDA_OK(cudaSetDevice(l.h->device));
-    CUDA_OK(cudaMemcpyAsync(c->memberCounts.data(), dev[i], (size_t)c->nranks * sizeof(int64_t), cudaMemcpyDeviceToHost,
-                            l.h->stream));
-    CUDA_OK(cudaStreamSynchronize(l.h->stream));
-    cudaFree(dev[i]);
-  }
+  std::vector<uint64_t> mine, all;
+  for (const Local &l : c->local) mine.push_back((uint64_t)l.h->nmembers);
+  if (int rc = gather_words(c, mine, all)) return rc;
+  for (int q = 0; q < c->nranks; ++q) c->memberCounts[(size_t)q] = (int64_t)all[(size_t)q];
   return 0;
 }
 
@@ -473,8 +477,6 @@ extern "C" void sipnet_gpu_comm_destroy(sipnet_gpu_comm *c) {
     free_local(l);
     if (l.comm) nccl_api()->CommDestroy(l.comm);
   }
-  if (c->ev0) cudaEventDestroy(c->ev0);
-  if (c->ev1) cudaEventDestroy(c->ev1);
   delete c;
 }
 
@@ -499,15 +501,16 @@ static int team_member_words(sipnet_gpu_comm *c, void *dst, size_t bytes, const 
   if (dst && bytes != (size_t)total * sizeof(double))
     return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "%s gather: buffer is %zu bytes, expected %zu", what, bytes,
                 (size_t)total * sizeof(double));
-  for (Local &l : c->local) {
-    sipnet_gpu_handle *h = l.h;
-    const void *from = src(h);
-    if (!from) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "%s output was not requested at init", what);
-    CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = grow(l.xchg, l.xchgCap, (size_t)c->nranks * width * sizeof(double), h->stream)) return rc;
-    CUDA_OK(cudaMemcpyAsync(l.xchg + (size_t)l.rank * width * sizeof(double), from, (size_t)h->nmembers * sizeof(double),
-                            cudaMemcpyDeviceToDevice, h->stream));
-  }
+  if (int rc = each_rank(c, [&](size_t, Local &l) {
+        sipnet_gpu_handle *h = l.h;
+        const void *from = src(h);
+        if (!from) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "%s output was not requested at init", what);
+        if (int rc = grow(l.xchg, l.xchgCap, (size_t)c->nranks * width * sizeof(double), h->stream)) return rc;
+        CUDA_OK(cudaMemcpyAsync(l.xchg + (size_t)l.rank * width * sizeof(double), from, (size_t)h->nmembers * sizeof(double),
+                                cudaMemcpyDeviceToDevice, h->stream));
+        return 0;
+      }))
+    return rc;
   if (int rc = all_gather_bytes(c, (size_t)width * sizeof(double), [](Local &l) -> void * { return l.xchg; })) return rc;
   if (dst) {
     Local &l = c->local[0];
@@ -521,11 +524,7 @@ static int team_member_words(sipnet_gpu_comm *c, void *dst, size_t bytes, const 
     CUDA_OK(cudaStreamSynchronize(l.h->stream));
   }
   // every local stream has finished its part before the caller reuses the handles
-  for (Local &l : c->local) {
-    CUDA_OK(cudaSetDevice(l.h->device));
-    CUDA_OK(cudaStreamSynchronize(l.h->stream));
-  }
-  return 0;
+  return sync_all(c);
 }
 
 extern "C" int sipnet_gpu_comm_gather_loglik(sipnet_gpu_comm *c, double *dst, size_t bytes) {
@@ -877,6 +876,69 @@ extern "C" int sipnet_gpu_multi_gather(sipnet_gpu_multi *m, int what, void *dst,
   return 0;
 }
 
+// ---- the ensemble filters: one run over a team, from a handle, a comm or a multi-GPU handle -----------------------
+namespace {
+
+// One site pass on every local rank: launch(i, l) queues the members and site launches; a team then all-gathers the
+// [nsites][rec] per-site partials (doubles) in xchg, and combine(i, l) sums them in rank order on every rank.  A team
+// of one makes no exchange and no host round trip.
+template <class Launch, class Combine>
+int site_pass(sipnet_gpu_comm *c, size_t rec, Launch launch, Combine combine) {
+  if (int rc = each_rank(c, launch)) return rc;
+  if (c->nranks == 1) return 0;
+  const size_t bytes = (size_t)c->local[0].h->nsites * rec * sizeof(double);
+  if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.xchg; })) return rc;
+  return each_rank(c, combine);
+}
+
+// A filter through the multi-GPU interface: split sites, run(m->comm, 0) over every device; whole sites, run(its team
+// of one, d) for each device d.  Device d's per-site arrays start at site m->parts[d].site0 (0 when sites are split).
+template <class F>
+int multi_run(sipnet_gpu_multi *m, F run) {
+  if (m->split) return run(m->comm, 0);
+  for (size_t d = 0; d < m->handles.size(); ++d) {
+    sipnet_gpu_comm one = team_of_one(m->handles[d]);
+    if (int rc = run(&one, d)) return rc;
+  }
+  return 0;
+}
+
+// sites [site0, ...) of an array of `per` elements per site; NULL stays NULL
+template <class T>
+T *from_site(T *p, int64_t site0, size_t per) {
+  return p ? p + (size_t)site0 * per : nullptr;
+}
+
+// a configuration-order array [rows][M] as every device's [rows][its members] copy; at[d] is device d's
+struct Copies {
+  std::vector<std::vector<double>> v;
+  std::vector<const double *> at;
+};
+
+Copies device_copies(const sipnet_gpu_multi *m, const double *a, size_t rows) {
+  Copies c;
+  const size_t M = (size_t)m->nmembers;
+  for (size_t d = 0; d < m->handles.size(); ++d) {
+    const size_t nm = (size_t)m->handles[d]->nmembers;
+    c.v.emplace_back(rows * nm);
+    for (size_t j = 0; j < rows; ++j)
+      for (const sipnet_gpu_multi::Run &r : m->parts[d].runs)
+        memcpy(c.v[d].data() + j * nm + r.local0, a + j * M + r.global0, (size_t)r.count * sizeof(double));
+  }
+  for (const std::vector<double> &v : c.v) c.at.push_back(v.data());
+  return c;
+}
+
+// the configuration index of each of device d's members
+std::vector<int64_t> config_index(const sipnet_gpu_multi *m, size_t d) {
+  std::vector<int64_t> g((size_t)m->handles[d]->nmembers);
+  for (const sipnet_gpu_multi::Run &r : m->parts[d].runs)
+    std::iota(g.begin() + r.local0, g.begin() + r.local0 + r.count, r.global0);
+  return g;
+}
+
+}  // namespace
+
 // ---- sequential data assimilation: the ensemble adjustment Kalman filter (sip_assim.cuh) --------------------------
 namespace {
 
@@ -963,7 +1025,7 @@ int check_inflation(const sipnet_gpu_inflation_spec *f, int64_t nsites) {
 sipnet_gpu_inflation_spec inflation_slice(const sipnet_gpu_inflation_spec *f, int64_t site0) {
   sipnet_gpu_inflation_spec g = *f;
   g.lambda += site0;
-  if (g.lambda_sd) g.lambda_sd += site0;
+  g.lambda_sd = from_site(g.lambda_sd, site0, 1);
   return g;
 }
 
@@ -1031,23 +1093,16 @@ int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const dou
     }
   }
   // one members pass and its site reduction on every rank; a team then exchanges and combines the site partials
-  auto run_pass = [&](int pass, bool apply, bool inflatePass) -> int {
-    for (size_t i = 0; i < c->local.size(); ++i) {
-      sipnet_gpu_handle *h = c->local[i].h;
-      CUDA_OK(cudaSetDevice(h->device));
-      if (int rc = launched(h, as::launch_members(args[i], pass, apply, false, inflatePass, h->stream), "assimilation"))
-        return rc;
-      if (int rc = launched(h, as::launch_site_reduce(args[i], pass, h->stream), "assimilation")) return rc;
-    }
-    if (R == 1) return 0;
-    const size_t bytes = (size_t)S * as::kRec * sizeof(double);
-    if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.xchg; })) return rc;
-    for (size_t i = 0; i < c->local.size(); ++i) {
-      sipnet_gpu_handle *h = c->local[i].h;
-      CUDA_OK(cudaSetDevice(h->device));
-      if (int rc = launched(h, as::launch_site_combine(args[i], pass, h->stream), "assimilation")) return rc;
-    }
-    return 0;
+  auto run_pass = [&](int pass, bool apply, bool inflatePass) {
+    const char *what = "assimilation";
+    return site_pass(
+        c, as::kRec,
+        [&](size_t i, Local &l) {
+          if (int rc = launched(l.h, as::launch_members(args[i], pass, apply, false, inflatePass, l.h->stream), what))
+            return rc;
+          return launched(l.h, as::launch_site_reduce(args[i], pass, l.h->stream), what);
+        },
+        [&](size_t i, Local &l) { return launched(l.h, as::launch_site_combine(args[i], pass, l.h->stream), what); });
   };
   if (inflate)  // the means the inflation centres on
     if (int rc = run_pass(as::kInflPass, false, false)) return rc;
@@ -1063,14 +1118,11 @@ int run_assimilation(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *o, const dou
     if (int rc = run_pass(1, k > 0, k == 0 && inflate)) return rc;
     if (int rc = run_pass(2, false, false)) return rc;
   }
-  for (size_t i = 0; i < c->local.size(); ++i) {  // the last observation's update and the floor
+  return each_rank(c, [&](size_t i, Local &l) {  // the last observation's update and the floor
     as::Args &a = args[i];
-    sipnet_gpu_handle *h = c->local[i].h;
     for (int j = 0; j < nr; ++j) a.opPrev[j] = o->op[(size_t)(nobs - 1) * nr + j];
-    CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = launched(h, as::launch_members(a, 0, true, true, false, h->stream), "assimilation")) return rc;
-  }
-  return 0;
+    return launched(l.h, as::launch_members(a, 0, true, true, false, l.h->stream), "assimilation");
+  });
 }
 
 // wait for the analysis of `h`; diag (may be NULL) gets its [nsites][nobs][4] diagnostics, infl (may be NULL) the
@@ -1119,18 +1171,8 @@ extern "C" int sipnet_gpu_assimilate_inflated(sipnet_gpu_handle *h, const sipnet
 static int team_agree(sipnet_gpu_comm *c, int bad, uint64_t mine, const char *what) {
   if (c->nranks == 1) return bad;
   const std::string why = bad ? sipnet_gpu_last_error() : "";
-  for (Local &l : c->local) {
-    CUDA_OK(cudaSetDevice(l.h->device));
-    if (int rc = grow(l.xchg, l.xchgCap, (size_t)c->nranks * sizeof mine, l.h->stream)) return rc;
-    CUDA_OK(cudaMemcpyAsync(l.xchg + l.rank * sizeof mine, &mine, sizeof mine, cudaMemcpyHostToDevice, l.h->stream));
-    CUDA_OK(cudaStreamSynchronize(l.h->stream));
-  }
-  if (int rc = all_gather_bytes(c, sizeof mine, [](Local &l) -> void * { return l.xchg; })) return rc;
-  std::vector<uint64_t> all((size_t)c->nranks);
-  Local &l0 = c->local[0];
-  CUDA_OK(cudaSetDevice(l0.h->device));
-  CUDA_OK(cudaMemcpyAsync(all.data(), l0.xchg, all.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, l0.h->stream));
-  CUDA_OK(cudaStreamSynchronize(l0.h->stream));
+  std::vector<uint64_t> all;
+  if (int rc = gather_words(c, std::vector<uint64_t>(c->local.size(), mine), all)) return rc;
   for (uint64_t v : all)
     if (v == 0 || v != all[0]) {
       if (bad) return fail(bad, "%s", why.c_str());
@@ -1161,9 +1203,7 @@ int assimilate_comm(sipnet_gpu_comm *c, const sipnet_gpu_obs_spec *obs, sipnet_g
   if (!bad && infl) bad = check_inflation(infl, S);
   if (int rc = team_agree(c, bad, bad ? 0 : assim_hash(obs, infl, S), "observation specs")) return rc;
   if (int rc = run_assimilation(c, obs, obs->value, obs->variance, infl)) return rc;
-  for (Local &l : c->local)
-    if (int rc = finish_assimilation(l.h, diag, obs->n_obs, infl)) return rc;
-  return 0;
+  return finish_assimilation(c->local[0].h, diag, obs->n_obs, infl);
 }
 
 int assimilate_multi(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, sipnet_gpu_inflation_spec *infl,
@@ -1173,25 +1213,20 @@ int assimilate_multi(sipnet_gpu_multi *m, const sipnet_gpu_obs_spec *obs, sipnet
   if (infl)
     if (int rc = check_inflation(infl, m->nsites)) return rc;
   const int nobs = obs->n_obs;
-  if (m->split) {  // every device ends with the same diagnostics and inflation: take device 0's
-    if (int rc = run_assimilation(m->comm, obs, obs->value, obs->variance, infl)) return rc;
-    for (size_t d = 0; d < m->handles.size(); ++d)
-      if (int rc = finish_assimilation(m->handles[d], d == 0 ? diag : nullptr, nobs, d == 0 ? infl : nullptr)) return rc;
-    return 0;
-  }
-  // whole sites: each device alone on its site range, all devices side by side
   std::vector<sipnet_gpu_inflation_spec> slice(m->handles.size());
+  if (int rc = multi_run(m, [&](sipnet_gpu_comm *c, size_t d) {  // whole sites: all devices side by side
+        const int64_t s0 = m->parts[d].site0;
+        if (infl) slice[d] = inflation_slice(infl, s0);
+        return run_assimilation(c, obs, obs->value + s0 * nobs, obs->variance + s0 * nobs, infl ? &slice[d] : nullptr);
+      }))
+    return rc;
+  // split sites: every device ends with the same diagnostics and inflation, take device 0's
   for (size_t d = 0; d < m->handles.size(); ++d) {
-    const size_t off = (size_t)m->parts[d].site0 * nobs;
-    if (infl) slice[d] = inflation_slice(infl, m->parts[d].site0);
-    sipnet_gpu_comm one = team_of_one(m->handles[d]);
-    if (int rc = run_assimilation(&one, obs, obs->value + off, obs->variance + off, infl ? &slice[d] : nullptr))
+    const bool out = d == 0 || !m->split;
+    if (int rc = finish_assimilation(m->handles[d], out ? from_site(diag, m->parts[d].site0, (size_t)nobs * 4) : nullptr,
+                                     nobs, out && infl ? &slice[d] : nullptr))
       return rc;
   }
-  for (size_t d = 0; d < m->handles.size(); ++d)
-    if (int rc = finish_assimilation(m->handles[d], diag ? diag + (size_t)m->parts[d].site0 * nobs * 4 : nullptr, nobs,
-                                     infl ? &slice[d] : nullptr))
-      return rc;
   return 0;
 }
 
@@ -1271,10 +1306,36 @@ struct CopyPlan {
   std::vector<int64_t> sendCnt, sendBase, recvCnt, recvBase;
 };
 
+// the resampler's arguments for the members of `h` and their records (the rest zero)
+void member_args(const sipnet_gpu_handle *h, rs::Args &a) {
+  memset(&a, 0, sizeof a);
+  a.status = h->status;
+  a.sites = h->sites;
+  a.memberSite = h->memberSite;
+  a.nmembers = h->nmembers;
+  a.ld = h->ld;
+  a.nsites = (int32_t)h->nsites;
+  a.nchunks = (int32_t)h->nchunks;
+  a.chunk = h->chunk;
+  a.siteChunks = h->siteChunks;
+  a.params = h->params;
+  a.state = h->state;
+  a.ringV = h->ringV;
+  a.ringW = h->ringW;
+  a.loglik = h->loglik;
+  a.loglikN = h->loglikN;
+  a.counters = h->counters;
+  a.recs = h->recs;
+  a.recCount = h->recCount;
+  a.ringCap = h->ringCap;
+  a.maxRecs = h->maxRecs;
+  a.words = rs::record_words(h);
+}
+
 // Resample every local rank of `c` (all ranks hold the same sites): logw[i] is local rank i's host log-weights or
 // NULL (its log-likelihood).  diag (may be NULL) gets [nsites][4]; ancAll the team's ancestors, rank-major.
-int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const std::vector<const double *> &logw,
-                 double *diag, std::vector<int64_t> &ancAll) {
+int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const double *const *logw, double *diag,
+                 std::vector<int64_t> &ancAll) {
   const int R = c->nranks;
   const int64_t S = c->local[0].h->nsites;
   const int words = rs::record_words(c->local[0].h);
@@ -1293,29 +1354,8 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
     if (logw[i])
       CUDA_OK(cudaMemcpyAsync(h->rsLogw, logw[i], (size_t)h->nmembers * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     rs::Args &a = args[i];
-    memset(&a, 0, sizeof a);
+    member_args(h, a);
     a.logw = logw[i] ? h->rsLogw : h->loglik;
-    a.status = h->status;
-    a.sites = h->sites;
-    a.memberSite = h->memberSite;
-    a.nmembers = h->nmembers;
-    a.ld = h->ld;
-    a.nsites = (int32_t)S;
-    a.nchunks = (int32_t)h->nchunks;
-    a.chunk = h->chunk;
-    a.siteChunks = h->siteChunks;
-    a.params = h->params;
-    a.state = h->state;
-    a.ringV = h->ringV;
-    a.ringW = h->ringW;
-    a.loglik = h->loglik;
-    a.loglikN = h->loglikN;
-    a.counters = h->counters;
-    a.recs = h->recs;
-    a.recCount = h->recCount;
-    a.ringCap = h->ringCap;
-    a.maxRecs = h->maxRecs;
-    a.words = words;
     a.nranks = R;
     a.rank = l.rank;
     a.idBase = rankBase[(size_t)l.rank];
@@ -1347,13 +1387,13 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
     if (n[(size_t)s] > rs::kMaxSiteMembers)
       return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "site %lld has %lld members; resampling takes at most 2^23 per site",
                   (long long)s, (long long)n[(size_t)s]);
-  for (size_t i = 0; i < L; ++i) {
-    sipnet_gpu_handle *h = c->local[i].h;
-    CUDA_OK(cudaSetDevice(h->device));
-    CUDA_OK(cudaMemcpyAsync(h->rsLmax, lmax.data(), (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    if (int rc = launched(h, rs::launch_weights(args[i], 1, h->stream), "resampling")) return rc;
-    if (int rc = launched(h, rs::launch_site(args[i], 1, h->stream), "resampling")) return rc;
-  }
+  if (int rc = each_rank(c, [&](size_t i, Local &l) {
+        sipnet_gpu_handle *h = l.h;
+        CUDA_OK(cudaMemcpyAsync(h->rsLmax, lmax.data(), (size_t)S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        if (int rc = launched(h, rs::launch_weights(args[i], 1, h->stream), "resampling")) return rc;
+        return launched(h, rs::launch_site(args[i], 1, h->stream), "resampling");
+      }))
+    return rc;
   // pass b over the ranks: ESS, the decision and the slot ranges of every site (integer sums: any order, same bits)
   if (int rc = site_records(c, recB)) return rc;
   const size_t R1 = (size_t)R + 1;
@@ -1483,11 +1523,10 @@ int run_resample(sipnet_gpu_comm *c, const double *u, double essFraction, const 
     }
     NCCL_OK(nccl_api()->GroupEnd());
   }
-  for (size_t i = 0; i < L; ++i) {
-    sipnet_gpu_handle *h = c->local[i].h;
-    CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = launched(h, rs::launch_unpack(args[i], h->stream), "resampling")) return rc;
-  }
+  if (int rc = each_rank(c, [&](size_t i, Local &l) {
+        return launched(l.h, rs::launch_unpack(args[i], l.h->stream), "resampling");
+      }))
+    return rc;
   // the ancestors of the whole team, and the distinct ancestors of every resampled site
   ancAll.assign((size_t)rankBase[(size_t)R], -1);
   if (R == 1) {
@@ -1522,7 +1561,7 @@ extern "C" int sipnet_gpu_resample(sipnet_gpu_handle *h, const double *u, double
   if (int rc = check_resample(h, u, h->nsites, ess_fraction, log_weights)) return rc;
   sipnet_gpu_comm one = team_of_one(h);
   std::vector<int64_t> anc;
-  if (int rc = run_resample(&one, u, ess_fraction, {log_weights}, diag, anc)) return rc;
+  if (int rc = run_resample(&one, u, ess_fraction, &log_weights, diag, anc)) return rc;
   if (ancestors) memcpy(ancestors, anc.data(), anc.size() * sizeof(int64_t));
   return 0;
 }
@@ -1535,8 +1574,7 @@ extern "C" int sipnet_gpu_comm_resample(sipnet_gpu_comm *c, const double *u, dou
   const int bad = check_resample(h, u, S, ess_fraction, log_weights);
   if (int rc = team_agree(c, bad, bad ? 0 : resample_hash(h, u, ess_fraction), "resampling arguments")) return rc;
   std::vector<int64_t> anc;
-  if (int rc = run_resample(c, u, ess_fraction, std::vector<const double *>(c->local.size(), log_weights), diag, anc))
-    return rc;
+  if (int rc = run_resample(c, u, ess_fraction, &log_weights, diag, anc)) return rc;
   if (ancestors) memcpy(ancestors, anc.data(), anc.size() * sizeof(int64_t));
   return 0;
 }
@@ -1546,13 +1584,6 @@ extern "C" int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, d
   if (!m) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
   if (int rc = check_resample(m->handles[0], u, m->nsites, ess_fraction, log_weights)) return rc;
   const size_t D = m->handles.size();
-  // configuration index of every device's members
-  std::vector<std::vector<int64_t>> glob(D);
-  for (size_t d = 0; d < D; ++d) {
-    glob[d].resize((size_t)m->handles[d]->nmembers);
-    for (const sipnet_gpu_multi::Run &r : m->parts[d].runs)
-      std::iota(glob[d].begin() + r.local0, glob[d].begin() + r.local0 + r.count, r.global0);
-  }
   // the log-weights per device, checked here: a device must not resample before another one rejects the call
   std::vector<double> all;
   if (!log_weights) {
@@ -1570,41 +1601,29 @@ extern "C" int sipnet_gpu_multi_resample(sipnet_gpu_multi *m, const double *u, d
     if (siteN[(size_t)s] > rs::kMaxSiteMembers)
       return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "site %lld has %lld members; resampling takes at most 2^23 per site",
                   (long long)s, (long long)siteN[(size_t)s]);
-  std::vector<std::vector<double>> lw(D);
-  for (size_t d = 0; d < D; ++d) {
-    lw[d].resize(glob[d].size());
-    for (size_t j = 0; j < glob[d].size(); ++j) lw[d][j] = log_weights[glob[d][j]];
-  }
-  std::vector<int64_t> anc;
-  if (m->split) {
-    std::vector<const double *> ptrs;
-    for (size_t d = 0; d < D; ++d) ptrs.push_back(lw[d].data());
-    if (int rc = run_resample(m->comm, u, ess_fraction, ptrs, diag, anc)) return rc;
+  const Copies lw = device_copies(m, log_weights, 1);
+  std::vector<std::vector<int64_t>> glob;
+  for (size_t d = 0; d < D; ++d) glob.push_back(config_index(m, d));
+  return multi_run(m, [&](sipnet_gpu_comm *c, size_t d) {
+    const int64_t s0 = m->parts[d].site0;
+    std::vector<int64_t> anc;
+    if (int rc = run_resample(c, u + s0, ess_fraction, lw.at.data() + d, from_site(diag, s0, 4), anc)) return rc;
     if (ancestors) {  // rank-major -> configuration order
-      std::vector<int64_t> base(D + 1, 0);
-      for (size_t d = 0; d < D; ++d) base[d + 1] = base[d] + m->handles[d]->nmembers;
-      for (size_t d = 0; d < D; ++d)
-        for (size_t j = 0; j < glob[d].size(); ++j) {
-          const int64_t v = anc[(size_t)base[d] + j];
+      std::vector<int64_t> base(1, 0);
+      for (int64_t n : c->memberCounts) base.push_back(base.back() + n);
+      for (size_t i = 0; i < c->local.size(); ++i)
+        for (size_t j = 0; j < glob[d + i].size(); ++j) {
+          const int64_t v = anc[(size_t)base[i] + j];
           int64_t g = -1;
           if (v >= 0) {
             const size_t q = (size_t)(std::upper_bound(base.begin(), base.end(), v) - base.begin()) - 1;
-            g = glob[q][(size_t)(v - base[q])];
+            g = glob[d + q][(size_t)(v - base[q])];
           }
-          ancestors[glob[d][j]] = g;
+          ancestors[glob[d + i][j]] = g;
         }
     }
     return 0;
-  }
-  // whole sites: each device alone on its site range
-  for (size_t d = 0; d < D; ++d) {
-    sipnet_gpu_comm one = team_of_one(m->handles[d]);
-    const size_t s0 = (size_t)m->parts[d].site0;
-    if (int rc = run_resample(&one, u + s0, ess_fraction, {lw[d].data()}, diag ? diag + s0 * 4 : nullptr, anc)) return rc;
-    if (ancestors)
-      for (size_t j = 0; j < glob[d].size(); ++j) ancestors[glob[d][j]] = anc[j] < 0 ? -1 : glob[d][(size_t)anc[j]];
-  }
-  return 0;
+  });
 }
 
 // ---- parameter rejuvenation: the Liu-West move (sip_jitter.cuh) ---------------------------------------------------
@@ -1707,23 +1726,14 @@ int jitter_args(sipnet_gpu_comm *c, Local &l, int32_t n, const int32_t *rows, co
 // One pass of the move on every local rank: members(pass) (unless the chunk records are already written), site(pass),
 // and for a team the exchange of the per-site partials and combine(pass).
 int jitter_pass(sipnet_gpu_comm *c, std::vector<jt::Args> &args, int pass, bool members, const char *what) {
-  for (size_t i = 0; i < c->local.size(); ++i) {
-    sipnet_gpu_handle *h = c->local[i].h;
-    CUDA_OK(cudaSetDevice(h->device));
-    if (members)
-      if (int rc = launched(h, jt::launch_members(args[i], pass, h->stream), what)) return rc;
-    if (int rc = launched(h, jt::launch_site(args[i], pass, h->stream), what)) return rc;
-  }
-  if (c->nranks > 1) {
-    const size_t bytes = (size_t)c->local[0].h->nsites * jt::kRec * sizeof(double);
-    if (int rc = all_gather_bytes(c, bytes, [](Local &l) -> void * { return l.xchg; })) return rc;
-    for (size_t i = 0; i < c->local.size(); ++i) {
-      sipnet_gpu_handle *h = c->local[i].h;
-      CUDA_OK(cudaSetDevice(h->device));
-      if (int rc = launched(h, jt::launch_combine(args[i], pass, h->stream), what)) return rc;
-    }
-  }
-  return 0;
+  return site_pass(
+      c, jt::kRec,
+      [&](size_t i, Local &l) {
+        if (members)
+          if (int rc = launched(l.h, jt::launch_members(args[i], pass, l.h->stream), what)) return rc;
+        return launched(l.h, jt::launch_site(args[i], pass, l.h->stream), what);
+      },
+      [&](size_t i, Local &l) { return launched(l.h, jt::launch_combine(args[i], pass, l.h->stream), what); });
 }
 
 // local rank 0's diagnostics into diag (may be NULL), and every local stream finished
@@ -1740,8 +1750,8 @@ int jitter_diag(sipnet_gpu_comm *c, double *diag) {
 // members.  A team of one needs no exchange and no host round trip; a larger team all-gathers the per-site partial
 // sums of the two moment passes and of the counts, and sums them in rank order on every rank.  diag (may be NULL)
 // gets local rank 0's [nsites][4].
-int run_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *sp, const double *shrink,
-                   const std::vector<const double *> &z, double *diag) {
+int run_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *sp, const double *shrink, const double *const *z,
+                   double *diag) {
   const int n = sp->n_rows;
   std::vector<jt::Args> args(c->local.size());
   for (size_t i = 0; i < c->local.size(); ++i) {
@@ -1762,7 +1772,7 @@ extern "C" int sipnet_gpu_rejuvenate(sipnet_gpu_handle *h, const sipnet_gpu_jitt
   if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
   if (int rc = check_jitter(spec, h->nsites, h->nmembers)) return rc;
   sipnet_gpu_comm one = team_of_one(h);
-  return run_rejuvenate(&one, spec, spec->shrink, {spec->z}, diag);
+  return run_rejuvenate(&one, spec, spec->shrink, &spec->z, diag);
 }
 
 extern "C" int sipnet_gpu_comm_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_jitter_spec *spec, double *diag) {
@@ -1771,34 +1781,17 @@ extern "C" int sipnet_gpu_comm_rejuvenate(sipnet_gpu_comm *c, const sipnet_gpu_j
   const int64_t S = h->nsites;
   const int bad = check_jitter(spec, S, h->nmembers);
   if (int rc = team_agree(c, bad, bad ? 0 : jitter_hash(spec, S), "rejuvenation specs")) return rc;
-  return run_rejuvenate(c, spec, spec->shrink, std::vector<const double *>(c->local.size(), spec->z), diag);
+  return run_rejuvenate(c, spec, spec->shrink, &spec->z, diag);
 }
 
 extern "C" int sipnet_gpu_multi_rejuvenate(sipnet_gpu_multi *m, const sipnet_gpu_jitter_spec *spec, double *diag) {
   if (!m) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
   if (int rc = check_jitter(spec, m->nsites, m->nmembers)) return rc;
-  const size_t D = m->handles.size(), n = (size_t)spec->n_rows, M = (size_t)m->nmembers;
-  // every device's normals, [n_rows][its members], from the configuration-order z
-  std::vector<std::vector<double>> zd(D);
-  for (size_t d = 0; d < D; ++d) {
-    const size_t nm = (size_t)m->handles[d]->nmembers;
-    zd[d].resize(n * nm);
-    for (size_t j = 0; j < n; ++j)
-      for (const sipnet_gpu_multi::Run &r : m->parts[d].runs)
-        memcpy(zd[d].data() + j * nm + r.local0, spec->z + j * M + r.global0, (size_t)r.count * sizeof(double));
-  }
-  if (m->split) {  // every device ends with the same diagnostics: take device 0's
-    std::vector<const double *> ptrs;
-    for (size_t d = 0; d < D; ++d) ptrs.push_back(zd[d].data());
-    return run_rejuvenate(m->comm, spec, spec->shrink, ptrs, diag);
-  }
-  // whole sites: each device alone on its site range
-  for (size_t d = 0; d < D; ++d) {
-    sipnet_gpu_comm one = team_of_one(m->handles[d]);
-    const size_t s0 = (size_t)m->parts[d].site0;
-    if (int rc = run_rejuvenate(&one, spec, spec->shrink + s0, {zd[d].data()}, diag ? diag + s0 * 4 : nullptr)) return rc;
-  }
-  return 0;
+  const Copies z = device_copies(m, spec->z, (size_t)spec->n_rows);
+  return multi_run(m, [&](sipnet_gpu_comm *c, size_t d) {
+    const int64_t s0 = m->parts[d].site0;
+    return run_rejuvenate(c, spec, spec->shrink + s0, z.at.data() + d, from_site(diag, s0, 4));
+  });
 }
 
 // ---- parameter calibration: the Metropolis-Hastings move (sip_jitter.cuh proposes, sip_resample.cuh decides) ------
@@ -1869,8 +1862,7 @@ int rerun_window(sipnet_gpu_handle *h, int64_t s) {
 // snapshot, the proposal, reset and run of every local handle over its window (no exchange), the accept pass, and the
 // site pass of the counts (a team exchanges them).  diag (may be NULL) gets local rank 0's [nsites][4].
 int run_mh(sipnet_gpu_comm *c, const sipnet_gpu_mh_spec *sp, const double *scale, const double *tau,
-           const std::vector<const double *> &curL, const std::vector<const double *> &z,
-           const std::vector<const double *> &logU, double *diag) {
+           const double *const *curL, const double *const *z, const double *const *logU, double *diag) {
   const int n = sp->n_rows;
   const int64_t S = c->local[0].h->nsites;
   const size_t L = c->local.size();
@@ -1908,26 +1900,7 @@ int run_mh(sipnet_gpu_comm *c, const sipnet_gpu_mh_spec *sp, const double *scale
     a.valid = h->mhValid;
     a.dlp = h->mhDlp;
     rs::Args &r = acc[i];
-    memset(&r, 0, sizeof r);
-    r.status = h->status;
-    r.sites = h->sites;
-    r.nmembers = h->nmembers;
-    r.ld = h->ld;
-    r.nsites = (int32_t)S;
-    r.nchunks = (int32_t)h->nchunks;
-    r.chunk = h->chunk;
-    r.params = h->params;
-    r.state = h->state;
-    r.ringV = h->ringV;
-    r.ringW = h->ringW;
-    r.loglik = h->loglik;
-    r.loglikN = h->loglikN;
-    r.counters = h->counters;
-    r.recs = h->recs;
-    r.recCount = h->recCount;
-    r.ringCap = h->ringCap;
-    r.maxRecs = h->maxRecs;
-    r.words = rs::record_words(h);
+    member_args(h, r);
     r.snap = h->mhSnap;
     r.valid = h->mhValid;
     r.dlp = h->mhDlp;
@@ -1940,21 +1913,21 @@ int run_mh(sipnet_gpu_comm *c, const sipnet_gpu_mh_spec *sp, const double *scale
   }
   for (int pass = 1; pass <= 2; ++pass)
     if (int rc = jitter_pass(c, args, pass, true, "Metropolis-Hastings")) return rc;
-  for (size_t i = 0; i < L; ++i) {
-    sipnet_gpu_handle *h = c->local[i].h;
-    CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = launched(h, rs::launch_snapshot(acc[i], h->stream), "Metropolis-Hastings")) return rc;
-    if (int rc = launched(h, jt::launch_members(args[i], 3, h->stream), "Metropolis-Hastings")) return rc;
-  }
-  for (size_t i = 0; i < L; ++i)  // asynchronous: the devices run side by side
-    if (int rc = rerun_window(c->local[i].h, window[i])) return rc;
-  for (size_t i = 0; i < L; ++i) {
-    sipnet_gpu_handle *h = c->local[i].h;
-    CUDA_OK(cudaSetDevice(h->device));
-    if (int rc = launched(h, rs::launch_accept(acc[i], h->stream), "Metropolis-Hastings")) return rc;
-    h->lastBegin = h->lastEnd = window[i];  // no run range: its outputs are the proposals' (or are gone)
-    h->summariesValid = false;
-  }
+  if (int rc = each_rank(c, [&](size_t i, Local &l) {
+        if (int rc = launched(l.h, rs::launch_snapshot(acc[i], l.h->stream), "Metropolis-Hastings")) return rc;
+        return launched(l.h, jt::launch_members(args[i], 3, l.h->stream), "Metropolis-Hastings");
+      }))
+    return rc;
+  // asynchronous: the devices run side by side
+  if (int rc = each_rank(c, [&](size_t i, Local &l) { return rerun_window(l.h, window[i]); })) return rc;
+  if (int rc = each_rank(c, [&](size_t i, Local &l) {
+        sipnet_gpu_handle *h = l.h;
+        if (int rc = launched(h, rs::launch_accept(acc[i], h->stream), "Metropolis-Hastings")) return rc;
+        h->lastBegin = h->lastEnd = window[i];  // no run range: its outputs are the proposals' (or are gone)
+        h->summariesValid = false;
+        return 0;
+      }))
+    return rc;
   if (int rc = jitter_pass(c, args, 3, false, "Metropolis-Hastings")) return rc;
   return jitter_diag(c, diag);
 }
@@ -1965,7 +1938,7 @@ extern "C" int sipnet_gpu_mh_move(sipnet_gpu_handle *h, const sipnet_gpu_mh_spec
   if (!h) return fail(SIPNET_GPU_ERR_BAD_ARGUMENT, "NULL handle");
   if (int rc = check_mh(spec, h->nsites, h->nmembers, h->stepsDone, h->loglik != nullptr)) return rc;
   sipnet_gpu_comm one = team_of_one(h);
-  return run_mh(&one, spec, spec->scale, spec->tempering, {spec->current_loglik}, {spec->z}, {spec->log_u}, diag);
+  return run_mh(&one, spec, spec->scale, spec->tempering, &spec->current_loglik, &spec->z, &spec->log_u, diag);
 }
 
 extern "C" int sipnet_gpu_comm_mh_move(sipnet_gpu_comm *c, const sipnet_gpu_mh_spec *spec, double *diag) {
@@ -1975,9 +1948,7 @@ extern "C" int sipnet_gpu_comm_mh_move(sipnet_gpu_comm *c, const sipnet_gpu_mh_s
   const bool ll = h->loglik != nullptr;
   const int bad = check_mh(spec, S, h->nmembers, h->stepsDone, ll);
   if (int rc = team_agree(c, bad, bad ? 0 : mh_hash(spec, S, h->stepsDone, ll), "Metropolis-Hastings specs")) return rc;
-  const size_t L = c->local.size();
-  return run_mh(c, spec, spec->scale, spec->tempering, std::vector<const double *>(L, spec->current_loglik),
-                std::vector<const double *>(L, spec->z), std::vector<const double *>(L, spec->log_u), diag);
+  return run_mh(c, spec, spec->scale, spec->tempering, &spec->current_loglik, &spec->z, &spec->log_u, diag);
 }
 
 extern "C" int sipnet_gpu_multi_mh_move(sipnet_gpu_multi *m, const sipnet_gpu_mh_spec *spec, double *diag) {
@@ -1985,37 +1956,11 @@ extern "C" int sipnet_gpu_multi_mh_move(sipnet_gpu_multi *m, const sipnet_gpu_mh
   int64_t step = 0;
   for (const sipnet_gpu_handle *h : m->handles) step = std::max(step, h->stepsDone);
   if (int rc = check_mh(spec, m->nsites, m->nmembers, step, m->handles[0]->loglik != nullptr)) return rc;
-  const size_t D = m->handles.size(), n = (size_t)spec->n_rows, M = (size_t)m->nmembers;
-  // every device's normals [n_rows][its members], log-likelihoods and log u, from the configuration-order arrays
-  std::vector<std::vector<double>> zd(D), cl(D), lu(D);
-  for (size_t d = 0; d < D; ++d) {
-    const size_t nm = (size_t)m->handles[d]->nmembers;
-    zd[d].resize(n * nm);
-    cl[d].resize(nm);
-    lu[d].resize(nm);
-    for (const sipnet_gpu_multi::Run &r : m->parts[d].runs) {
-      for (size_t j = 0; j < n; ++j)
-        memcpy(zd[d].data() + j * nm + r.local0, spec->z + j * M + r.global0, (size_t)r.count * sizeof(double));
-      memcpy(cl[d].data() + r.local0, spec->current_loglik + r.global0, (size_t)r.count * sizeof(double));
-      memcpy(lu[d].data() + r.local0, spec->log_u + r.global0, (size_t)r.count * sizeof(double));
-    }
-  }
-  if (m->split) {  // every device ends with the same diagnostics: take device 0's
-    std::vector<const double *> zp, cp, up;
-    for (size_t d = 0; d < D; ++d) {
-      zp.push_back(zd[d].data());
-      cp.push_back(cl[d].data());
-      up.push_back(lu[d].data());
-    }
-    return run_mh(m->comm, spec, spec->scale, spec->tempering, cp, zp, up, diag);
-  }
-  // whole sites: each device alone on its site range
-  for (size_t d = 0; d < D; ++d) {
-    sipnet_gpu_comm one = team_of_one(m->handles[d]);
-    const size_t s0 = (size_t)m->parts[d].site0;
-    if (int rc = run_mh(&one, spec, spec->scale + s0, spec->tempering + s0, {cl[d].data()}, {zd[d].data()},
-                        {lu[d].data()}, diag ? diag + s0 * 4 : nullptr))
-      return rc;
-  }
-  return 0;
+  const Copies z = device_copies(m, spec->z, (size_t)spec->n_rows), cl = device_copies(m, spec->current_loglik, 1),
+               lu = device_copies(m, spec->log_u, 1);
+  return multi_run(m, [&](sipnet_gpu_comm *c, size_t d) {
+    const int64_t s0 = m->parts[d].site0;
+    return run_mh(c, spec, spec->scale + s0, spec->tempering + s0, cl.at.data() + d, z.at.data() + d, lu.at.data() + d,
+                  from_site(diag, s0, 4));
+  });
 }
