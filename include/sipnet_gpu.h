@@ -533,8 +533,8 @@ int sipnet_gpu_resample(sipnet_gpu_handle *h, const double *u, double ess_fracti
  *   phi_ij = g_j(theta_ij);  mean_j = (1/N) sum_i phi_ij;
  *   V_jl = (1/N) sum_i (phi_ij - mean_j)(phi_il - mean_l)   (population covariance, two passes)
  *   L: semidefinite Cholesky factor of V in column order: for each j, d = V_jj - sum_{m<j} L_jm^2; if
- *      d > 2^-40 V_jj then L_jj = sqrt(d) and L_ij = (V_ij - sum_{m<j} L_im L_jm) / L_jj (i > j), else column j is
- *      zero; rank = the number of nonzero columns
+ *      d > 2^-40 V_jj and V_jj > 2^-80 mean_j^2 then L_jj = sqrt(d) and L_ij = (V_ij - sum_{m<j} L_im L_jm) / L_jj
+ *      (i > j), else column j is zero; rank = the number of nonzero columns
  *   phi'_ij = a phi_ij + (1 - a) mean_j + h sum_{m<=j} L_jm z_mi;  theta'_ij = g_j^-1(phi'_ij)
  * The population covariance is what makes the mixture keep the ensemble's mean and covariance exactly.  A member's
  * proposal is rejected -- the member stays bit-identical and counts as kept -- when some theta' is not finite or not

@@ -230,8 +230,10 @@ __device__ void finish(const Args &a, int s, const double *r) {
     const double vjj = r[kSum0 + tri(j, j)] / N;
     double acc = 0.0;
     for (int m = 0; m < j; ++m) acc += L[tri(j, m)] * L[tri(j, m)];
-    const double d = vjj - acc;
-    if (d > 0x1p-40 * vjj) {
+    const double d = vjj - acc, mu = mom[1 + j];
+    // a row whose spread is below 2^-40 of its mean is constant: its variance is the rounding of the mean, which
+    // a summation of up to 2^23 members keeps below about 2^-42 |mean|, whatever the site's size or split
+    if (d > 0x1p-40 * vjj && vjj > 0x1p-80 * (mu * mu)) {
       const double ljj = sqrt(d);
       L[tri(j, j)] = ljj;
       for (int i = j + 1; i < n; ++i) {

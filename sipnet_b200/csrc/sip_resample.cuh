@@ -28,7 +28,7 @@ namespace rs {
 constexpr int kRec = 6;             // uint64 words per (rank, site) record
 constexpr int kFixBits = 100;     // w and w^2 are summed as floor(x 2^100)
 constexpr int kWeightBits = 40;   // W = floor(w 2^40)
-constexpr int64_t kMaxSiteMembers = int64_t(1) << 23;  // keeps T = sum W below 2^63
+constexpr int64_t kMaxSiteMembers = int64_t(1) << 23;  // keeps T = sum W <= 2^63 (equal weights: 2^23 2^40)
 
 // Record layouts (uint64 words):
 //   pass a  [0] participants N  [1] max l of the participants (double bits; -inf if none)  [2] members n

@@ -176,7 +176,7 @@ def proposal_reference(params, status, cur, ms, nsites, rows, scale, z):
         c = phi - mean[:, None]
         V = np.array([[math.fsum(c[j] * c[l]) / N for l in range(n)] for j in range(n)])
         sd[:, s] = np.sqrt(np.diag(V))
-        Lm, rank = cholesky(V)
+        Lm, rank = cholesky(V, mean)
         diag[s, 1] = rank
         pn = phi + scale[s] * (Lm @ z[:, idx])
         th = np.array([inv(pn[j], r[1], r[2], r[3]) for j, r in enumerate(rows)])

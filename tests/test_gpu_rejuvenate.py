@@ -75,14 +75,15 @@ def in_domain(t, tf, lo, hi):
     return ok & (t > 0) if tf == L else ok & (t > lo) & (t < hi) if tf == G else ok
 
 
-def cholesky(V):
-    """The header's semidefinite Cholesky, column order; -> (L, rank)."""
+def cholesky(V, mean=None):
+    """The header's semidefinite Cholesky, column order; -> (L, rank).  mean: the rows' means (a row whose variance
+    is not above 2^-80 mean^2 is constant); None leaves that test out."""
     n = V.shape[0]
     Lm = np.zeros((n, n))
     rank = 0
     for j in range(n):
         d = V[j, j] - math.fsum(Lm[j, m] * Lm[j, m] for m in range(j))
-        if d > 2.0 ** -40 * V[j, j]:
+        if d > 2.0 ** -40 * V[j, j] and (mean is None or V[j, j] > 2.0 ** -80 * mean[j] ** 2):
             Lm[j, j] = math.sqrt(d)
             for i in range(j + 1, n):
                 Lm[i, j] = (V[i, j] - math.fsum(Lm[i, m] * Lm[j, m] for m in range(j))) / Lm[j, j]
@@ -116,7 +117,7 @@ def reference(params, status, ms, nsites, rows, tf, lo, hi, shrink, z):
         c = phi - mean[:, None]
         V = np.array([[math.fsum(c[j] * c[l]) / N for l in range(n)] for j in range(n)])
         sd[:, s] = np.sqrt(np.diag(V))
-        Lm, rank = cholesky(V)
+        Lm, rank = cholesky(V, mean)
         h = math.sqrt(1 - a * a)
         pn = a * phi + ((1 - a) * mean)[:, None] + h * (Lm @ z[:, idx])
         th = np.array([inv(pn[j], tf[j], lo[j], hi[j]) for j in range(n)])
@@ -138,12 +139,22 @@ def reference(params, status, ms, nsites, rows, tf, lo, hi, shrink, z):
     return Q, diag, phin, moved, sd, margin
 
 
-def within_bound(got_params, phin, sd, ms, rows, tf, lo, hi, cols):
+def within_bound(got_params, phin, sd, ms, rows, tf, lo, hi, cols, theta=False, extra=None):
+    """|phi(got) - phi'| <= 1e-9 sd + 4 ulp (+ extra[j][member], a caller's derived slack).  theta=True compares in
+    theta instead: got inside that interval mapped through the monotone inverse transform, widened by 4 ulp of theta
+    for the transform's own rounding (near a LOGIT bound the round trip theta -> phi loses the digits the bound is
+    about)."""
     for j in range(len(rows)):
-        g = fwd(got_params[rows[j], cols], tf[j], lo[j], hi[j])
         w = phin[j, cols]
-        tol = 1e-9 * sd[j, ms[cols]] + 4 * np.spacing(np.abs(w))
-        if not np.all(np.abs(g - w) <= tol):
+        tol = 1e-9 * sd[j, ms[cols]] + 4 * np.spacing(np.abs(w)) + (0.0 if extra is None else extra[j, cols])
+        if theta:
+            a, b = inv(w - tol, tf[j], lo[j], hi[j]), inv(w + tol, tf[j], lo[j], hi[j])
+            g = got_params[rows[j], cols]
+            slack = 4 * np.spacing(np.maximum(np.abs(a), np.abs(b)))
+            ok = (g >= np.minimum(a, b) - slack) & (g <= np.maximum(a, b) + slack)
+        else:
+            ok = np.abs(fwd(got_params[rows[j], cols], tf[j], lo[j], hi[j]) - w) <= tol
+        if not np.all(ok):
             return False
     return True
 
